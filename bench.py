@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ALS ratings/s per sweep (headline) on synthetic data of the BASELINE.json shapes.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c1] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c1] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one ALS sweep (item half-step, all-gather, user half-step, all-gather) over the
 whole ratings matrix, factors and CSR shards resident in HBM.  `value` = nnz / (time per sweep),
@@ -10,6 +10,8 @@ with HOST inputs: pinned COO triples -> H2D -> CSR build + plan -> `e2e_sweeps` 
 D2H, all inside the timed region.  `roofline` is the half-step kernel sequence against the
 measured HBM peak with SURVEY.md 8(d) algorithmic bytes; `cpu_baseline` is the CPU oracle port
 (Spark local[N] cannot run in this image) on a bounded row sample.  Prints ONE JSON line.
+`--dump-outputs DIR` writes the factor matrices of the last timed sweep as DIR/<name>.npy, so that two builds
+can be compared output for output (same arguments -> same inputs).
 """
 from __future__ import annotations
 
@@ -124,6 +126,20 @@ def assert_same_on_all_ranks(values, what, dev, world):
     dist.all_reduce(lo, op=dist.ReduceOp.MIN)
     if not torch.equal(hi, lo):
         raise RuntimeError(f"ranks disagree on {what}: max {hi.tolist()} min {lo.tolist()}")
+
+
+DUMP_BUDGET = 60 << 20      # bytes of .npy payload: under 64 MB (10^6 bytes each) with the headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy.  When they hold more than DUMP_BUDGET bytes in all, every array keeps
+    the same fixed, seeded sample of its rows (in row order), so dumps of two runs stay comparable row for row."""
+    os.makedirs(out_dir, exist_ok=True)
+    keep = min(1.0, DUMP_BUDGET / sum(a.nbytes for a in arrays.values()))
+    for name, a in arrays.items():
+        if keep < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * keep), replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def algorithmic_bytes(w):
@@ -465,8 +481,12 @@ def main():
     ap.add_argument("--score-slab", type=int, default=65536)
     ap.add_argument("--score-items-per-gpu", type=int, default=1_250_000)
     ap.add_argument("--score-topk", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the user / item factors of the last timed sweep as "
+                    "DIR/als_user_factors.npy and DIR/als_item_factors.npy (fp32; a seeded sample of rows above 60 MiB)")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args, w)
 
@@ -529,6 +549,10 @@ def main():
     total_ms, t_item, t_user = (float(x) for x in tm.tolist())
     ms_per_step = total_ms / args.steps
     value = w["nnz"] / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        eng.sync_factors()          # what fit() returns: the full fp32 factors on every rank (a collective when sharded)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"als_user_factors": eng.X.cpu().numpy(), "als_item_factors": eng.Y.cpu().numpy()})
     rmse_train = eng.rmse(u[:1_000_000], i[:1_000_000], r[:1_000_000])
 
     # ---- end-to-end: host COO in pinned memory -> H2D -> CSR + plan -> sweeps -> factors D2H ----------

@@ -4,9 +4,8 @@ Restates src/hybrid_system.py:57-75 (adaptive_fusion), :108 (stable descending s
 first top_k) and src/als_model.py:171-177 (compute_f1_score, the weight selector used at
 hybrid_system.py:47-48).  PINNED: oracle/ref_loader.py loads the reference's own,
 unmodified hybrid_system.py in the build container and tests/golden/make_golden.py
-commits its outputs as fixtures (tests/golden/hybrid_*.npz); tests/test_oracle_golden.py
-checks this restatement against them, and against the live reference when
-/root/reference is present.
+commits its outputs as fixtures (tests/golden/hybrid_reference_cases.json);
+tests/test_oracle_golden.py checks this restatement against them.
 
 MinMaxScaler semantics (sklearn 1.2.2 pinned, requirements.txt:3; formula unchanged in
 the installed 1.9.0): scale_ = 1/(max-min) with a zero range replaced by 1,

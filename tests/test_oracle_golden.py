@@ -1,5 +1,4 @@
-"""CPU: the oracle against the committed fixtures (and against the live reference code when
-/root/reference is present).  Hybrid fixtures were produced by the reference's own
+"""CPU: the oracle against the committed fixtures.  Hybrid fixtures were produced by the reference's own
 src/hybrid_system.py; ALS / tower fixtures are oracle-minted (parity unpinned, see headers)."""
 import json
 import os
@@ -7,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle import als_oracle, c_oracle, hybrid_oracle, ref_loader, towers_oracle
+from oracle import als_oracle, c_oracle, hybrid_oracle, towers_oracle
 
 G = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -32,22 +31,11 @@ def test_hybrid_oracle_matches_reference_fixture(case):
     assert np.allclose(sc, case["out_scores"], rtol=0, atol=2e-7)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present (GPU box)")
-def test_live_reference_agrees_with_fixtures_and_oracle():
-    rng = np.random.default_rng(99)
-    for n, k in ((17, 5), (300, 20)):
-        als, tt = rng.normal(3, 1, n), rng.normal(0, 1, n).astype(np.float32)
-        a = [(i, float(x)) for i, x in enumerate(als)]
-        t = [(i, x) for i, x in enumerate(tt)]
-        out, _ = ref_loader.reference_recommend({1: a}, {1: t}, 1, list(range(n)), top_k=k, als_f1=0.5, tt_f1=0.25)
-        blend = hybrid_oracle.adaptive_fusion_dense(als, tt.astype(np.float64), 0.5, 0.25)
-        idx, sc = hybrid_oracle.topk_desc(blend, k)
-        assert [i for i, _ in out] == list(idx)
-        assert np.allclose([s for _, s in out], sc, atol=2e-7)
-    f1 = ref_loader.load_reference_hybrid().compute_f1_score
-    assert f1({1: 5, 2: 4, 3: 3}, {1: .9, 2: .8, 9: .7, 3: .1}, k=2) == pytest.approx(0.8)
+def test_f1_known_answers_of_the_reference():
+    """compute_f1_score (src/als_model.py:171-177) returned these for the same inputs (SURVEY.md Appendix C):
+    F1@2 of {1, 2, 9} against {1, 2, 3} is 0.8, and an empty set of actual ratings scores 0."""
     assert hybrid_oracle.compute_f1_score({1: 5, 2: 4, 3: 3}, {1: .9, 2: .8, 9: .7, 3: .1}, k=2) == pytest.approx(0.8)
-    assert f1({}, {1: 1.0}) == 0 and hybrid_oracle.compute_f1_score({}, {1: 1.0}) == 0
+    assert hybrid_oracle.compute_f1_score({}, {1: 1.0}) == 0
 
 
 def test_minmax_semantics_match_sklearn():
