@@ -82,6 +82,9 @@ SIGNATURES = {
     "hals_score_blend_topk": (ctypes.c_int, [c_vp, c_i64, c_vp, c_i64, ctypes.c_int, c_vp, c_i64, c_vp, c_i64,
                                              ctypes.c_int, c_i64, c_i64, c_vp, c_f32, c_f32, ctypes.c_int, c_i32,
                                              c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "hals_score_blend_topk_excluding": (ctypes.c_int, [c_vp, c_i64, c_vp, c_i64, ctypes.c_int, c_vp, c_i64, c_vp, c_i64,
+                                                       ctypes.c_int, c_i64, c_i64, c_vp, c_f32, c_f32, ctypes.c_int, c_i32,
+                                                       c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "hals_topk_merge": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_i64, ctypes.c_int, c_vp, c_vp, c_vp]),
     "hals_score_one_user": (ctypes.c_int, [c_vp, c_vp, c_i64, ctypes.c_int, c_vp, c_i64, c_vp, c_vp]),
     "hals_fuse_lists": (ctypes.c_int, [c_vp, c_vp, c_i64, c_f32, c_f32, c_vp, c_vp, c_vp]),

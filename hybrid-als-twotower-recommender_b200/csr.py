@@ -61,14 +61,16 @@ def build_csr(rows: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, n_rows
               row_begin: int = 0, row_end: int | None = None, counts: torch.Tensor | None = None) -> CsrShard:
     """Stable COO -> CSR for rows in [row_begin, row_end): the ratings of a row keep their
     input order, duplicates are kept (Spark does not merge them).  `counts` (int64 [n_rows], device) may pass
-    the per-row rating counts of the WHOLE matrix when the caller already has them."""
+    the per-row rating counts of the WHOLE matrix when the caller already has them.  `vals` may be None (a pattern
+    without values; the shard's `vals` is then None)."""
     if row_end is None:
         row_end = n_rows
     dev = rows.device
     whole = row_begin == 0 and row_end == n_rows
     if not whole:
         keep = (rows >= row_begin) & (rows < row_end)
-        rows, cols, vals = rows[keep], cols[keep], vals[keep]
+        rows, cols = rows[keep], cols[keep]
+        vals = vals[keep] if vals is not None else None
     # 32-bit sort keys: the radix sort moves half the bytes of an int64 sort
     local = (rows - row_begin).to(torch.int32) if not whole else rows.to(torch.int32)
     order = torch.sort(local, stable=True).indices
@@ -79,7 +81,7 @@ def build_csr(rows: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, n_rows
     rowptr = torch.zeros(row_end - row_begin + 1, dtype=torch.int64, device=dev)
     torch.cumsum(cnt, 0, out=rowptr[1:])
     return CsrShard(row_begin, row_end, n_rows, rowptr, cols[order].to(torch.int32).contiguous(),
-                    vals[order].to(torch.float32).contiguous(), rowptr.cpu().numpy())
+                    vals[order].to(torch.float32).contiguous() if vals is not None else None, rowptr.cpu().numpy())
 
 
 class AlsPlanHandle:

@@ -79,12 +79,26 @@ __device__ __forceinline__ float blend_value(const BlendCoef& c, float wa, float
   return fmaf(wa, (sa - c.min_a) * c.sc_a, wt * ((st - c.min_t) * c.sc_t));
 }
 
-template <bool EXTREMA, int CAP>
+// true when the ascending list items[lo, hi) holds v
+__device__ __forceinline__ bool sorted_contains(const int32_t* __restrict__ items, int64_t lo, int64_t hi, int32_t v) {
+  const int64_t end = hi;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (items[mid] < v) lo = mid + 1; else hi = mid;
+  }
+  return lo < end && items[lo] == v;
+}
+
+// EXCL: items listed for a user in the exclusion CSR (excl_rowptr indexed by the user -- uid(r), not the tile row --,
+// global item ids) never pass the filter; the lookup runs only for items that already beat the row threshold.
+template <bool EXTREMA, int CAP, bool EXCL = false>
 __global__ void __launch_bounds__(kScThreads)
 score_simt_kernel(ScoreArgs A, float* __restrict__ extrema_out, const float* __restrict__ extrema_in,
                   float w_als, float w_tt, int topk, int32_t item_offset,
                   uint64_t* __restrict__ cand /* [splits][n_users][CAP] */,
-                  int32_t* __restrict__ out_idx, float* __restrict__ out_score /* [splits][n_users][topk] */) {
+                  int32_t* __restrict__ out_idx, float* __restrict__ out_score /* [splits][n_users][topk] */,
+                  const int64_t* __restrict__ excl_rowptr = nullptr, const int32_t* __restrict__ excl_items = nullptr) {
+  static_assert(!EXCL || !EXTREMA, "exclusion lists apply to the top-k pass");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int K = A.ka + A.kt;
   const int LD = K + 1;
@@ -94,6 +108,7 @@ score_simt_kernel(ScoreArgs A, float* __restrict__ extrema_out, const float* __r
   float* rowstat = St + kScUsers * 65;                       // [64][4]: extrema or coefficients
   __shared__ int cnt[kScUsers];
   __shared__ unsigned long long thr[kScUsers];
+  __shared__ int64_t xrow[EXCL ? kScUsers : 1][2];            // EXCL: [begin, end) of each row's exclusion list
 
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
   const int lane = tid & 31, warp = tid >> 5;
@@ -121,6 +136,7 @@ score_simt_kernel(ScoreArgs A, float* __restrict__ extrema_out, const float* __r
     cnt[tid] = 0;
     thr[tid] = kTopkEmpty;
     const int64_t u = uid(tid);
+    if (EXCL && u0 + tid < n_rows) { xrow[tid][0] = excl_rowptr[u]; xrow[tid][1] = excl_rowptr[u + 1]; }
     float4 ex;
     if (EXTREMA) {
       const float inf = __int_as_float(0x7f800000);
@@ -214,13 +230,15 @@ score_simt_kernel(ScoreArgs A, float* __restrict__ extrema_out, const float* __r
         if (c + kScItems > CAP) {
           c = topk_compact<CAP>(buf, c, topk, lane, &t);
         }
+        const int64_t xlo = EXCL ? xrow[r][0] : 0, xhi = EXCL ? xrow[r][1] : 0;
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
           const int col = lane + 32 * h;
           const int64_t i = it0 + col;
           const float s = St[r * 65 + col];
           const uint64_t key = topk_key(s, (int32_t)(i + item_offset));
-          const bool pass = (i < i_end) && (key > t);
+          const bool pass = (i < i_end) && (key > t) &&
+                            !(EXCL && sorted_contains(excl_items, xlo, xhi, (int32_t)(i + item_offset)));
           const unsigned m = __ballot_sync(0xffffffffu, pass);
           if (pass) buf[c + __popc(m & ((1u << lane) - 1u))] = key;
           c += __popc(m);
@@ -450,26 +468,37 @@ int score_extrema_simt(const ScoreOperands& O, int64_t n_users, int64_t n_items,
   return 0;
 }
 
-template <bool EX, int CAPV>
+template <int CAPV, bool EXCL>
 static int launch_simt_topk(const ScoreArgs& A, dim3 grid, size_t smem, const float* extrema, float w_als, float w_tt,
-                            int topk, int32_t item_offset, uint64_t* cand, int32_t* oi, float* os, cudaStream_t st) {
-  HALS_CUDA(cudaFuncSetAttribute(score_simt_kernel<EX, CAPV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  score_simt_kernel<EX, CAPV><<<grid, kScThreads, smem, st>>>(A, nullptr, extrema, w_als, w_tt, topk, item_offset, cand, oi, os);
+                            int topk, int32_t item_offset, uint64_t* cand, int32_t* oi, float* os,
+                            const int64_t* excl_rowptr, const int32_t* excl_items, cudaStream_t st) {
+  HALS_CUDA(cudaFuncSetAttribute(score_simt_kernel<false, CAPV, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  score_simt_kernel<false, CAPV, EXCL><<<grid, kScThreads, smem, st>>>(A, nullptr, extrema, w_als, w_tt, topk, item_offset,
+                                                                       cand, oi, os, excl_rowptr, excl_items);
   HALS_LAUNCH_CHECK();
   return 0;
 }
+template <int CAPV>
+static int launch_simt_topk_excl(const ScoreArgs& A, dim3 grid, size_t smem, const float* extrema, float w_als, float w_tt,
+                                 int topk, int32_t item_offset, uint64_t* cand, int32_t* oi, float* os,
+                                 const int64_t* excl_rowptr, const int32_t* excl_items, cudaStream_t st) {
+  if (excl_rowptr != nullptr)
+    return launch_simt_topk<CAPV, true>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, excl_rowptr,
+                                        excl_items, st);
+  return launch_simt_topk<CAPV, false>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, nullptr, nullptr, st);
+}
 static int launch_simt_topk_cap(int cap, const ScoreArgs& A, dim3 grid, size_t smem, const float* extrema, float w_als,
                                 float w_tt, int topk, int32_t item_offset, uint64_t* cand, int32_t* oi, float* os,
-                                cudaStream_t st) {
-  if (cap == 128) return launch_simt_topk<false, 128>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, st);
-  if (cap == 256) return launch_simt_topk<false, 256>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, st);
-  return launch_simt_topk<false, 512>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, st);
+                                const int64_t* xr, const int32_t* xi, cudaStream_t st) {
+  if (cap == 128) return launch_simt_topk_excl<128>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, xr, xi, st);
+  if (cap == 256) return launch_simt_topk_excl<256>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, xr, xi, st);
+  return launch_simt_topk_excl<512>(A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand, oi, os, xr, xi, st);
 }
 
 int score_blend_topk_simt(const ScoreOperands& O, int64_t n_users, int64_t n_items, const float* extrema,
                           float w_als, float w_tt, int topk, int32_t item_offset, int32_t* out_idx,
                           float* out_score, void* workspace, const int32_t* user_list, const int32_t* user_count,
-                          cudaStream_t st) {
+                          const int64_t* excl_rowptr, const int32_t* excl_items, cudaStream_t st) {
   const int cap = topk_capacity(topk);
   const size_t smem = score_smem_bytes(O.ka + O.kt);
   ScoreArgs A{O.Ua, O.ua_stride, O.Ia, O.ia_stride, O.Ut, O.ut_stride, O.It, O.it_stride, O.ka, O.kt,
@@ -482,7 +511,7 @@ int score_blend_topk_simt(const ScoreOperands& O, int64_t n_users, int64_t n_ite
     float* pscore = (float*)(pidx + (size_t)splits * n_users * topk);
     dim3 grid((unsigned)((n_users + kScUsers - 1) / kScUsers), (unsigned)splits);
     if (int rc = launch_simt_topk_cap(cap, A, grid, smem, extrema, w_als, w_tt, topk, item_offset, cand,
-                                      splits == 1 ? out_idx : pidx, splits == 1 ? out_score : pscore, st)) return rc;
+                                      splits == 1 ? out_idx : pidx, splits == 1 ? out_score : pscore, excl_rowptr, excl_items, st)) return rc;
     if (splits > 1) return hals_topk_merge(pidx, pscore, splits, n_users, topk, out_idx, out_score, (void*)st);
     return 0;
   }
@@ -498,7 +527,7 @@ int score_blend_topk_simt(const ScoreOperands& O, int64_t n_users, int64_t n_ite
   int64_t gx = (rows + kScUsers - 1) / kScUsers;
   if (gx > 32) gx = 32;
   if (int rc = launch_simt_topk_cap(cap, A, dim3((unsigned)gx, (unsigned)splits), smem, extrema, w_als, w_tt, topk,
-                                    item_offset, cand, pidx, pscore, st)) return rc;
+                                    item_offset, cand, pidx, pscore, excl_rowptr, excl_items, st)) return rc;
   {
     const unsigned blocks = (unsigned)((rows + 3) / 4);
     if (cap == 128) topk_merge_kernel<128><<<blocks, 128, 0, st>>>(pidx, pscore, splits, rows, topk, out_idx, out_score, user_list, user_count, 0, rows);
@@ -514,7 +543,7 @@ int score_blend_topk_simt(const ScoreOperands& O, int64_t n_users, int64_t n_ite
     // candidate rows of the overflow live in the plain (unsplit) SIMT workspace that follows the list region
     uint64_t* cand2 = (uint64_t*)((uint8_t*)workspace + score_simt_list_workspace_bytes(n_users, n_items, topk));
     if (int rc = launch_simt_topk_cap(cap, A, dim3((unsigned)g2, 1), smem, extrema, w_als, w_tt, topk, item_offset,
-                                      cand2, out_idx, out_score, st)) return rc;
+                                      cand2, out_idx, out_score, excl_rowptr, excl_items, st)) return rc;
   }
   return 0;
 }

@@ -140,12 +140,46 @@ __device__ __noinline__ int compact_row(uint64_t* buf, int count, int keep, int 
   return topk_select_compact<CAP>(buf, count, keep, lane, thr_out);
 }
 
-template <int PASS, int BN, int CAP, int PARTS>
+// Pass 2 with an exclusion list (EXCL): each epilogue thread walks its user's ascending list with a forward-only cursor.
+// A thread meets its columns in ascending item order (half * HB + g * W + 8 * o + c within a tile, tiles ascending), so
+// the cursor never moves back; it is consulted only for items that passed the threshold, and excluded items never enter
+// a candidate buffer -- the threshold and the compactions only ever see allowed items.  Exactness is unchanged: the
+// verification bounds what a stream REJECTED, and an excluded item cannot belong to the answer.  A user left with fewer
+// than k allowed items has kth = -inf; if one of its streams still raised its threshold (the final trim to `keep`, or a
+// compaction at k > 224) the verification flags it and the exact SIMT re-run, which filters too, produces the list.
+struct ExclCursor {
+  const int32_t* p;        // next unread entry
+  int left;                // entries from p to the end of the row
+  int32_t next;            // the smallest excluded id not yet passed (INT32_MAX: none)
+  __device__ __forceinline__ void init(const int64_t* rowptr, const int32_t* items, int64_t u, int32_t first) {
+    int64_t lo = rowptr[u], hi = rowptr[u + 1];
+    const int64_t end = hi;
+    while (lo < hi) {                                  // lower bound of `first`
+      const int64_t mid = (lo + hi) >> 1;
+      if (items[mid] < first) lo = mid + 1; else hi = mid;
+    }
+    p = items + lo;
+    left = (int)(end - lo);
+    next = left > 0 ? *p : 0x7fffffff;
+  }
+  // true when item `gi` (global id, ascending across calls) is excluded
+  __device__ __forceinline__ bool excluded(int32_t gi) {
+    while (next < gi) {
+      ++p;
+      next = --left > 0 ? *p : 0x7fffffff;
+    }
+    return next == gi;
+  }
+};
+
+template <int PASS, int BN, int CAP, int PARTS, bool EXCL>
 __global__ void __launch_bounds__(64 + 128 * PARTS, 1)
 score_tc_kernel(const __grid_constant__ CUtensorMap map_u, const __grid_constant__ CUtensorMap map_i, ScoreTcArgs A,
                 float* __restrict__ ex_val /* [splits][U][4][4] */, int32_t* __restrict__ ex_idx,
                 uint64_t* __restrict__ cand /* [splits][U][CAP] */, int32_t* __restrict__ cand_cnt,
-                float* __restrict__ cand_thr /* [splits][U] */) {
+                float* __restrict__ cand_thr /* [splits][U] */,
+                const int64_t* __restrict__ excl_rowptr /* EXCL: [U+1] */, const int32_t* __restrict__ excl_items) {
+  static_assert(!EXCL || PASS == 2, "exclusion lists apply to the top-k pass");
   constexpr int JPT = (PASS == 1) ? 2 : 1;             // accumulator jobs per item tile: pass 1 scores the two models
                                                        // one after the other (N = 256 each: an N = 128 MMA pair is
                                                        // shared-memory-bandwidth bound at M = 128)
@@ -269,6 +303,11 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_u, const __grid_constant
     } else {
       mybuf = cand + ((size_t)vs * A.n_users + (live ? u : 0)) * CAP;
       if (!live) thr = __int_as_float(0x7f800000);
+    }
+    ExclCursor xc;
+    if (EXCL) {
+      if (live) xc.init(excl_rowptr, excl_items, u, (int32_t)i_begin + A.item_offset);
+      else { xc.left = 0; xc.next = 0x7fffffff; }     // a dead row never has a survivor
     }
 
     for (int t = 0; t < n_tiles; ++t) {
@@ -398,7 +437,8 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_u, const __grid_constant
               const int64_t ib = it0 + c0 + 8 * o;
               if ((m & (m - 1)) == 0) {
                 const int64_t i = ib + (__ffs(m) - 1);
-                if (!ragged || i < i_end) mybuf[cnt++] = topk_key(gm, (int32_t)i);
+                if ((!ragged || i < i_end) && !(EXCL && xc.excluded((int32_t)i + A.item_offset)))
+                  mybuf[cnt++] = topk_key(gm, (int32_t)i);
               } else {
                 while (m) {
                   const int c = __ffs(m) - 1;
@@ -407,7 +447,8 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_u, const __grid_constant
 #pragma unroll
                   for (int cc = 1; cc < 8; ++cc) s = (cc == c) ? v[8 * o + cc] : s;
                   const int64_t i = ib + c;
-                  if (!ragged || i < i_end) mybuf[cnt++] = topk_key(s, (int32_t)i);
+                  if ((!ragged || i < i_end) && !(EXCL && xc.excluded((int32_t)i + A.item_offset)))
+                    mybuf[cnt++] = topk_key(s, (int32_t)i);
                 }
               }
             }
@@ -739,15 +780,25 @@ TcPlan make_plan(int64_t n_users, int64_t n_items, int ka, int kt, int topk) {
   return p;
 }
 
-template <int PASS, int BN, int CAP, int PARTS>
+template <int PASS, int BN, int CAP, int PARTS, bool EXCL = false>
 int launch_tc(const CUtensorMap& mu, const CUtensorMap& mi, const ScoreTcArgs& A, int nkb, float* exv, int32_t* exi,
-              uint64_t* cand, int32_t* cnt, float* thr, cudaStream_t st) {
+              uint64_t* cand, int32_t* cnt, float* thr, cudaStream_t st, const int64_t* excl_rowptr = nullptr,
+              const int32_t* excl_items = nullptr) {
   const size_t smem = (size_t)nkb * kStM * 128 + (size_t)kStRing * BN * 128 + 1024;
-  HALS_CUDA(cudaFuncSetAttribute(score_tc_kernel<PASS, BN, CAP, PARTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  HALS_CUDA(cudaFuncSetAttribute(score_tc_kernel<PASS, BN, CAP, PARTS, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((unsigned)((A.n_users + kStM - 1) / kStM), (unsigned)A.n_splits);
-  score_tc_kernel<PASS, BN, CAP, PARTS><<<grid, 64 + 128 * PARTS, smem, st>>>(mu, mi, A, exv, exi, cand, cnt, thr);
+  score_tc_kernel<PASS, BN, CAP, PARTS, EXCL><<<grid, 64 + 128 * PARTS, smem, st>>>(mu, mi, A, exv, exi, cand, cnt, thr,
+                                                                                    excl_rowptr, excl_items);
   HALS_LAUNCH_CHECK();
   return 0;
+}
+
+template <int CAP>
+int launch_tc_topk(const CUtensorMap& mu, const CUtensorMap& mi, const ScoreTcArgs& A, int nkb, uint64_t* cand,
+                   int32_t* cnt, float* thr, cudaStream_t st, const int64_t* excl_rowptr, const int32_t* excl_items) {
+  if (excl_rowptr != nullptr)
+    return launch_tc<2, kTcBN, CAP, kStParts2, true>(mu, mi, A, nkb, nullptr, nullptr, cand, cnt, thr, st, excl_rowptr, excl_items);
+  return launch_tc<2, kTcBN, CAP, kStParts2>(mu, mi, A, nkb, nullptr, nullptr, cand, cnt, thr, st);
 }
 
 }  // namespace
@@ -806,12 +857,12 @@ extern "C" int hals_score_extrema(const float* Ua, int64_t ua_stride, const floa
   return score_extrema_simt(O, n_users, n_items, extrema, list, fcount, st);   // exact re-run of unproven users
 }
 
-extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride,
-                                     int ka, const float* Ut, int64_t ut_stride, const float* It,
-                                     int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
-                                     const float* extrema, float w_als, float w_tt, int topk,
-                                     int32_t item_offset, int32_t* out_idx, float* out_score,
-                                     void* workspace, size_t workspace_bytes, void* stream) {
+// The body of hals_score_blend_topk and hals_score_blend_topk_excluding (excl_rowptr == NULL: no exclusion).
+static int blend_topk(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride, int ka, const float* Ut,
+                      int64_t ut_stride, const float* It, int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
+                      const float* extrema, float w_als, float w_tt, int topk, int32_t item_offset, int32_t* out_idx,
+                      float* out_score, const int64_t* excl_rowptr, const int32_t* excl_items, void* workspace,
+                      size_t workspace_bytes, void* stream) {
   if (int rc = check_score_args(Ua, Ia, ka, Ut, It, kt, n_users, n_items)) return rc;
   HALS_REQUIRE(extrema && out_idx && out_score && workspace, "null pointer");
   HALS_REQUIRE(topk >= 1 && topk <= 256, "topk must be in [1,256]");
@@ -823,7 +874,7 @@ extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const f
   uint8_t* W = (uint8_t*)workspace;
   if (!p.use_tc)
     return score_blend_topk_simt(O, n_users, n_items, extrema, w_als, w_tt, topk, item_offset, out_idx, out_score,
-                                 W + p.off_simt, nullptr, nullptr, st);
+                                 W + p.off_simt, nullptr, nullptr, excl_rowptr, excl_items, st);
   __nv_bfloat16* ub = (__nv_bfloat16*)(W + p.off_ub);
   __nv_bfloat16* ib = (__nv_bfloat16*)(W + p.off_ib);
   float2* unorm = (float2*)(W + p.off_unorm);
@@ -847,10 +898,11 @@ extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const f
       !tma::make_bf16_rowmajor_map(&mi, ib, (uint64_t)n_items, (uint64_t)p.Kp, kTcBN))
     return fail(HALS_ERR_CUDA, "%s: cuTensorMapEncodeTiled failed%s", __func__);
   ScoreTcArgs A{p.nkb_a, p.nkb_t, n_users, n_items, p.items_per_split, p.splits, p.keep, item_offset};
+  const int nkb = p.nkb_a + p.nkb_t;
   int rc;
-  if (p.cap == 128) rc = launch_tc<2, kTcBN, 128, kStParts2>(mu, mi, A, p.nkb_a + p.nkb_t, nullptr, nullptr, cand, cnt, thr, st);
-  else if (p.cap == 256) rc = launch_tc<2, kTcBN, 256, kStParts2>(mu, mi, A, p.nkb_a + p.nkb_t, nullptr, nullptr, cand, cnt, thr, st);
-  else rc = launch_tc<2, kTcBN, 512, kStParts2>(mu, mi, A, p.nkb_a + p.nkb_t, nullptr, nullptr, cand, cnt, thr, st);
+  if (p.cap == 128) rc = launch_tc_topk<128>(mu, mi, A, nkb, cand, cnt, thr, st, excl_rowptr, excl_items);
+  else if (p.cap == 256) rc = launch_tc_topk<256>(mu, mi, A, nkb, cand, cnt, thr, st, excl_rowptr, excl_items);
+  else rc = launch_tc_topk<512>(mu, mi, A, nkb, cand, cnt, thr, st, excl_rowptr, excl_items);
   if (rc) return rc;
   const int vsplits = kStParts2 * p.splits;
   ExactArgs E{Ua, ua_stride, Ia, ia_stride, ka, Ut, ut_stride, It, it_stride, kt, n_users, vsplits};
@@ -876,5 +928,27 @@ extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const f
   score_flag_list_kernel<<<(unsigned)((n_users + 255) / 256), 256, 0, st>>>(flag, n_users, 2, list, fcount, nullptr);
   HALS_LAUNCH_CHECK();
   return score_blend_topk_simt(O, n_users, n_items, extrema, w_als, w_tt, topk, item_offset, out_idx, out_score,
-                               W + p.off_simt, list, fcount, st);    // exact re-run of unproven users
+                               W + p.off_simt, list, fcount, excl_rowptr, excl_items, st);    // exact re-run of unproven users
+}
+
+extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride,
+                                     int ka, const float* Ut, int64_t ut_stride, const float* It,
+                                     int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
+                                     const float* extrema, float w_als, float w_tt, int topk,
+                                     int32_t item_offset, int32_t* out_idx, float* out_score,
+                                     void* workspace, size_t workspace_bytes, void* stream) {
+  return blend_topk(Ua, ua_stride, Ia, ia_stride, ka, Ut, ut_stride, It, it_stride, kt, n_users, n_items, extrema, w_als,
+                    w_tt, topk, item_offset, out_idx, out_score, nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int hals_score_blend_topk_excluding(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride,
+                                               int ka, const float* Ut, int64_t ut_stride, const float* It,
+                                               int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
+                                               const float* extrema, float w_als, float w_tt, int topk,
+                                               int32_t item_offset, int32_t* out_idx, float* out_score,
+                                               const int64_t* excl_rowptr, const int32_t* excl_items,
+                                               void* workspace, size_t workspace_bytes, void* stream) {
+  HALS_REQUIRE((excl_rowptr == nullptr) == (excl_items == nullptr), "excl_rowptr and excl_items must both be set or both NULL");
+  return blend_topk(Ua, ua_stride, Ia, ia_stride, ka, Ut, ut_stride, It, it_stride, kt, n_users, n_items, extrema, w_als,
+                    w_tt, topk, item_offset, out_idx, out_score, excl_rowptr, excl_items, workspace, workspace_bytes, stream);
 }

@@ -130,14 +130,32 @@ class HybridRecommendationSystem:
             return []
 
     # -- additive batched path ------------------------------------------------------------------
-    def recommend_batch(self, user_ids, item_features, top_k=5, user_chunk=65536):
+    @staticmethod
+    def _exclusion(exclude, user_ids, cand_ids, dev):
+        """DataFrame of (userId, itemId) pairs -> exclusion CSR over the rows of a batched call (None -> None).
+        The id matching runs on the device (sorted ids + searchsorted)."""
+        if exclude is None:
+            return None
+        import torch
+        from .scoring import exclusion_lists_by_id
+
+        def t(a):
+            return torch.from_numpy(np.ascontiguousarray(np.asarray(a, dtype=np.int64))).to(dev)
+        return exclusion_lists_by_id(t(user_ids), t(cand_ids), t(exclude["userId"].values), t(exclude["itemId"].values))
+
+    def recommend_batch(self, user_ids, item_features, top_k=5, user_chunk=65536, *, exclude=None):
         """Top-k hybrid recommendations for many users at once.
 
         user_ids: raw user ids known to both models; item_features: DataFrame of candidates
         (itemId, manufacturer_id, category_id, price, average_review_rating), items known to the
         ALS model.  Returns (item_ids [U,top_k] int64 numpy, scores [U,top_k] float32 numpy); ties
         are broken by candidate order (the order of `item_features`), as a stable sort would.
-        Uses the current F1-selected weights (fusion_weights())."""
+        Uses the current F1-selected weights (fusion_weights()).
+
+        exclude: optional DataFrame with userId / itemId columns (e.g. the training ratings): each user's list
+        leaves those items out and is filled with the next best (padded with -1 / -inf when fewer than top_k
+        candidates remain).  The min-max scaling still spans all candidates, so a kept item's score is the one it
+        has without `exclude`.  Pairs whose user is not in user_ids or whose item is not a candidate are ignored."""
         import torch
         from .scoring import HybridScorer
         if not self.models_loaded:
@@ -154,23 +172,26 @@ class HybridRecommendationSystem:
         It = self.twotower_model.item_vectors(item_features)
         w_als, w_tt = self.fusion_weights()
         item_ids = np.asarray(item_features["itemId"].values)
+        excl = self._exclusion(exclude, user_ids, item_ids, dev)
         out_i, out_s = [], []
         sc = HybridScorer(Ua, Ia, Ut, It)       # one scorer (items, workspace) for every slab of users
         for u0 in range(0, len(urows), user_chunk):
             u1 = min(len(urows), u0 + user_chunk)
-            idx, s = sc.recommend(top_k, w_als, w_tt, u0, u1)
+            idx, s = sc.recommend(top_k, w_als, w_tt, u0, u1, exclude=excl)
             out_i.append(idx.cpu().numpy())
             out_s.append(s.cpu().numpy())
         idx = np.concatenate(out_i)
         return np.where(idx >= 0, item_ids[np.maximum(idx, 0)], -1), np.concatenate(out_s)
 
-    def evaluate_models_batch(self, user_ids, actual_ratings_by_user, item_features, k=10, user_chunk=65536):
+    def evaluate_models_batch(self, user_ids, actual_ratings_by_user, item_features, k=10, user_chunk=65536, *,
+                              exclude=None):
         """evaluate_individual_models (hybrid_system.py:42-55) for many users at once: each model's top-k by its own
         score (the fused scoring kernels with weights (1,0) / (0,1): min-max scaling does not change a model's order)
         and F1@k against the users' rated items (hals_f1_at_k).  actual_ratings_by_user: per user a dict / iterable of
         rated item ids (the keys of the reference's `actual_ratings`).  Returns (als_f1, tt_f1) float32 numpy [U];
         the sticky scalars als_f1_score / twotower_f1_score are set to the LAST user's values, which is what a loop
-        over evaluate_individual_models leaves behind."""
+        over evaluate_individual_models leaves behind.  exclude: as for recommend_batch (e.g. the training ratings,
+        so that held-out items are scored against lists without the items the models were fitted on)."""
         import torch
         from .evaluation import f1_at_k_batch
         from .scoring import HybridScorer
@@ -197,11 +218,12 @@ class HybridRecommendationSystem:
             return np.concatenate([order[pos[ok]], extra]).astype(np.int32)
 
         actual = [cand_rows(a.keys() if hasattr(a, "keys") else a) for a in actual_ratings_by_user]
+        excl = self._exclusion(exclude, user_ids, cand_ids, dev)
         f_als, f_tt = [], []
         for u0 in range(0, len(urows), user_chunk):
             u1 = min(len(urows), u0 + user_chunk)
-            ia, _ = sc.recommend(k, 1.0, 0.0, u0, u1)
-            it, _ = sc.recommend(k, 0.0, 1.0, u0, u1)
+            ia, _ = sc.recommend(k, 1.0, 0.0, u0, u1, exclude=excl)
+            it, _ = sc.recommend(k, 0.0, 1.0, u0, u1, exclude=excl)
             f_als.append(f1_at_k_batch(ia, actual[u0:u1], k).cpu().numpy())
             f_tt.append(f1_at_k_batch(it, actual[u0:u1], k).cpu().numpy())
         f_als, f_tt = np.concatenate(f_als), np.concatenate(f_tt)

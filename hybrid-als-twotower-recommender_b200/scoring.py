@@ -68,6 +68,39 @@ def reduce_extrema(ex, world: int):
     return ex * sign
 
 
+def exclusion_lists(user_pos: torch.Tensor, item_pos: torch.Tensor, n_users: int):
+    """(call row, global item index) pairs -> the exclusion CSR of hals_score_blend_topk_excluding:
+    (rowptr int64 [n_users+1], items int32, ascending within a row; duplicates kept), on the pairs' device.
+    Sorting by item first (stably) makes build_csr's stable grouping by row yield ascending rows."""
+    from .csr import build_csr
+    user_pos, item_pos = user_pos.reshape(-1).to(torch.int64), item_pos.reshape(-1).to(torch.int64)
+    order = torch.sort(item_pos, stable=True).indices
+    sh = build_csr(user_pos[order], item_pos[order], None, int(n_users))
+    return sh.rowptr, sh.colidx
+
+
+def _matches(ids: torch.Tensor, query: torch.Tensor):
+    """Every (q, p) with ids[p] == query[q] (ids may repeat), by a sort of `ids` and two binary searches."""
+    s, order = torch.sort(ids, stable=True)
+    lo = torch.searchsorted(s, query, side="left")
+    n = torch.searchsorted(s, query, side="right") - lo
+    q = torch.repeat_interleave(torch.arange(query.numel(), device=query.device), n)
+    first = torch.cumsum(n, 0) - n
+    p = order[lo[q] + torch.arange(q.numel(), device=query.device) - first[q]]
+    return q, p
+
+
+def exclusion_lists_by_id(user_ids: torch.Tensor, item_ids: torch.Tensor, pair_users: torch.Tensor,
+                          pair_items: torch.Tensor):
+    """Exclusion CSR over the rows of a call from (raw user id, raw item id) pairs: row r = the call's r-th user
+    (user_ids[r]), item = the position of the item among the call's candidates (item_ids).  A pair whose user is not
+    a row or whose item is not a candidate is ignored; a user id listed twice gets its exclusions in both rows (and a
+    candidate id listed twice is excluded at both positions)."""
+    q, rows = _matches(user_ids.reshape(-1), pair_users.reshape(-1))
+    q2, cols = _matches(item_ids.reshape(-1), pair_items.reshape(-1)[q])
+    return exclusion_lists(rows[q2], cols, user_ids.numel())
+
+
 def shard_items(n_items: int, rank: int, world: int):
     """Contiguous equal item shards (item-sharded scoring): [begin, end) of this rank."""
     per = (n_items + world - 1) // world
@@ -121,27 +154,41 @@ class HybridScorer:
         ex = reduce_extrema(ex, self.world)
         return ex
 
-    def topk_local(self, extrema, k, w_als, w_tt, u0=0, u1=None):
-        """Top-k of this item shard only (global item numbering via item_offset)."""
+    def topk_local(self, extrema, k, w_als, w_tt, u0=0, u1=None, exclude=None):
+        """Top-k of this item shard only (global item numbering via item_offset).  exclude: optional (rowptr, items)
+        exclusion CSR over ALL of the scorer's users (see exclusion_lists; global item numbering, so every shard takes
+        the same lists): the items of a user's row are left out of its list (hals_score_blend_topk_excluding)."""
         L = nat.lib()
         u1 = self.n_users if u1 is None else u1
         n = u1 - u0
         self._workspace(n, k)
         idx = torch.empty((n, k), dtype=torch.int32, device=self.device)
         sc = torch.empty((n, k), dtype=torch.float32, device=self.device)
-        nat.check(L.hals_score_blend_topk(*self._ops(u0, u1), n, self.n_items, nat.ptr(extrema), float(w_als),
-                                          float(w_tt), int(k), self.item_offset, nat.ptr(idx), nat.ptr(sc),
-                                          nat.ptr(self._ws), self._ws.numel(), nat.current_stream()),
-                  "hals_score_blend_topk")
+        head = (*self._ops(u0, u1), n, self.n_items, nat.ptr(extrema), float(w_als), float(w_tt), int(k),
+                self.item_offset, nat.ptr(idx), nat.ptr(sc))
+        tail = (nat.ptr(self._ws), self._ws.numel(), nat.current_stream())
+        if exclude is None:
+            nat.check(L.hals_score_blend_topk(*head, *tail), "hals_score_blend_topk")
+        else:
+            rowptr, items = exclude
+            if rowptr.dtype != torch.int64 or items.dtype != torch.int32 or rowptr.numel() != self.n_users + 1:
+                raise ValueError("exclude must be (rowptr int64 [n_users+1], items int32) over the scorer's users")
+            if rowptr.device != self.device or items.device != self.device:
+                raise ValueError("exclude must live on the scorer's device")
+            rowptr, items = rowptr.contiguous(), items.contiguous()
+            if items.numel() == 0:            # a valid pointer for an empty list set
+                items = torch.zeros(1, dtype=torch.int32, device=self.device)
+            nat.check(L.hals_score_blend_topk_excluding(*head, nat.ptr(rowptr[u0:]), nat.ptr(items), *tail),
+                      "hals_score_blend_topk_excluding")
         return idx, sc
 
-    def recommend(self, k: int, w_als: float, w_tt: float, u0: int = 0, u1: int | None = None):
+    def recommend(self, k: int, w_als: float, w_tt: float, u0: int = 0, u1: int | None = None, exclude=None):
         """Final top-k for users [u0,u1).  Item-sharded runs return, on every rank, the merged
         lists of ITS slice of those users (rank r owns the r-th equal chunk) -- see
-        `user_slice`."""
+        `user_slice`.  exclude: as for topk_local."""
         u1 = self.n_users if u1 is None else u1
         ex = self.extrema(u0, u1)
-        idx, sc = self.topk_local(ex, k, w_als, w_tt, u0, u1)
+        idx, sc = self.topk_local(ex, k, w_als, w_tt, u0, u1, exclude=exclude)
         return exchange_topk(idx, sc, self.rank, self.world, merge_lists)
 
     def user_slice(self, u0, u1):

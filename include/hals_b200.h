@@ -262,6 +262,23 @@ int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const float* Ia, i
                           int topk, int32_t item_offset, int32_t* out_idx /* [n_users,topk] */,
                           float* out_score /* [n_users,topk] */, void* workspace,
                           size_t workspace_bytes, void* stream);
+/* hals_score_blend_topk with a per-user exclusion set X_u (e.g. the items the user already rated), as a CSR:
+ * X_u = excl_items[excl_rowptr[u] .. excl_rowptr[u+1]), u = 0 .. n_users-1 the rows of this call.  excl_rowptr values
+ * are absolute offsets into excl_items, so rows [u0, u1) of a larger CSR are passed as excl_rowptr + u0.  Ids use the
+ * call's global numbering (local index + item_offset), ascending within a row; duplicates are allowed, and ids outside
+ * [item_offset, item_offset + n_items) are ignored (every shard of an item-sharded run can receive the same lists).
+ *   - the result is the first topk items i not in X_u in the usual order (blend descending, then lower index), padded
+ *     with -1 / -inf when fewer remain: the reference's `combined` with X_u removed before sorted(...)[:top_k];
+ *   - the blend still uses the extrema over ALL items (hals_score_extrema is unchanged), so a kept item's score is
+ *     bit-identical to its score in the call without exclusions;
+ *   - both pointers NULL: exactly hals_score_blend_topk; only one NULL: HALS_ERR_INVALID.
+ * Workspace: hals_score_workspace_bytes, as for hals_score_blend_topk. */
+int hals_score_blend_topk_excluding(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride,
+                                    int ka, const float* Ut, int64_t ut_stride, const float* It,
+                                    int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
+                                    const float* extrema, float w_als, float w_tt, int topk, int32_t item_offset,
+                                    int32_t* out_idx, float* out_score, const int64_t* excl_rowptr /* [n_users+1] */,
+                                    const int32_t* excl_items, void* workspace, size_t workspace_bytes, void* stream);
 
 int hals_topk_merge(const int32_t* part_idx, const float* part_score, int n_parts,
                     int64_t n_users, int topk, int32_t* out_idx, float* out_score, void* stream);
