@@ -11,7 +11,7 @@ import pytest
 import torch
 
 from oracle import als_oracle, c_oracle
-from tests.util import rel_l2
+from tests.util import assert_ran, draw_ratings, launched_kernels, rel_l2
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(__file__), "golden")
@@ -28,14 +28,25 @@ def _mods():
     return als_engine, csr
 
 
-def gpu_half_step(rows, cols, vals, n_rows, src, reg, implicit=False, alpha=1.0, seg_len=None):
+def gpu_half_step(rows, cols, vals, n_rows, src, reg, implicit=False, alpha=1.0, seg_len=None, packed=True,
+                  plan_implicit=None, src_offset=0):
+    """One hals_als_half_step.  packed=False clears the plan's packed ratings (ranks 64 / 128: the round-1 kernels
+    that split the fp32 ratings themselves); plan_implicit=False with implicit=True calls implicit mode with a plan
+    built for explicit feedback (the CUDA-core kernel at every rank); src_offset > 0 places the source factors that
+    many floats into a larger buffer (not 16-byte aligned: the CUDA-core kernel's scalar gather; CUDA-core ranks only,
+    the tensor-core kernels and the rank-64 / 128 Gram assume aligned rows)."""
     als_engine, csr = _mods()
     dev = torch.device("cuda")
     shard = csr.build_csr(torch.as_tensor(rows).to(dev), torch.as_tensor(cols).to(dev),
                           torch.as_tensor(vals).to(dev), n_rows)
     k = src.shape[1]
-    plan = csr.AlsPlanHandle(shard, k, seg_len, n_src=src.shape[0], implicit=implicit, alpha=alpha)
-    s = torch.from_numpy(np.ascontiguousarray(src)).to(dev)
+    plan_implicit = implicit if plan_implicit is None else plan_implicit
+    plan = csr.AlsPlanHandle(shard, k, seg_len, n_src=src.shape[0], implicit=plan_implicit, alpha=alpha)
+    if not packed:
+        plan.struct.vals_hl = None
+    buf = torch.empty(src.size + src_offset, dtype=torch.float32, device=dev)
+    s = buf[src_offset:].view(src.shape)
+    s.copy_(torch.from_numpy(np.ascontiguousarray(src)))
     dst = torch.full((n_rows, k), 7.0, dtype=torch.float32, device=dev)   # poison: rows must be overwritten
     gram = None
     if implicit:
@@ -64,47 +75,66 @@ def synth(U, I, nnz, seed, skew=False):
     return u, i, r
 
 
-def assert_close(got, want, rel=HS_REL, ab=HS_ABS):
+def assert_close(got, want, rel=HS_REL, ab=HS_ABS, floor=1.0):
+    """rel-L2 <= rel and max-abs <= ab * max(floor, max|want|); floor=0 makes both bounds purely relative."""
     assert np.isfinite(got).all()
     assert rel_l2(got, want) <= rel, rel_l2(got, want)
-    assert np.abs(got - want).max() <= ab * max(1.0, np.abs(want).max()), np.abs(got - want).max()
+    assert np.abs(got - want).max() <= ab * max(floor, np.abs(want).max()), np.abs(got - want).max()
 
 
-@pytest.mark.parametrize("k", [2, 10, 16, 20, 32, 50, 64, 100, 128])
+def half_step_kernel(k, implicit, aligned=True):
+    """Name (as launched_kernels reports it) of the main kernel hals_als_half_step runs for a default plan."""
+    if k in (64, 128):
+        return f"als_ws{k}_kernel"
+    kp = 16 if k <= 16 else 32 if k <= 32 else 64 if k <= 64 else 128
+    vec = k % 4 == 0 and aligned
+    return f"als_build_solve_kernel<{kp},{str(implicit).lower()},{str(vec).lower()}>"
+
+
+# odd ranks take the scalar gather; 33 / 127 sit one past / one below a padded-rank bucket
+@pytest.mark.parametrize("k", [1, 2, 3, 10, 16, 20, 32, 33, 50, 64, 100, 127, 128])
 def test_half_step_explicit_matches_oracle(k):
     U, I, nnz = 700, 300, 9000
     u, i, r = synth(U, I, nnz, k)
     X = als_oracle.init_factors(U, k, 1)
-    got, _ = gpu_half_step(i, u, r, I, X, 0.1)
+    with launched_kernels() as names:
+        got, _ = gpu_half_step(i, u, r, I, X, 0.1)
+    assert_ran(names, half_step_kernel(k, False))
     rp, ci, v = als_oracle.coo_to_csr(i, u, r, I)
     assert_close(got, c_oracle.als_half_step(rp, ci, v, X, 0.1))
 
 
-@pytest.mark.parametrize("k", [10, 64, 128])
+# 16 / 32 / 100: the vectorised-gather implicit instantiations at padded ranks 16, 32 and 128
+@pytest.mark.parametrize("k", [10, 16, 32, 64, 100, 128])
 def test_half_step_implicit_matches_oracle(k):
     U, I, nnz = 500, 260, 6000
     rng = np.random.default_rng(k)
     u, i = rng.integers(0, U, nnz), rng.integers(0, I, nnz)
     r = (rng.geometric(0.4, nnz) * rng.choice([1, 1, 1, -1, 0], nnz)).astype(np.float32)
     X = als_oracle.init_factors(U, k, 3)
-    got, _ = gpu_half_step(i, u, r, I, X, 0.05, implicit=True, alpha=40.0)
+    with launched_kernels() as names:
+        got, _ = gpu_half_step(i, u, r, I, X, 0.05, implicit=True, alpha=40.0)
+    assert_ran(names, half_step_kernel(k, True))
     rp, ci, v = als_oracle.coo_to_csr(i, u, r, I)
     want = c_oracle.als_half_step(rp, ci, v, X, 0.05, implicit=True, alpha=40.0)
     assert_close(got, want, **IMPL_TOL[k in (64, 128)])
 
 
-@pytest.mark.parametrize("k", [64, 128])
+@pytest.mark.parametrize("k", [10, 20, 64, 100, 128])
 def test_implicit_long_rows_and_mixed_signs(k):
-    """Implicit feedback with sliced rows (rank 128: tensor-core build with rows rescaled by sqrt(c), Gram added in the
-    solver / the long-row reduce; rank 64: CUDA-core kernel), ratings of both signs, zeros and non-integer weights."""
+    """Implicit feedback with sliced rows, ratings of both signs, zeros and non-integer weights.  Ranks 64 / 128: the
+    tensor-core build with rows rescaled by sqrt(c), the Gram added in the solver / the long-row reduce; other ranks:
+    the CUDA-core kernel, whose long-row reduce (als_reduce_solve_kernel) adds the Gram."""
     U, I, nnz = 2500, 60, 24000
     rng = np.random.default_rng(11)
     p = 1.0 / np.arange(1, I + 1); p /= p.sum()
     i, u = rng.choice(I, nnz, p=p), rng.integers(0, U, nnz)
     r = (rng.gamma(1.5, 2.0, nnz) * rng.choice([1, 1, 1, -1, 0], nnz)).astype(np.float32)
     X = als_oracle.init_factors(U, k, 4)
-    got, plan = gpu_half_step(i, u, r, I, X, 0.05, implicit=True, alpha=15.0, seg_len=96)
+    with launched_kernels() as names:
+        got, plan = gpu_half_step(i, u, r, I, X, 0.05, implicit=True, alpha=15.0, seg_len=96)
     assert plan.n_long > 0
+    assert_ran(names, half_step_kernel(k, True), *(() if k in (64, 128) else ("als_reduce_solve_kernel<",)))
     rp, ci, v = als_oracle.coo_to_csr(i, u, r, I)
     want = c_oracle.als_half_step(rp, ci, v, X, 0.05, implicit=True, alpha=15.0)
     assert_close(got, want, **IMPL_TOL[k in (64, 128)])
@@ -186,15 +216,19 @@ def test_config1_amazon_shape_rank10_10_iters():
     assert abs(eng.rmse(u, i, r) - als_oracle.rmse(Xo, Yo, u, i, r)) <= 1e-4
 
 
+@pytest.mark.parametrize("kind", ["int", "decimal"])
 @pytest.mark.parametrize("k", [64, 128])
-def test_fit_10_sweeps_on_the_tensor_core_ranks(k):
+def test_fit_10_sweeps_on_the_tensor_core_ranks(k, kind):
     """Ten full sweeps through the tcgen05 kernels (rank 64: warp-specialised kernel; rank 128) on a Zipf-skewed shape
-    with sliced long rows, against the fp64-accumulating C oracle from identical initial factors.
+    with sliced long rows, against the fp64-accumulating C oracle from identical initial factors.  Decimal ratings are
+    mostly not bf16 numbers: they exercise the low rating part of the engine's split-form half-steps and the RMSE.
     Tolerance (north star: "factors and RMSE within a stated fp32 tolerance"): rel-L2 <= 1e-3 on both factor
     matrices, |RMSE difference| <= 1e-4.  (Parity unpinned: the oracle restates Spark MLlib 3.5.1, SURVEY App. A.)"""
     als_engine, _ = _mods()
     U, I, nnz = 6000, 900, 240_000
     u, i, r = synth(U, I, nnz, 21 + k, skew=True)
+    if kind != "int":
+        r = draw_ratings(kind, nnz, np.random.default_rng(k))
     X0 = als_oracle.init_factors(U, k, 5)
     Xo, Yo = als_oracle.als_fit(u, i, r, U, I, k, 10, 0.1, X0, half_step=c_oracle.als_half_step)
     eng = als_engine.AlsEngine(u, i, r, U, I, k, 0.1, seg_len=1024)
@@ -215,20 +249,12 @@ def test_fit_10_sweeps_on_the_tensor_core_ranks(k):
 def test_rank64_kernels_agree():
     """The warp-specialised rank-64 kernel (default) and the round-1 kernel (plan without chunk table / packed ratings)
     build the same normal equations and must agree to solver rounding."""
-    als_engine, csr = _mods()
     U, I, nnz = 3000, 500, 90_000
     u, i, r = synth(U, I, nnz, 77, skew=True)
     X = als_oracle.init_factors(U, 64, 2)
-    got, plan = gpu_half_step(i, u, r, I, X, 0.1, seg_len=512)
-    dev = torch.device("cuda")
-    shard = csr.build_csr(torch.as_tensor(i).to(dev), torch.as_tensor(u).to(dev), torch.as_tensor(r).to(dev), I)
-    plan2 = csr.AlsPlanHandle(shard, 64, 512, n_src=U)
-    plan2.struct.vals_hl = None                        # -> als_tc64_kernel
-    s = torch.from_numpy(X).to(dev)
-    dst = torch.full((I, 64), 7.0, dtype=torch.float32, device=dev)
-    als_engine.native_half_step(shard, plan2, s, dst, 64, 0.1, False, 1.0, None)
-    torch.cuda.synchronize()
-    assert rel_l2(dst.cpu().numpy(), got) <= 5e-6
+    got, _ = gpu_half_step(i, u, r, I, X, 0.1, seg_len=512)
+    old, _ = gpu_half_step(i, u, r, I, X, 0.1, seg_len=512, packed=False)     # -> als_tc64_kernel
+    assert rel_l2(old, got) <= 5e-6
 
 
 @pytest.mark.parametrize("k", [64, 128])
