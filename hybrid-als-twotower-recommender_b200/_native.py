@@ -63,6 +63,9 @@ SIGNATURES = {
     "hals_als_plan_count_positive": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "hals_als_half_step": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, ctypes.c_int, c_f32,
                                           ctypes.c_int, c_f32, c_vp, ctypes.POINTER(AlsPlan), c_vp, c_sz, c_vp]),
+    "hals_als_half_step_nonnegative": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, ctypes.c_int, c_f32,
+                                                      ctypes.c_int, c_f32, c_vp, ctypes.POINTER(AlsPlan), c_vp, c_sz,
+                                                      c_vp, c_vp]),
     "hals_als_split_factors": (ctypes.c_int, [c_vp, c_i64, ctypes.c_int, c_vp, c_vp]),
     "hals_als_half_step_split": (ctypes.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, ctypes.c_int, c_f32, ctypes.POINTER(AlsPlan), c_vp,
                                                   c_sz, c_vp]),

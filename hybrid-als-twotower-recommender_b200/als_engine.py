@@ -4,7 +4,8 @@ One process per GPU.  Rank r owns an nnz-balanced contiguous range of user rows 
 of item rows of R^T (CSR shards resident in HBM) plus full replicas of both factor
 matrices.  A sweep is   item half-step -> all-gather(Y) -> user half-step -> all-gather(X)
 (Spark's loop order; ALS.scala train).  The half-step itself is one C-ABI call
-(hals_als_half_step); the all-gather is NCCL through torch.distributed.
+(hals_als_half_step, or hals_als_half_step_nonnegative for Spark's nonnegative=True); the all-gather is NCCL through
+torch.distributed.
 """
 from __future__ import annotations
 
@@ -77,11 +78,21 @@ def route_to_owners(users, items, ratings, key, bounds, world: int):
 
 
 def native_half_step(shard: CsrShard, plan: AlsPlanHandle, src: torch.Tensor, dst_full: torch.Tensor,
-                     k: int, reg: float, implicit: bool, alpha: float, gram: torch.Tensor | None):
-    """dst_full[row_begin:row_end] = solve(shard, src).  The only compute path (CUDA)."""
+                     k: int, reg: float, implicit: bool, alpha: float, gram: torch.Tensor | None,
+                     nonnegative: bool = False, n_capped: torch.Tensor | None = None):
+    """dst_full[row_begin:row_end] = solve(shard, src).  The only compute path (CUDA).  nonnegative=True: the
+    bound-constrained solve (x >= 0); rows that reach its iteration cap are added to n_capped (int32 [1], optional)."""
     L = nat.lib()
     dst = dst_full[shard.row_begin: shard.row_end]
     assert src.is_contiguous() and dst.is_contiguous() and src.dtype == torch.float32
+    if nonnegative:
+        assert n_capped is None or (n_capped.dtype == torch.int32 and n_capped.device == dst.device)
+        nat.check(L.hals_als_half_step_nonnegative(
+            nat.ptr(shard.rowptr), nat.ptr(shard.colidx), nat.ptr(shard.vals), shard.n_rows,
+            nat.ptr(src), src.shape[0], nat.ptr(dst), k, float(reg), int(bool(implicit)), float(alpha),
+            nat.ptr(gram) if gram is not None else None, plan.struct, nat.ptr(plan.workspace),
+            plan.workspace_bytes, nat.current_stream(), nat.ptr(n_capped)), "hals_als_half_step_nonnegative")
+        return
     nat.check(L.hals_als_half_step(
         nat.ptr(shard.rowptr), nat.ptr(shard.colidx), nat.ptr(shard.vals), shard.n_rows,
         nat.ptr(src), src.shape[0], nat.ptr(dst), k, float(reg), int(bool(implicit)), float(alpha),
@@ -151,12 +162,15 @@ class AlsEngine:
     def __init__(self, users, items, ratings, n_users: int, n_items: int, rank: int, reg: float,
                  implicit: bool = False, alpha: float = 1.0, device=None, seg_len: int | None = None,
                  dist_rank: int = 0, world: int = 1, half_step=None, make_plans: bool = True,
-                 partitioned: bool = False):
+                 partitioned: bool = False, nonnegative: bool = False):
         """users / items / ratings: the COO triples.  partitioned=False: every rank passes the WHOLE matrix and keeps
         its row shards.  partitioned=True (world > 1): every rank passes only ITS slice of the triples (rank q the q-th
         contiguous chunk, so that the concatenation over ranks is the original order); row counts are all-reduced
         and the triples are routed to the owner of their user row (for R) and of their item row (for R^T) with one
-        all-to-all each -- 1/N of the upload and of the sort per rank."""
+        all-to-all each -- 1/N of the upload and of the sort per rank.
+        nonnegative=True: Spark's nonnegative=True, every factor row is the nonnegative least-squares solution of its
+        normal equations (hals_als_half_step_nonnegative, fp32 factors only -- no split form).  An injected half_step
+        then receives nonnegative=True as a keyword."""
         import os
         import time
         _t = [time.perf_counter()]
@@ -170,6 +184,7 @@ class AlsEngine:
                     print(f"[als_engine] {what}: {(now - _t[0]) * 1e3:.2f} ms", flush=True)
                 _t[0] = now
         self.k, self.reg, self.implicit, self.alpha = int(rank), float(reg), bool(implicit), float(alpha)
+        self.nonnegative = bool(nonnegative)
         self.n_users, self.n_items = int(n_users), int(n_items)
         self.rank, self.world = dist_rank, world
         self.device = torch.device(device) if device is not None else torch.device("cuda")
@@ -218,13 +233,17 @@ class AlsEngine:
         # exchange the split rows in place and the fp32 replicas of the OTHER ranks' rows are refreshed lazily
         self.split = None
         self._fp32_stale = False
-        if (self.k in (64, 128) and not self.implicit and self.device.type == "cuda" and self._half_step is native_half_step
-                and make_plans):
+        if (self.k in (64, 128) and not self.implicit and not self.nonnegative and self.device.type == "cuda"
+                and self._half_step is native_half_step and make_plans):
             self.split = {"X": SplitFactors(self.user_bounds, world, self.device, self.k),
                           "Y": SplitFactors(self.item_bounds, world, self.device, self.k)}
             self.colidx_pad_R = self.split["Y"].pad_of[self.R.colidx.long()].to(torch.int32) if world > 1 else self.R.colidx
             self.colidx_pad_Rt = self.split["X"].pad_of[self.Rt.colidx.long()].to(torch.int32) if world > 1 else self.Rt.colidx
         _mark("factor buffers + column remap")
+        # rows of nonnegative half-steps that reached the solver's iteration cap, summed by the kernels
+        self._n_capped = None
+        if self.nonnegative and self.device.type == "cuda" and self._half_step is native_half_step:
+            self._n_capped = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._gather_cache = {}
         self._graphs = None                # (item, user) CUDA graphs after enable_graphs()
         self._graph_launch_counts = (0, 0)
@@ -258,6 +277,20 @@ class AlsEngine:
         self.X.copy_(f)
         self._after_user_init()
 
+    def nonneg_capped_rows(self) -> int:
+        """Rows, over every nonnegative half-step this engine ran, whose NNLS solve reached its iteration cap (each
+        keeps its last iterate with x >= 0).  0 when nonnegative=False."""
+        return 0 if self._n_capped is None else int(self._n_capped.item())
+
+    def _solve(self, shard, plan, src, dst, gram):
+        if not self.nonnegative:
+            self._half_step(shard, plan, src, dst, self.k, self.reg, self.implicit, self.alpha, gram)
+        elif self._half_step is native_half_step:
+            native_half_step(shard, plan, src, dst, self.k, self.reg, self.implicit, self.alpha, gram,
+                             nonnegative=True, n_capped=self._n_capped)
+        else:   # injected half-step (CPU tests): told only when the option is set, so plain callables keep working
+            self._half_step(shard, plan, src, dst, self.k, self.reg, self.implicit, self.alpha, gram, nonnegative=True)
+
     def _gram_of(self, src):
         if not self.implicit:
             return None
@@ -275,8 +308,7 @@ class AlsEngine:
             self.split["Y"].all_gather(self.rank)
             self._fp32_stale = self.world > 1
             return
-        self._half_step(self.Rt, self.plan_Rt, self.X, self.Y, self.k, self.reg, self.implicit, self.alpha,
-                        self._gram_of(self.X))
+        self._solve(self.Rt, self.plan_Rt, self.X, self.Y, self._gram_of(self.X))
         all_gather_rows(self.Y, self.item_bounds, self.rank, self.world, cache=self._gather_cache)
 
     def _user_half_eager(self):
@@ -286,8 +318,7 @@ class AlsEngine:
             self.split["X"].all_gather(self.rank)
             self._fp32_stale = self.world > 1
             return
-        self._half_step(self.R, self.plan_R, self.Y, self.X, self.k, self.reg, self.implicit, self.alpha,
-                        self._gram_of(self.Y))
+        self._solve(self.R, self.plan_R, self.Y, self.X, self._gram_of(self.Y))
         all_gather_rows(self.X, self.user_bounds, self.rank, self.world, cache=self._gather_cache)
 
     def sync_factors(self):
@@ -323,7 +354,7 @@ class AlsEngine:
             return True
         if self.device.type != "cuda" or self._half_step is not native_half_step or self.plan_R is None:
             return False
-        keep = (self.X.clone(), self.Y.clone())
+        keep = (self.X.clone(), self.Y.clone(), None if self._n_capped is None else self._n_capped.clone())
         keep_split = None if self.split is None else (self.split["X"].hl.clone(), self.split["Y"].hl.clone(), self._fp32_stale)
         try:
             side = torch.cuda.Stream(self.device)
@@ -349,6 +380,8 @@ class AlsEngine:
             torch.cuda.synchronize(self.device)
         self.X.copy_(keep[0])
         self.Y.copy_(keep[1])
+        if keep[2] is not None:          # the warm-up half-steps do not count
+            self._n_capped.copy_(keep[2])
         if keep_split is not None:
             self.split["X"].hl.copy_(keep_split[0])
             self.split["Y"].hl.copy_(keep_split[1])

@@ -8,6 +8,7 @@ libhals_b200.so (csrc/), driven by als_engine.AlsEngine.
 
 Additive (keyword-only) extensions, none of which changes the reference behaviour:
   ALSModel(..., implicit_prefs=False, alpha=1.0, seed=0)   Spark's implicitPrefs / alpha / seed
+  ALSModel(..., nonnegative=False)                         Spark's nonnegative: factors >= 0 (NNLS half-steps)
   train(data, init_user_factors=None)                      explicit initial factors for parity runs
   predict_for_users(user_ids, item_ids)                    dense [U,I] block of scores (device)
 """
@@ -108,7 +109,7 @@ def _as_item_ids(all_items):
 
 class ALSModel:
     def __init__(self, rank=10, max_iter=10, reg_param=0.1, cold_start_strategy="drop", *,
-                 implicit_prefs=False, alpha=1.0, seed=0):
+                 implicit_prefs=False, alpha=1.0, seed=0, nonnegative=False):
         self.rank = rank
         self.max_iter = max_iter
         self.reg_param = reg_param
@@ -122,6 +123,7 @@ class ALSModel:
         self.implicit_prefs = implicit_prefs
         self.alpha = alpha
         self.seed = seed
+        self.nonnegative = nonnegative
 
     @property
     def item_features(self):
@@ -165,7 +167,7 @@ class ALSModel:
             item_ids_d, i = torch.unique(iid, sorted=True, return_inverse=True)
             user_ids, item_ids = user_ids_d.cpu().numpy(), item_ids_d.cpu().numpy()
             eng = AlsEngine(u, i, r, len(user_ids), len(item_ids), self.rank, self.reg_param,
-                            implicit=self.implicit_prefs, alpha=self.alpha)
+                            implicit=self.implicit_prefs, alpha=self.alpha, nonnegative=self.nonnegative)
             if init_user_factors is not None:
                 eng.set_user_factors(init_user_factors)
             else:

@@ -13,27 +13,31 @@
 //     hand side carried as an extra row so the forward substitution is free) and the
 //     solution is written straight to the destination factor row;
 //   * slices of long rows write their partial (A, b, n) to the workspace; a second
-//     kernel sums the slots in slot order (deterministic) and solves.
+//     kernel sums the slots in slot order (deterministic) and solves;
+//   * nonnegative factors (Spark's nonnegative=True): the *_nnls_kernel instantiations replace the
+//     Cholesky solve by the block-principal-pivoting NNLS of als_common.cuh, same build and reduce.
 // This path is the correctness baseline and the fallback for ranks the tensor-core path
 // (als_tc.cu) does not cover.
 #include "als_common.cuh"
 
 namespace hals {
 
-template <int KP, bool IMPLICIT, bool VEC>
-__global__ void __launch_bounds__(kAlsThreads)
-als_build_solve_kernel(const int32_t* __restrict__ colidx, const float* __restrict__ vals,
-                       const float* __restrict__ src, float* __restrict__ dst, int k, float reg,
-                       float alpha, const float* __restrict__ gram,
-                       const int32_t* __restrict__ item_row, const int64_t* __restrict__ item_begin,
-                       const int32_t* __restrict__ item_len, const int32_t* __restrict__ item_slot,
-                       float* __restrict__ workspace) {
+// Body of the build kernels.  tid = threadIdx.x is read in the kernel itself, where its range is known (the plain
+// kernels compile to the same code as before the body was shared).  NONNEG: solve with nnls_solve_smem (x >= 0) instead
+// of cholesky_solve_smem; rows that reach its iteration cap are counted in *n_capped (optional).
+template <int KP, bool IMPLICIT, bool VEC, bool NONNEG>
+__device__ __forceinline__ void
+als_build_solve(const int32_t* __restrict__ colidx, const float* __restrict__ vals,
+                const float* __restrict__ src, float* __restrict__ dst, int k, float reg,
+                float alpha, const float* __restrict__ gram,
+                const int32_t* __restrict__ item_row, const int64_t* __restrict__ item_begin,
+                const int32_t* __restrict__ item_len, const int32_t* __restrict__ item_slot,
+                float* __restrict__ workspace, int32_t* __restrict__ n_capped, const int tid) {
   using TL = AlsTile<KP>;
   constexpr int TM = TL::TM, V = TL::V, NG = TL::NG, LD = TL::LD, T = kAlsChunk;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   AlsSmem<KP>& sm = *reinterpret_cast<AlsSmem<KP>*>(smem_raw);
 
-  const int tid = threadIdx.x;
   const int tx = tid & 15, ty = tid >> 4;
   const int item = blockIdx.x;
   const int row = item_row[item];
@@ -189,17 +193,52 @@ als_build_solve_kernel(const int32_t* __restrict__ colidx, const float* __restri
   }
   if (tid < k) S[tid * LD + tid] += lam;
   __syncthreads();
+  if (NONNEG) {
+    // the gather buffers are idle now: they hold the solver's scratch
+    static_assert(sizeof(NnlsScratch<KP>) <= sizeof(sm.G), "NNLS scratch must fit the gather buffers");
+    float x;
+    const bool capped = nnls_solve_smem<KP>(S, k, *reinterpret_cast<NnlsScratch<KP>*>(&sm.G[0][0]), x);
+    if (tid < k) dst[(int64_t)row * k + tid] = x;
+    if (capped && tid == 0 && n_capped != nullptr) atomicAdd(n_capped, 1);
+    return;
+  }
   cholesky_solve_smem<KP>(S, k);
   if (tid < k) dst[(int64_t)row * k + tid] = S[KP * LD + tid];
 }
 
-// Long rows: sum the per-slice partials in slot order, add Gram / ridge, solve.
-template <int KP>
+template <int KP, bool IMPLICIT, bool VEC>
 __global__ void __launch_bounds__(kAlsThreads)
-als_reduce_solve_kernel(const float* __restrict__ workspace, float* __restrict__ dst, int k,
-                        float reg, const float* __restrict__ gram,
-                        const int32_t* __restrict__ long_row, const int32_t* __restrict__ long_slot0,
-                        const int32_t* __restrict__ long_nseg) {
+als_build_solve_kernel(const int32_t* __restrict__ colidx, const float* __restrict__ vals,
+                       const float* __restrict__ src, float* __restrict__ dst, int k, float reg,
+                       float alpha, const float* __restrict__ gram,
+                       const int32_t* __restrict__ item_row, const int64_t* __restrict__ item_begin,
+                       const int32_t* __restrict__ item_len, const int32_t* __restrict__ item_slot,
+                       float* __restrict__ workspace) {
+  als_build_solve<KP, IMPLICIT, VEC, false>(colidx, vals, src, dst, k, reg, alpha, gram, item_row, item_begin,
+                                            item_len, item_slot, workspace, nullptr, threadIdx.x);
+}
+
+// The same kernel with the nonnegative solve (a kernel name of its own: profiles tell the two apart).
+template <int KP, bool IMPLICIT, bool VEC>
+__global__ void __launch_bounds__(kAlsThreads)
+als_build_solve_nnls_kernel(const int32_t* __restrict__ colidx, const float* __restrict__ vals,
+                            const float* __restrict__ src, float* __restrict__ dst, int k, float reg,
+                            float alpha, const float* __restrict__ gram,
+                            const int32_t* __restrict__ item_row, const int64_t* __restrict__ item_begin,
+                            const int32_t* __restrict__ item_len, const int32_t* __restrict__ item_slot,
+                            float* __restrict__ workspace, int32_t* __restrict__ n_capped) {
+  als_build_solve<KP, IMPLICIT, VEC, true>(colidx, vals, src, dst, k, reg, alpha, gram, item_row, item_begin,
+                                           item_len, item_slot, workspace, n_capped, threadIdx.x);
+}
+
+// Long rows: sum the per-slice partials in slot order, add Gram / ridge, solve.  NONNEG: the NNLS scratch follows the
+// (KP + 1) x LD system in shared memory.
+template <int KP, bool NONNEG>
+__device__ __forceinline__ void
+als_reduce_solve(const float* __restrict__ workspace, float* __restrict__ dst, int k,
+                 float reg, const float* __restrict__ gram,
+                 const int32_t* __restrict__ long_row, const int32_t* __restrict__ long_slot0,
+                 const int32_t* __restrict__ long_nseg, int32_t* __restrict__ n_capped) {
   constexpr int LD = AlsTile<KP>::LD;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* S = reinterpret_cast<float*>(smem_raw);
@@ -222,14 +261,39 @@ als_reduce_solve_kernel(const float* __restrict__ workspace, float* __restrict__
   __syncthreads();
   if (tid < k) S[tid * LD + tid] += lam;
   __syncthreads();
+  if (NONNEG) {
+    float x;
+    const bool capped = nnls_solve_smem<KP>(S, k, *reinterpret_cast<NnlsScratch<KP>*>(S + als_reduce_system_floats(KP)), x);
+    if (tid < k) dst[(int64_t)row * k + tid] = x;
+    if (capped && tid == 0 && n_capped != nullptr) atomicAdd(n_capped, 1);
+    return;
+  }
   cholesky_solve_smem<KP>(S, k);
   if (tid < k) dst[(int64_t)row * k + tid] = S[KP * LD + tid];
 }
 
 template <int KP>
+__global__ void __launch_bounds__(kAlsThreads)
+als_reduce_solve_kernel(const float* __restrict__ workspace, float* __restrict__ dst, int k,
+                        float reg, const float* __restrict__ gram,
+                        const int32_t* __restrict__ long_row, const int32_t* __restrict__ long_slot0,
+                        const int32_t* __restrict__ long_nseg) {
+  als_reduce_solve<KP, false>(workspace, dst, k, reg, gram, long_row, long_slot0, long_nseg, nullptr);
+}
+
+template <int KP>
+__global__ void __launch_bounds__(kAlsThreads)
+als_reduce_solve_nnls_kernel(const float* __restrict__ workspace, float* __restrict__ dst, int k,
+                             float reg, const float* __restrict__ gram,
+                             const int32_t* __restrict__ long_row, const int32_t* __restrict__ long_slot0,
+                             const int32_t* __restrict__ long_nseg, int32_t* __restrict__ n_capped) {
+  als_reduce_solve<KP, true>(workspace, dst, k, reg, gram, long_row, long_slot0, long_nseg, n_capped);
+}
+
+template <int KP>
 static int launch_simt(const int32_t* colidx, const float* vals, const float* src, float* dst, int k,
                        float reg, int implicit, float alpha, const float* gram,
-                       const hals_als_plan* plan, float* ws, cudaStream_t st) {
+                       const hals_als_plan* plan, float* ws, cudaStream_t st, bool nonneg, int32_t* n_capped) {
   const size_t smem = sizeof(AlsSmem<KP>);
   const bool vec = (k % 4 == 0) && ((reinterpret_cast<uintptr_t>(src) & 15) == 0);
   auto run = [&](auto kern) -> int {
@@ -240,18 +304,40 @@ static int launch_simt(const int32_t* colidx, const float* vals, const float* sr
     HALS_LAUNCH_CHECK();
     return 0;
   };
+  auto run_nn = [&](auto kern) -> int {
+    HALS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)plan->n_items, kAlsThreads, smem, st>>>(
+        colidx, vals, src, dst, k, reg, alpha, gram, plan->item_row, plan->item_begin,
+        plan->item_len, plan->item_slot, ws, n_capped);
+    HALS_LAUNCH_CHECK();
+    return 0;
+  };
   int rc;
-  if (implicit) rc = vec ? run(als_build_solve_kernel<KP, true, true>) : run(als_build_solve_kernel<KP, true, false>);
-  else rc = vec ? run(als_build_solve_kernel<KP, false, true>) : run(als_build_solve_kernel<KP, false, false>);
+  if (nonneg) {
+    if (implicit) rc = vec ? run_nn(als_build_solve_nnls_kernel<KP, true, true>) : run_nn(als_build_solve_nnls_kernel<KP, true, false>);
+    else rc = vec ? run_nn(als_build_solve_nnls_kernel<KP, false, true>) : run_nn(als_build_solve_nnls_kernel<KP, false, false>);
+  } else {
+    if (implicit) rc = vec ? run(als_build_solve_kernel<KP, true, true>) : run(als_build_solve_kernel<KP, true, false>);
+    else rc = vec ? run(als_build_solve_kernel<KP, false, true>) : run(als_build_solve_kernel<KP, false, false>);
+  }
   if (rc) return rc;
-  if (plan->n_long_rows > 0) return als_launch_reduce_solve(ws, dst, k, reg, implicit ? gram : nullptr, plan, st);
+  if (plan->n_long_rows > 0)
+    return als_launch_reduce_solve(ws, dst, k, reg, implicit ? gram : nullptr, plan, st, nonneg, n_capped);
   return 0;
 }
 
 template <int KP>
 static int launch_reduce(const float* ws, float* dst, int k, float reg, const float* gram,
-                         const hals_als_plan* plan, cudaStream_t st) {
+                         const hals_als_plan* plan, cudaStream_t st, bool nonneg, int32_t* n_capped) {
   const size_t smem2 = sizeof(float) * (KP + 1) * AlsTile<KP>::LD;
+  if (nonneg) {
+    const size_t smem3 = sizeof(float) * als_reduce_system_floats(KP) + sizeof(NnlsScratch<KP>);
+    HALS_CUDA(cudaFuncSetAttribute(als_reduce_solve_nnls_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
+    als_reduce_solve_nnls_kernel<KP><<<(unsigned)plan->n_long_rows, kAlsThreads, smem3, st>>>(
+        ws, dst, k, reg, gram, plan->long_row, plan->long_slot0, plan->long_nseg, n_capped);
+    HALS_LAUNCH_CHECK();
+    return 0;
+  }
   HALS_CUDA(cudaFuncSetAttribute(als_reduce_solve_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
   als_reduce_solve_kernel<KP><<<(unsigned)plan->n_long_rows, kAlsThreads, smem2, st>>>(
       ws, dst, k, reg, gram, plan->long_row, plan->long_slot0, plan->long_nseg);
@@ -260,24 +346,24 @@ static int launch_reduce(const float* ws, float* dst, int k, float reg, const fl
 }
 
 int als_launch_reduce_solve(const float* ws, float* dst, int k, float reg, const float* gram,
-                            const hals_als_plan* plan, cudaStream_t st) {
+                            const hals_als_plan* plan, cudaStream_t st, bool nonneg, int32_t* n_capped) {
   if (plan->n_long_rows <= 0) return 0;
   switch (als_padded_rank(k)) {
-    case 16: return launch_reduce<16>(ws, dst, k, reg, gram, plan, st);
-    case 32: return launch_reduce<32>(ws, dst, k, reg, gram, plan, st);
-    case 64: return launch_reduce<64>(ws, dst, k, reg, gram, plan, st);
-    default: return launch_reduce<128>(ws, dst, k, reg, gram, plan, st);
+    case 16: return launch_reduce<16>(ws, dst, k, reg, gram, plan, st, nonneg, n_capped);
+    case 32: return launch_reduce<32>(ws, dst, k, reg, gram, plan, st, nonneg, n_capped);
+    case 64: return launch_reduce<64>(ws, dst, k, reg, gram, plan, st, nonneg, n_capped);
+    default: return launch_reduce<128>(ws, dst, k, reg, gram, plan, st, nonneg, n_capped);
   }
 }
 
 int als_half_step_simt(const int32_t* colidx, const float* vals, const float* src, float* dst, int k,
                        float reg, int implicit, float alpha, const float* gram,
-                       const hals_als_plan* plan, float* ws, cudaStream_t st) {
+                       const hals_als_plan* plan, float* ws, cudaStream_t st, bool nonneg, int32_t* n_capped) {
   switch (als_padded_rank(k)) {
-    case 16: return launch_simt<16>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st);
-    case 32: return launch_simt<32>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st);
-    case 64: return launch_simt<64>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st);
-    default: return launch_simt<128>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st);
+    case 16: return launch_simt<16>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st, nonneg, n_capped);
+    case 32: return launch_simt<32>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st, nonneg, n_capped);
+    case 64: return launch_simt<64>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st, nonneg, n_capped);
+    default: return launch_simt<128>(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, ws, st, nonneg, n_capped);
   }
 }
 

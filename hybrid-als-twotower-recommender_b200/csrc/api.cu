@@ -10,7 +10,7 @@ std::atomic<int64_t> g_launch_count{0};
 
 int als_half_step_simt(const int32_t* colidx, const float* vals, const float* src, float* dst, int k,
                        float reg, int implicit, float alpha, const float* gram,
-                       const hals_als_plan* plan, float* ws, cudaStream_t st);
+                       const hals_als_plan* plan, float* ws, cudaStream_t st, bool nonneg, int32_t* n_capped);
 int als_half_step_tc128(const int32_t* colidx, const float* vals, const float* src, int64_t n_src, float* dst,
                         float reg, const hals_als_plan* plan, float* slots, void* split_buf, cudaStream_t st);
 int als_half_step_tc64(const int32_t* colidx, const float* vals, const float* src, int64_t n_src, float* dst,
@@ -213,12 +213,11 @@ extern "C" int hals_als_plan_count_positive(const float* vals, const int64_t* it
   return als_count_positive(vals, item_begin, item_len, n_items, item_npos, (cudaStream_t)stream);
 }
 
-extern "C" int hals_als_half_step(const int64_t* rowptr, const int32_t* colidx, const float* vals,
-                                  int64_t m_dst, const float* src, int64_t n_src, float* dst, int k,
-                                  float reg, int implicit, float alpha, const float* gram,
-                                  const hals_als_plan* plan, void* workspace, size_t workspace_bytes,
-                                  void* stream) {
-  (void)rowptr;
+// Body of hals_als_half_step and hals_als_half_step_nonnegative.
+static int als_half_step_impl(const int32_t* colidx, const float* vals, int64_t m_dst, const float* src, int64_t n_src,
+                              float* dst, int k, float reg, int implicit, float alpha, const float* gram,
+                              const hals_als_plan* plan, void* workspace, size_t workspace_bytes, void* stream,
+                              bool nonneg, int32_t* n_capped) {
   HALS_REQUIRE(plan != nullptr, "null plan");
   HALS_REQUIRE(k >= 1 && k <= 128, "rank must be in [1,128]");
   HALS_REQUIRE(m_dst >= 0, "negative row count");
@@ -235,6 +234,9 @@ extern "C" int hals_als_half_step(const int64_t* rowptr, const int32_t* colidx, 
   if (workspace_bytes < hals_als_workspace_bytes(plan->n_slots, k, n_src))
     return fail(HALS_ERR_WORKSPACE, "%s: workspace too small%s", __func__);
   HALS_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, "workspace must be 16-byte aligned");
+  // the tensor-core solvers have no bound-constrained variant: nonnegative half-steps always run the CUDA-core kernels
+  if (nonneg) return als_half_step_simt(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, (float*)workspace, st,
+                                        true, n_capped);
   if (use_tc(k, implicit, alpha, plan)) {
     void* split = reinterpret_cast<uint8_t*>(workspace) + slot_region_bytes(plan->n_slots, k);
     if (implicit) {
@@ -259,5 +261,28 @@ extern "C" int hals_als_half_step(const int64_t* rowptr, const int32_t* colidx, 
     return als_half_step_ws64(colidx, plan->vals_hl, src, n_src, dst, reg, plan, (float*)workspace, split, nullptr, nullptr,
                               nullptr, st);
   }
-  return als_half_step_simt(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, (float*)workspace, st);
+  return als_half_step_simt(colidx, vals, src, dst, k, reg, implicit, alpha, gram, plan, (float*)workspace, st, false,
+                            nullptr);
+}
+
+extern "C" int hals_als_half_step(const int64_t* rowptr, const int32_t* colidx, const float* vals,
+                                  int64_t m_dst, const float* src, int64_t n_src, float* dst, int k,
+                                  float reg, int implicit, float alpha, const float* gram,
+                                  const hals_als_plan* plan, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+  (void)rowptr;
+  return als_half_step_impl(colidx, vals, m_dst, src, n_src, dst, k, reg, implicit, alpha, gram, plan, workspace,
+                            workspace_bytes, stream, false, nullptr);
+}
+
+extern "C" int hals_als_half_step_nonnegative(const int64_t* rowptr, const int32_t* colidx, const float* vals,
+                                              int64_t m_dst, const float* src, int64_t n_src, float* dst, int k,
+                                              float reg, int implicit, float alpha, const float* gram,
+                                              const hals_als_plan* plan, void* workspace, size_t workspace_bytes,
+                                              void* stream, int32_t* n_capped) {
+  (void)rowptr;
+  // A = (Gram +) sum y y^T + reg n I is positive definite only with reg > 0; the NNLS minimiser rests on it
+  HALS_REQUIRE(reg > 0.f, "nonnegative half-steps need reg > 0");
+  return als_half_step_impl(colidx, vals, m_dst, src, n_src, dst, k, reg, implicit, alpha, gram, plan, workspace,
+                            workspace_bytes, stream, true, n_capped);
 }

@@ -130,6 +130,22 @@ int hals_als_half_step(const int64_t* rowptr, const int32_t* colidx, const float
                        const hals_als_plan* plan /* device arrays inside */, void* workspace,
                        size_t workspace_bytes, void* stream);
 
+/* Nonnegative factors (Spark's ALS nonnegative=True, NNLSSolver): the same A and b as hals_als_half_step, in both modes,
+ * and dst_j = argmin_{x >= 0} 1/2 x^T A x - b^T x, the unique minimiser (A is positive definite because reg n > 0).
+ * Solved by block principal pivoting (Kim & Park 2011, Judice-Pires backup rule); each iterate solves the free
+ * subsystem A_FF x_F = b_F by Cholesky, so the accuracy is that of hals_als_half_step.  Deterministic.
+ *   - always the CUDA-core kernels, at ranks 64 and 128 too, whatever the plan carries (vals_hl etc. are ignored);
+ *   - reg <= 0: HALS_ERR_INVALID;
+ *   - the pivoting loop is capped at 3k + 8 free-set factorisations per row; a row that reaches the cap keeps its
+ *     last iterate with x >= 0 (finite, nonnegative) and, when n_capped (device int32) is not NULL, is added to
+ *     *n_capped atomically.  The caller zeroes *n_capped;
+ *   - workspace: hals_als_workspace_bytes, as for hals_als_half_step.  Rows without ratings get 0. */
+int hals_als_half_step_nonnegative(const int64_t* rowptr, const int32_t* colidx, const float* vals,
+                                   int64_t m_dst, const float* src, int64_t n_src, float* dst, int k,
+                                   float reg, int implicit, float alpha, const float* gram,
+                                   const hals_als_plan* plan, void* workspace, size_t workspace_bytes,
+                                   void* stream, int32_t* n_capped);
+
 /* Ranks 64 and 128, factors kept in split form across half-steps (what als_engine does; the stateless call above re-splits
  * the whole source matrix every time, which is a replicated pass on every rank of a sharded run).
  *   hals_als_split_factors: out_hl[r] = [bf16(x) (k) | bf16(x - bf16(x)) (k)] for n_rows rows (k = 64 or 128).
