@@ -53,28 +53,6 @@ constexpr int kTcSolverBytes = 64 * 68 * 4 + 256 + 256 + 128;   // Pall (every p
 constexpr int kTcTmemCols = 128;
 constexpr int kTcN = 80;
 
-__global__ void split_bf16_kernel(const float* __restrict__ src, int64_t n_rows, int k,
-                                  __nv_bfloat16* __restrict__ out) {
-  // one thread per 8 consecutive factors: writes a 16-byte h chunk and a 16-byte l chunk
-  const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int per_row = k >> 3;
-  if (gid >= n_rows * per_row) return;
-  const int64_t row = gid / per_row;
-  const int c = (int)(gid - row * per_row);
-  const float4 a = *reinterpret_cast<const float4*>(src + row * k + c * 8);
-  const float4 b = *reinterpret_cast<const float4*>(src + row * k + c * 8 + 4);
-  const float y[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-  __align__(16) __nv_bfloat16 h[8], l[8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    h[i] = __float2bfloat16_rn(y[i]);
-    l[i] = __float2bfloat16_rn(y[i] - __bfloat162float(h[i]));
-  }
-  __nv_bfloat16* o = out + row * (2 * k);
-  *reinterpret_cast<uint4*>(o + c * 8) = *reinterpret_cast<const uint4*>(h);
-  *reinterpret_cast<uint4*>(o + k + c * 8) = *reinterpret_cast<const uint4*>(l);
-}
-
 // Register-resident solve of one 64x64 SPD system by the two solver warps (thread m owns row m
 // of the symmetric matrix, a[0..63], and its right-hand side element a[64]).
 // Square-root-free Cholesky (A = L D L^T, the same elimination dppsv performs up to the scaling
@@ -551,32 +529,6 @@ als_tc64_kernel(const int32_t* __restrict__ colidx, const float* __restrict__ va
   if (warp == 0) umma::tmem_dealloc(tmem, kTcTmemCols);
 }
 
-// Long rows, level 1 of the deterministic slot reduction: groups of kSlotGroup consecutive slots of one row
-// are summed (fixed order) into the group's first slot; a Zipf-head row with hundreds of slices would otherwise
-// be summed by a single CTA.  grid = (n_long_rows, ceil(max_nseg / kSlotGroup)).
-constexpr int kSlotGroup = 16;
-// `stride` = distance between the partial sums of this level (1: raw slots, 16: the level-1 group leaders).
-__global__ void __launch_bounds__(256)
-als_slot_group_sum_kernel(float* __restrict__ workspace, const int32_t* __restrict__ long_slot0,
-                          const int32_t* __restrict__ long_nseg, int slot_floats, int stride) {
-  const int ns = long_nseg[blockIdx.x];
-  const int span = kSlotGroup * stride;                 // slots covered by one group of this level
-  const int g0 = blockIdx.y * span;
-  if (g0 >= ns || ns <= stride * kSlotGroup) return;    // this row does not need this level
-  const int g1 = min(ns, g0 + span);
-  float* base = workspace + (size_t)(long_slot0[blockIdx.x] + g0) * slot_floats;
-  for (int e = threadIdx.x; e < slot_floats; e += 256) {
-    float s = base[e];
-    for (int q = stride; q < g1 - g0; q += stride) s += base[(size_t)q * slot_floats + e];
-    base[e] = s;
-  }
-}
-
-// distance between the partial sums the solve kernels still have to add for a row of ns slices
-__host__ __device__ inline int slot_final_stride(int ns) {
-  return ns > kSlotGroup * kSlotGroup ? kSlotGroup * kSlotGroup : ns > kSlotGroup ? kSlotGroup : 1;
-}
-
 // Long rows (rank 64): sums the per-slice partial (A, b, n) slots in slot order -- deterministic -- adds the
 // ridge and solves with the same register-resident LDL^T as the main kernel.  One 64-thread CTA per long row.
 __global__ void __launch_bounds__(64)
@@ -618,42 +570,10 @@ als_reduce_solve64_kernel(const float* __restrict__ workspace, float* __restrict
   }
 }
 
-int als_launch_slot_group_sum(float* slots, const hals_als_plan* plan, int slot_floats, cudaStream_t st) {
-  // level 1: groups of 16 slices; level 2 (rows with more than 256 slices): groups of 16 level-1 leaders
-  for (int stride = 1; stride <= kSlotGroup; stride *= kSlotGroup) {
-    if (plan->max_nseg <= stride * kSlotGroup) break;
-    const int span = stride * kSlotGroup;
-    // rows sorted by slice count (csr.py): only the first n_long_gt16 / n_long_gt256 need this level
-    const int64_t hint = stride == 1 ? plan->n_long_gt16 : plan->n_long_gt256;
-    const int64_t rows = hint > 0 && hint < plan->n_long_rows ? hint : plan->n_long_rows;
-    dim3 g((unsigned)rows, (unsigned)((plan->max_nseg + span - 1) / span));
-    als_slot_group_sum_kernel<<<g, 256, 0, st>>>(slots, plan->long_slot0, plan->long_nseg, slot_floats, stride);
-    HALS_LAUNCH_CHECK();
-  }
-  return 0;
-}
-
-int als_launch_reduce_solve64(const float* slots, float* dst, float reg, const hals_als_plan* plan, void* dst_hl,
-                              cudaStream_t st) {
-  als_reduce_solve64_kernel<<<(unsigned)plan->n_long_rows, 64, 0, st>>>(slots, dst, reg, plan->long_row, plan->long_slot0,
-                                                                        plan->long_nseg, reinterpret_cast<__nv_bfloat16*>(dst_hl));
-  HALS_LAUNCH_CHECK();
-  return 0;
-}
-
-int als_launch_split_bf16(const float* src, int64_t n_src, int k, void* out, cudaStream_t st) {
-  const int64_t nthreads = n_src * (k / 8);
-  split_bf16_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, st>>>(src, n_src, k, reinterpret_cast<__nv_bfloat16*>(out));
-  HALS_LAUNCH_CHECK();
-  return 0;
-}
-
 int als_half_step_tc64(const int32_t* colidx, const float* vals, const float* src, int64_t n_src, float* dst,
                        float reg, const hals_als_plan* plan, float* slots, void* split_buf, cudaStream_t st) {
   __nv_bfloat16* hl = reinterpret_cast<__nv_bfloat16*>(split_buf);
-  const int64_t nthreads = n_src * (kTcK / 8);
-  split_bf16_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, st>>>(src, n_src, kTcK, hl);
-  HALS_LAUNCH_CHECK();
+  if (int rc = als_launch_split_bf16(src, n_src, kTcK, hl, st)) return rc;
   const size_t smem = (size_t)kTcStages * kTcStageBytes + kTcSolverBytes + 1024;
   static_assert(kTcStages * kTcStageBytes >= 2 * 64 * kTcLDS * 4 + 512, "accumulator hand-over must fit in the stage ring");
   HALS_CUDA(cudaFuncSetAttribute(als_tc64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

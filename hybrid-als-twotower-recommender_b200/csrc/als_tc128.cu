@@ -473,7 +473,7 @@ als_tc128_kernel(const int32_t* __restrict__ colidx, const float* __restrict__ v
 __global__ void __launch_bounds__(128)
 als_reduce_solve128_kernel(const float* __restrict__ workspace, float* __restrict__ dst, float reg,
                            const int32_t* __restrict__ long_row, const int32_t* __restrict__ long_slot0,
-                           const int32_t* __restrict__ long_nseg, int slot_group, __nv_bfloat16* __restrict__ dst_hl,
+                           const int32_t* __restrict__ long_nseg, __nv_bfloat16* __restrict__ dst_hl,
                            const float* __restrict__ gram) {
   constexpr int K = k8K;
   __shared__ __align__(16) float PS[2 * k8LDP + 128];
@@ -484,7 +484,7 @@ als_reduce_solve128_kernel(const float* __restrict__ workspace, float* __restric
 #pragma unroll
   for (int n = 0; n < 128; ++n) a[n] = 0.f;
   float bm = 0.f, cnt = 0.f;
-  const int stride = ns > slot_group * slot_group ? slot_group * slot_group : ns > slot_group ? slot_group : 1;   // two pre-sum levels
+  const int stride = slot_final_stride(ns);               // rows with many slices were pre-summed per group (two levels)
   for (int q = 0; q < ns; q += stride) {
     const float* W = workspace + (size_t)(s0 + q) * k8SlotFloats;
 #pragma unroll
@@ -517,9 +517,6 @@ als_reduce_solve128_kernel(const float* __restrict__ workspace, float* __restric
   }
 }
 
-int als_launch_slot_group_sum(float* slots, const hals_als_plan* plan, int slot_floats, cudaStream_t st);   // als_tc.cu
-int als_launch_split_bf16(const float* src, int64_t n_src, int k, void* out, cudaStream_t st);                 // als_tc.cu
-
 int als_half_step_tc128(const int32_t* colidx, const float* vals, const float* src, int64_t n_src, float* dst,
                         float reg, const hals_als_plan* plan, float* slots, void* split_buf, cudaStream_t st) {
   __nv_bfloat16* hl = reinterpret_cast<__nv_bfloat16*>(split_buf);
@@ -534,10 +531,9 @@ int als_half_step_tc128(const int32_t* colidx, const float* vals, const float* s
                                                              plan->item_len, plan->item_slot, plan->n_items, slots);
   HALS_LAUNCH_CHECK();
   if (plan->n_long_rows > 0) {
-    constexpr int kGroup = 16;                            // == kSlotGroup of als_tc.cu
     if (int rc = als_launch_slot_group_sum(slots, plan, (int)k8SlotFloats, st)) return rc;
     als_reduce_solve128_kernel<<<(unsigned)plan->n_long_rows, 128, 0, st>>>(slots, dst, reg, plan->long_row,
-                                                                            plan->long_slot0, plan->long_nseg, kGroup, nullptr, nullptr);
+                                                                            plan->long_slot0, plan->long_nseg, nullptr, nullptr);
     HALS_LAUNCH_CHECK();
   }
   return 0;
@@ -547,8 +543,8 @@ int als_half_step_tc128(const int32_t* colidx, const float* vals, const float* s
 int als_launch_reduce_solve128(const float* slots, float* dst, float reg, const hals_als_plan* plan, void* dst_hl,
                                const float* gram, cudaStream_t st) {
   als_reduce_solve128_kernel<<<(unsigned)plan->n_long_rows, 128, 0, st>>>(slots, dst, reg, plan->long_row, plan->long_slot0,
-                                                                          plan->long_nseg, 16,
-                                                                          reinterpret_cast<__nv_bfloat16*>(dst_hl), gram);
+                                                                          plan->long_nseg, reinterpret_cast<__nv_bfloat16*>(dst_hl),
+                                                                          gram);
   HALS_LAUNCH_CHECK();
   return 0;
 }

@@ -1,8 +1,10 @@
-// Device helpers shared by the tensor-core ALS kernels (als_tc.cu: rank 64, als_tc128.cu: rank 128).
+// Device helpers shared by the tensor-core ALS kernels (als_tc.cu / als_ws64.cu: rank 64, als_tc128.cu / als_ws128.cu:
+// rank 128).
 #pragma once
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include "als_prep.cuh"
 #include "common.cuh"
 
 namespace hals {
@@ -73,7 +75,8 @@ __device__ __forceinline__ void bar_sync_n(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;\n" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-// fp32 [n][k] -> bf16 [n][h(k) | l(k)], h = bf16(y), l = bf16(y - h)   (als_tc.cu)
-__global__ void split_bf16_kernel(const float* __restrict__ src, int64_t n_rows, int k, __nv_bfloat16* __restrict__ out);
+// the rank-128 long-row reduce + solve (als_tc128.cu), also the tail of als_ws128.cu
+int als_launch_reduce_solve128(const float* slots, float* dst, float reg, const hals_als_plan* plan, void* dst_hl,
+                               const float* gram, cudaStream_t st);
 
 }  // namespace hals

@@ -27,18 +27,14 @@
 
 #include <cstdlib>
 
-#include "als_common.cuh"
-#include "als_tc_common.cuh"
-#include "umma.cuh"
+#include "als_ws_common.cuh"
 
 namespace hals {
 namespace ws128 {
+using namespace ws;
 
 constexpr int K = 128;
-constexpr int KC = 32;
-constexpr int kRowBytes = 128;               // one 64-wide bf16 MN atom row
-constexpr int kBlk = KC * kRowBytes;         // 4096: one [KC][64] block
-constexpr int kStageBytes = 5 * kBlk;        // H0 | H1 | L0 | L1 | R
+constexpr int kStageBytes = stage_bytes(K);  // H0 | H1 | L0 | L1 | R
 constexpr int kStages = 6;
 constexpr int kLdc = 132;                    // hand-over row stride (floats)
 constexpr int kCBytes = 128 * kLdc * 4 + 512;            // C | b
@@ -46,13 +42,11 @@ constexpr int kGroups = 3;
 constexpr int kGroupScratch = 4096;          // P (2 x 512) | Y (512) | DI (512) | T (1024) | RH (64) | X (512)
 constexpr int kThreads = 512;
 constexpr int kWarpGather = 12, kWarpMma = 14;
-constexpr int kBurst = 8;
 // setmaxnreg (warpgroup-wide): the kernel is compiled for 128 registers per thread; the front-end warpgroup (warps
 // 12-15) gives 56 per thread back, which lets the three solver warpgroups grow to 144 -- room for the loads of the
 // next pivot next to the operands of the current trailing update (checked on the host before the launch).
 constexpr int kRegsLaunch = 128, kRegsFront = 72, kRegsSolver = 144;
 static_assert((kThreads / 32 - 4 * kGroups) * (kRegsLaunch - kRegsFront) >= 4 * kGroups * (kRegsSolver - kRegsLaunch), "register pool");
-constexpr int kGatherScratch = 2 * kBurst * 32 * 4 + 2 * kBurst * 8 + 2 * kBurst * 4;
 constexpr size_t kSlotFloats = (size_t)K * K + K + 4;
 static_assert(kStages % 2 == 0, "the two gather warps own alternate stages");
 
@@ -63,40 +57,6 @@ struct Bars {
   uint64_t acc_free;               // accumulator drained (128 arrivals of the draining group)
   uint64_t c_turn[kGroups];        // hand-over matrix free for group g's next row (arrival by the group before it)
 };
-struct Range {
-  int64_t item_lo, item_hi, chunk_lo, chunk_hi;
-};
-
-#ifdef HALS_WS_PROFILE
-#define WS_T0() const long long t0__ = clock64()
-#define WS_ACC(v) (v) += clock64() - t0__
-#else
-#define WS_T0() do { } while (0)
-#define WS_ACC(v) do { } while (0)
-#endif
-
-__device__ __forceinline__ void sts64_if(bool pred, uint32_t addr, f32x2 p) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p st.shared.b64 [%0], %1;\n\t}\n"
-               ::"r"(addr), "l"(p), "r"((uint32_t)pred) : "memory");
-}
-__device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* mbar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];\n" ::"r"(umma::smem_u32(mbar)) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-  uint32_t p;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(p));
-  return p != 0;
-}
-__device__ __forceinline__ f32x2 fmul2(f32x2 a, f32x2 b) { return ffma2(a, b, 0ull); }
-__device__ __forceinline__ float rcp_fast(float d) {
-  float r;
-  asm("rcp.approx.ftz.f32 %0, %1;\n" : "=f"(r) : "f"(d));
-  return r;
-}
-__host__ __device__ constexpr int tri(int q, int c) { return q * (q + 1) / 2 + c; }
-__device__ __forceinline__ void cp_async16_raw(uint32_t smem_dst, uint64_t gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
 
 // ---- G: gather (see als_ws64.cu for the scheme; here one warp instruction copies one 512-byte row) -------------
 __device__ __noinline__ void gather_role(uint32_t stages, Bars* bars, uint8_t* gscratch, const Range* rg,
@@ -199,50 +159,8 @@ __device__ __noinline__ void gather_role(uint32_t stages, Bars* bars, uint8_t* g
   }
 }
 
-// ---- implicit mode: rescale a landed stage in place, row t (= lane) by sqrt(c_t) ------------------------------------
-__device__ __forceinline__ uint32_t cvt_bf16x2(float hi, float lo) {
-  uint32_t d;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;\n" : "=r"(d) : "f"(hi), "f"(lo));
-  return d;
-}
-__device__ __forceinline__ f32x2 unpack_bf16x2(uint32_t w) {             // (element 0, element 1) as fp32
-  return pack2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
-}
-__device__ __noinline__ void scaler_role(uint32_t stages, Bars* bars, const Range* rg, const int32_t* __restrict__ chunk_cnt,
-                                         int lane) {
-  const int64_t k_lo = rg->chunk_lo, k_hi = rg->chunk_hi;
-  const uint32_t rowo = (uint32_t)lane * kRowBytes, x = (uint32_t)(lane & 7);
-  const f32x2 one2 = pack2(1.f, 1.f), mone2 = pack2(-1.f, -1.f);
-  uint32_t s = 0, su = 0;
-  for (int64_t k = k_lo; k < k_hi; ++k) {
-    umma::mbar_wait(&bars->st_full[s], su & 1);
-    const uint32_t st = stages + s * kStageBytes;
-    const float sc = lds32(st + 4 * kBlk + rowo + ((7u ^ x) << 4));
-    const f32x2 sc2 = pack2(sc, sc);
-#pragma unroll 2
-    for (int i = 0; i < 16; ++i) {
-      const uint32_t off = st + (uint32_t)(i >> 3) * kBlk + rowo + ((((uint32_t)i & 7u) ^ x) << 4);
-      const float4 hv = lds128(off), lv = lds128(off + 2 * kBlk);
-      const uint32_t hw[4] = {__float_as_uint(hv.x), __float_as_uint(hv.y), __float_as_uint(hv.z), __float_as_uint(hv.w)};
-      const uint32_t lw[4] = {__float_as_uint(lv.x), __float_as_uint(lv.y), __float_as_uint(lv.z), __float_as_uint(lv.w)};
-      uint32_t oh[4], ol[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const f32x2 y = ffma2(unpack_bf16x2(hw[j]), one2, unpack_bf16x2(lw[j]));
-        const f32x2 v = fmul2(y, sc2);
-        oh[j] = cvt_bf16x2(hi2(v), lo2(v));
-        const f32x2 r = ffma2(unpack_bf16x2(oh[j]), mone2, v);
-        ol[j] = cvt_bf16x2(hi2(r), lo2(r));
-      }
-      sts128(off, __uint_as_float(oh[0]), __uint_as_float(oh[1]), __uint_as_float(oh[2]), __uint_as_float(oh[3]));
-      sts128(off + 2 * kBlk, __uint_as_float(ol[0]), __uint_as_float(ol[1]), __uint_as_float(ol[2]), __uint_as_float(ol[3]));
-    }
-    umma::fence_proxy_async();                      // generic-proxy writes -> the tensor core's async-proxy reads
-    __syncwarp();
-    if (lane == 0) umma::mbar_arrive(&bars->st_scaled[s]);
-    if (++s == (uint32_t)kStages) { s = 0; ++su; }
-  }
-  (void)chunk_cnt;
+__device__ __noinline__ void scaler_role(uint32_t stages, Bars* bars, const Range* rg, int lane) {
+  scale_stages<K, kStages>(stages, bars, rg, lane);
 }
 
 // ---- M: MMA issue --------------------------------------------------------------------------------------------
@@ -608,22 +526,8 @@ als_ws128_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict_
     umma::mbar_init(&bars.acc_free, 128);
     umma::mbar_fence_init();
   }
-  if (tid < 2) {
-    const int64_t total = item_cost0[n_items];
-    const int64_t bq = (int64_t)blockIdx.x + tid;
-    const int64_t target = (total * bq + gridDim.x - 1) / gridDim.x;
-    int64_t lo = 0, hi = n_items;
-    while (lo < hi) {
-      const int64_t mid = (lo + hi) >> 1;
-      if (__ldg(item_cost0 + mid) < target) lo = mid + 1; else hi = mid;
-    }
-    if (bq == gridDim.x) lo = n_items;
-    const int64_t ck = __ldg(item_chunk0 + lo);
-    if (tid == 0) { range.item_lo = lo; range.chunk_lo = ck; } else { range.item_hi = lo; range.chunk_hi = ck; }
-  }
-  // the R blocks (rating columns of the B operand) are zero except for the 4 bytes per rating the gather copies in
-  for (int i = tid; i < kStages * (kBlk / 16); i += kThreads)
-    *reinterpret_cast<uint4*>(base + (i / (kBlk / 16)) * kStageBytes + 4 * kBlk + (i % (kBlk / 16)) * 16) = make_uint4(0u, 0u, 0u, 0u);
+  if (tid < 2) cta_range(&range, item_cost0, item_chunk0, n_items, tid);
+  zero_r_blocks<K, kStages, kThreads>(base, tid);
   umma::fence_proxy_async();
   umma::fence_before_sync();
   __syncthreads();
@@ -644,7 +548,7 @@ als_ws128_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict_
     gather_role(sbase, &bars, gscratch + (warp - kWarpGather) * kGatherScratch, &range, colidx, vals_hl, vals_sc,
                 reinterpret_cast<const uint8_t*>(src_hl), zero_row, chunk_pos, chunk_cnt, warp - kWarpGather, lane);
     else if (warp == kWarpMma) mma_role(sbase, tmem, &bars, &range, chunk_cnt, vals_sc != nullptr, lane);
-    else if (vals_sc != nullptr) scaler_role(sbase, &bars, &range, chunk_cnt, lane);
+    else if (vals_sc != nullptr) scaler_role(sbase, &bars, &range, lane);
   }
   umma::fence_before_sync();
   __syncthreads();
@@ -663,10 +567,6 @@ __global__ void gram_to_tiles128_kernel(const float* __restrict__ G, float* __re
         tiles[gl * 72 + ws128::tri(q, c) * 2 + h] = G[(ti + 8 * h + 16 * q) * ws128::K + tj + 16 * c];
 }
 
-int als_launch_slot_group_sum(float* slots, const hals_als_plan* plan, int slot_floats, cudaStream_t st);   // als_tc.cu
-int als_launch_reduce_solve128(const float* slots, float* dst, float reg, const hals_als_plan* plan, void* dst_hl,
-                               const float* gram, cudaStream_t st);                                          // als_tc128.cu
-
 // src != nullptr: fp32 source factors, split into `split_buf` first.  src == nullptr: `split_buf` already holds the
 // split source ([n_src + 1][256] bf16, row n_src all zero); see als_half_step_ws64.
 // gram != nullptr selects implicit feedback: the plan must carry vals_scale / item_npos (packed for the caller's alpha),
@@ -678,9 +578,7 @@ int als_half_step_ws128(const int32_t* colidx, const uint32_t* vals_hl, const fl
   __nv_bfloat16* hl = reinterpret_cast<__nv_bfloat16*>(split_buf);
   HALS_REQUIRE(n_src < (int64_t)1 << 31, "at most 2^31 - 1 source rows");
   if (src != nullptr) {
-    const int64_t nthreads = n_src * (K / 8);
-    split_bf16_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, st>>>(src, n_src, K, hl);
-    HALS_LAUNCH_CHECK();
+    if (int rc = als_launch_split_bf16(src, n_src, K, hl, st)) return rc;
     HALS_CUDA(cudaMemsetAsync(hl + (size_t)n_src * 2 * K, 0, 4 * K, st));
   }
   const bool implicit = gram != nullptr;

@@ -8,6 +8,7 @@
 //     G  warps 9-10 gather: cp.async 16-byte pieces of the h|l rows straight into the swizzled MN-major stage
 //                   (layout pinned by tests/test_gpu_umma.py), a flat stream of 32-rating chunks across row
 //                   boundaries, completion through the stage mbarrier (cp.async.mbarrier.arrive), column indices prefetched two bursts of 8 chunks ahead
+//                   (the implicit-mode scaler_role is shared with als_ws128.cu: als_ws_common.cuh)
 //     M  warp 11    one thread issues tcgen05.mma (M=128, N=80, K=16) per 16 ratings into one of four TMEM
 //                   accumulators; tcgen05.commit recycles the stage and publishes the finished accumulator
 //     D  warps 12-15 drain: TMEM lane = matrix row; rows of h h^T (warps 0,1) and l h^T (warps 2,3) go to one of
@@ -23,18 +24,14 @@
 
 #include <cstdlib>
 
-#include "als_common.cuh"
-#include "als_tc_common.cuh"
-#include "umma.cuh"
+#include "als_ws_common.cuh"
 
 namespace hals {
 namespace ws64 {
+using namespace ws;
 
 constexpr int K = 64;
-constexpr int KC = 32;                       // ratings per stage
-constexpr int kRowBytes = 128;               // one 64-wide bf16 MN atom row
-constexpr int kBlk = KC * kRowBytes;         // 4096: one [KC][64] block
-constexpr int kStageBytes = 3 * kBlk;        // H | L | R
+constexpr int kStageBytes = stage_bytes(K);  // H | L | R
 #ifndef HALS_WS_STAGES
 #define HALS_WS_STAGES 10
 #endif
@@ -63,41 +60,9 @@ struct Bars {
   uint64_t slot_free[kSlots];
 };
 
-#ifdef HALS_WS_PROFILE
-#define WS_T0() const long long t0__ = clock64()
-#define WS_ACC(v) (v) += clock64() - t0__
-#else
-#define WS_T0() do { } while (0)
-#define WS_ACC(v) do { } while (0)
-#endif
-
-__device__ __forceinline__ void sts64_if(bool pred, uint32_t addr, f32x2 p) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p st.shared.b64 [%0], %1;\n\t}\n"
-               ::"r"(addr), "l"(p), "r"((uint32_t)pred) : "memory");
-}
-__device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* mbar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];\n" ::"r"(umma::smem_u32(mbar)) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {   // true in exactly one lane of the (converged) warp
-  uint32_t p;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(p));
-  return p != 0;
-}
-__device__ __forceinline__ f32x2 fmul2(f32x2 a, f32x2 b) { return ffma2(a, b, 0ull); }
 __device__ __forceinline__ float sel4(float a, float b, float c, float d, int i) {
   return i == 0 ? a : i == 1 ? b : i == 2 ? c : d;
 }
-__device__ __forceinline__ float rcp_fast(float d) {   // pivots are >= lambda * n > 0 and never denormal
-  float r;
-  asm("rcp.approx.ftz.f32 %0, %1;\n" : "=f"(r) : "f"(d));
-  return r;
-}
-__host__ __device__ constexpr int tri(int q, int c) { return q * (q + 1) / 2 + c; }
-
-// This CTA's share of the plan: a contiguous range of work items (equal cost across CTAs) and of their chunks.
-struct Range {
-  int64_t item_lo, item_hi, chunk_lo, chunk_hi;
-};
 
 // ---- G: gather ---------------------------------------------------------------------------------------
 // The two gather warps take ALTERNATE chunks of the CTA's chunk table (chunk = up to 32 ratings of one item; warp w:
@@ -116,13 +81,6 @@ struct Range {
 // cycles each, once per chunk, serial in whichever warp executes it): every byte of a stage is written by cp.async,
 // whose completion through the mbarrier is what the MMA thread waits for -- the pattern of the cp.async
 // warp-specialised mainloops in CUTLASS.
-constexpr int kBurst = 8;
-constexpr int kGatherScratch = 2 * kBurst * 32 * 4 + 2 * kBurst * 8 + 2 * kBurst * 4;   // idx ring | pos | cnt
-
-__device__ __forceinline__ void cp_async16_raw(uint32_t smem_dst, uint64_t gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
-
 __device__ __noinline__ void gather_role(uint32_t stages, Bars* bars, uint8_t* gscratch, const Range* rg,
                                          const int32_t* __restrict__ colidx, const uint32_t* __restrict__ vals_hl,
                                          const float* __restrict__ vals_sc, const uint8_t* __restrict__ src_hl, int zero_row,
@@ -241,50 +199,8 @@ __device__ __noinline__ void gather_role(uint32_t stages, Bars* bars, uint8_t* g
 #endif
 }
 
-// ---- implicit mode (Hu-Koren): rescale a landed stage in place, row t (= lane) by sqrt(c_t), c = alpha |r| ----------
-// s = sqrt(c) (h + l) in fp32, re-split into bf16 hi/lo: the SAME two MMAs then build sum c y y^T, and the rating column
-// (which carries (1 + c) / sqrt(c) where r > 0) gives b = sum_{r>0} (1 + c) y.  See als_ws128.cu for the rank-128 twin.
-__device__ __forceinline__ uint32_t cvt_bf16x2(float hi, float lo) {
-  uint32_t d;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;\n" : "=r"(d) : "f"(hi), "f"(lo));
-  return d;
-}
-__device__ __forceinline__ f32x2 unpack_bf16x2(uint32_t w) {             // (element 0, element 1) as fp32
-  return pack2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
-}
 __device__ __noinline__ void scaler_role(uint32_t stages, Bars* bars, const Range* rg, int lane) {
-  const int64_t k_lo = rg->chunk_lo, k_hi = rg->chunk_hi;
-  const uint32_t rowo = (uint32_t)lane * kRowBytes, x = (uint32_t)(lane & 7);
-  const f32x2 one2 = pack2(1.f, 1.f), mone2 = pack2(-1.f, -1.f);
-  uint32_t s = 0, su = 0;
-  for (int64_t k = k_lo; k < k_hi; ++k) {
-    umma::mbar_wait(&bars->st_full[s], su & 1);
-    const uint32_t st = stages + s * kStageBytes;
-    const float sc = lds32(st + 2 * kBlk + rowo + ((7u ^ x) << 4));
-    const f32x2 sc2 = pack2(sc, sc);
-#pragma unroll 2
-    for (int i = 0; i < 8; ++i) {                       // the eight 16-byte chunks of row t: h in block 0, l in block 1
-      const uint32_t off = st + rowo + ((((uint32_t)i) ^ x) << 4);
-      const float4 hv = lds128(off), lv = lds128(off + kBlk);
-      const uint32_t hw[4] = {__float_as_uint(hv.x), __float_as_uint(hv.y), __float_as_uint(hv.z), __float_as_uint(hv.w)};
-      const uint32_t lw[4] = {__float_as_uint(lv.x), __float_as_uint(lv.y), __float_as_uint(lv.z), __float_as_uint(lv.w)};
-      uint32_t oh[4], ol[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const f32x2 y = ffma2(unpack_bf16x2(hw[j]), one2, unpack_bf16x2(lw[j]));
-        const f32x2 v = fmul2(y, sc2);
-        oh[j] = cvt_bf16x2(hi2(v), lo2(v));
-        const f32x2 r = ffma2(unpack_bf16x2(oh[j]), mone2, v);
-        ol[j] = cvt_bf16x2(hi2(r), lo2(r));
-      }
-      sts128(off, __uint_as_float(oh[0]), __uint_as_float(oh[1]), __uint_as_float(oh[2]), __uint_as_float(oh[3]));
-      sts128(off + kBlk, __uint_as_float(ol[0]), __uint_as_float(ol[1]), __uint_as_float(ol[2]), __uint_as_float(ol[3]));
-    }
-    umma::fence_proxy_async();                          // generic-proxy writes -> the tensor core's async-proxy reads
-    __syncwarp();
-    if (lane == 0) umma::mbar_arrive(&bars->st_scaled[s]);
-    if (++s == (uint32_t)kStages) { s = 0; ++su; }
-  }
+  scale_stages<K, kStages>(stages, bars, rg, lane);
 }
 
 // ---- M: MMA issue (whole warp walks the chunk table, lane 0 issues) --------------------------------------
@@ -520,6 +436,46 @@ __device__ __forceinline__ void back_block(const f32x2 (&R)[36], f32x2 (&x2)[8],
   }
 }
 
+// One system, after its tile is loaded: eliminate (z = L^-1 b published in Y, -1/d in DI), then substitute back and
+// store the row as fp32 and as the bf16 hi|lo split the NEXT half-step gathers (no separate split pass).
+// P | Y | DI | T | RH = the warp's kScratchBytes of shared memory.
+__device__ __forceinline__ void eliminate(f32x2 (&R)[36], f32x2& bb2, const uint32_t P, const uint32_t Y, const uint32_t DI,
+                                          int ti, int tj, int lane) {
+  elim_block<0>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<1>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<2>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<3>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<4>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<5>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<6>(R, bb2, P, Y, DI, ti, tj, lane);
+  elim_block<7>(R, bb2, P, Y, DI, ti, tj, lane);
+  __syncwarp();                            // DI[63] / Y[63] visible to every lane
+}
+__device__ __forceinline__ void back_store(const f32x2 (&R)[36], const uint32_t Y, const uint32_t DI, const uint32_t T,
+                                           const uint32_t RH, int ti, int tj, int lane, float* __restrict__ dst,
+                                           __nv_bfloat16* __restrict__ dst_hl, int row) {
+  f32x2 x2[8];
+#pragma unroll
+  for (int q = 0; q < 8; ++q) x2[q] = 0ull;
+  float out0 = 0.f, out1 = 0.f;
+  back_block<7>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<6>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<5>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<4>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<3>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<2>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<1>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  back_block<0>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
+  *reinterpret_cast<float2*>(dst + (int64_t)row * K + 2 * lane) = make_float2(out0, out1);
+  if (dst_hl) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(out0, out1);
+    const __nv_bfloat162 l = __floats2bfloat162_rn(out0 - __low2float(h), out1 - __high2float(h));
+    __nv_bfloat162* o = reinterpret_cast<__nv_bfloat162*>(dst_hl + (int64_t)row * (2 * K));
+    o[lane] = h;
+    o[K / 2 + lane] = l;
+  }
+}
+
 __device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars* bars, float* __restrict__ dst,
                                          __nv_bfloat16* __restrict__ dst_hl, float* __restrict__ workspace, float reg,
                                          const int32_t* __restrict__ item_row, const int32_t* __restrict__ item_len,
@@ -599,39 +555,12 @@ __device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars*
     }
     {
       WS_T0();
-      elim_block<0>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<1>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<2>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<3>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<4>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<5>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<6>(R, bb2, P, Y, DI, ti, tj, lane);
-      elim_block<7>(R, bb2, P, Y, DI, ti, tj, lane);
-      __syncwarp();                        // DI[63] / Y[63] visible to every lane
+      eliminate(R, bb2, P, Y, DI, ti, tj, lane);
       WS_ACC(t_elim);
     }
     {
       WS_T0();
-      f32x2 x2[8];
-#pragma unroll
-      for (int q = 0; q < 8; ++q) x2[q] = 0ull;
-      float out0 = 0.f, out1 = 0.f;
-      back_block<7>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<6>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<5>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<4>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<3>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<2>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<1>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      back_block<0>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-      *reinterpret_cast<float2*>(dst + (int64_t)row * K + 2 * lane) = make_float2(out0, out1);
-      if (dst_hl) {   // the bf16 hi|lo split of the row, what the NEXT half-step gathers (no separate split pass)
-        const __nv_bfloat162 h = __floats2bfloat162_rn(out0, out1);
-        const __nv_bfloat162 l = __floats2bfloat162_rn(out0 - __low2float(h), out1 - __high2float(h));
-        __nv_bfloat162* o = reinterpret_cast<__nv_bfloat162*>(dst_hl + (int64_t)row * (2 * K));
-        o[lane] = h;
-        o[K / 2 + lane] = l;
-      }
+      back_store(R, Y, DI, T, RH, ti, tj, lane, dst, dst_hl, row);
       WS_ACC(t_back);
     }
 #ifdef HALS_WS_PROFILE
@@ -671,23 +600,8 @@ als_ws64_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict__
     for (int s = 0; s < kSolvers; ++s) umma::mbar_init(&bars.sol_full[s], 128);
     umma::mbar_fence_init();
   }
-  if (tid < 2) {
-    // items [lo, hi) with lo = first item whose cost prefix reaches (total * b / grid): contiguous, equal-cost shares
-    const int64_t total = item_cost0[n_items];
-    const int64_t bq = (int64_t)blockIdx.x + tid;
-    const int64_t target = (total * bq + gridDim.x - 1) / gridDim.x;
-    int64_t lo = 0, hi = n_items;              // lower bound of `target` in item_cost0[0..n_items]
-    while (lo < hi) {
-      const int64_t mid = (lo + hi) >> 1;
-      if (__ldg(item_cost0 + mid) < target) lo = mid + 1; else hi = mid;
-    }
-    if (bq == gridDim.x) lo = n_items;
-    const int64_t ck = __ldg(item_chunk0 + lo);
-    if (tid == 0) { range.item_lo = lo; range.chunk_lo = ck; } else { range.item_hi = lo; range.chunk_hi = ck; }
-  }
-  // the R blocks (rating columns of the B operand) are zero except for the 4 bytes per rating the gather copies in
-  for (int i = tid; i < kStages * (kBlk / 16); i += kThreads)
-    *reinterpret_cast<uint4*>(base + (i / (kBlk / 16)) * kStageBytes + 2 * kBlk + (i % (kBlk / 16)) * 16) = make_uint4(0u, 0u, 0u, 0u);
+  if (tid < 2) cta_range(&range, item_cost0, item_chunk0, n_items, tid);
+  zero_r_blocks<K, kStages, kThreads>(base, tid);
   umma::fence_proxy_async();
   umma::fence_before_sync();
   __syncthreads();
@@ -736,15 +650,15 @@ als_ws64_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict__
 __global__ void __launch_bounds__(128)
 als_reduce_solve64_warp_kernel(const float* __restrict__ workspace, float* __restrict__ dst,
                                __nv_bfloat16* __restrict__ dst_hl, float reg, const int32_t* __restrict__ long_row,
-                               const int32_t* __restrict__ long_slot0, const int32_t* __restrict__ long_nseg, int final_stride_1,
-                               int final_stride_2, const float* __restrict__ gram) {
+                               const int32_t* __restrict__ long_slot0, const int32_t* __restrict__ long_nseg,
+                               const float* __restrict__ gram) {
   constexpr int SF = K * K + K + 4;
   __shared__ __align__(16) float sA[SF];
   __shared__ __align__(16) uint8_t sScratch[kScratchBytes];
   const int tid = threadIdx.x, lane = tid & 31;
   const int row = long_row[blockIdx.x];
   const int s0 = long_slot0[blockIdx.x], ns = long_nseg[blockIdx.x];
-  const int stride = ns > final_stride_2 ? final_stride_2 : ns > final_stride_1 ? final_stride_1 : 1;
+  const int stride = slot_final_stride(ns);
   for (int e = tid * 4; e < SF; e += 128 * 4) {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int q = 0; q < ns; q += stride) {
@@ -773,107 +687,12 @@ als_reduce_solve64_warp_kernel(const float* __restrict__ workspace, float* __res
   }
   f32x2 bb2 = pack2(sA[K * K + ti + 8 * tj], sA[K * K + ti + 4 + 8 * tj]);
   const uint32_t P = umma::smem_u32(sScratch), Y = P + 512, DI = Y + 256, T = DI + 256, RH = T + 256;
-  elim_block<0>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<1>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<2>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<3>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<4>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<5>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<6>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<7>(R, bb2, P, Y, DI, ti, tj, lane);
-  __syncwarp();
-  f32x2 x2[8];
-#pragma unroll
-  for (int q = 0; q < 8; ++q) x2[q] = 0ull;
-  float out0 = 0.f, out1 = 0.f;
-  back_block<7>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<6>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<5>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<4>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<3>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<2>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<1>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  back_block<0>(R, x2, Y, DI, T, RH, ti, tj, lane, out0, out1);
-  *reinterpret_cast<float2*>(dst + (int64_t)row * K + 2 * lane) = make_float2(out0, out1);
-  if (dst_hl) {
-    const __nv_bfloat162 h = __floats2bfloat162_rn(out0, out1);
-    const __nv_bfloat162 l = __floats2bfloat162_rn(out0 - __low2float(h), out1 - __high2float(h));
-    __nv_bfloat162* o = reinterpret_cast<__nv_bfloat162*>(dst_hl + (int64_t)row * (2 * K));
-    o[lane] = h;
-    o[K / 2 + lane] = l;
-  }
+  eliminate(R, bb2, P, Y, DI, ti, tj, lane);
+  back_store(R, Y, DI, T, RH, ti, tj, lane, dst, dst_hl, row);
 }
 
 }  // namespace ws64
 
-int als_launch_slot_group_sum(float* slots, const hals_als_plan* plan, int slot_floats, cudaStream_t st);
-int als_launch_reduce_solve64(const float* slots, float* dst, float reg, const hals_als_plan* plan, void* dst_hl,
-                              cudaStream_t st);
-
-__global__ void pack_ratings_kernel(const float* __restrict__ vals, int64_t nnz, uint32_t* __restrict__ out) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= nnz) return;
-  const float r = vals[i];
-  const __nv_bfloat16 rh = __float2bfloat16_rn(r);
-  const __nv_bfloat16 rl = __float2bfloat16_rn(r - __bfloat162float(rh));
-  out[i] = (uint32_t)__bfloat16_as_ushort(rh) | ((uint32_t)__bfloat16_as_ushort(rl) << 16);
-}
-
-int als_pack_ratings(const float* vals, int64_t nnz, uint32_t* out, cudaStream_t st) {
-  pack_ratings_kernel<<<(unsigned)((nnz + 255) / 256), 256, 0, st>>>(vals, nnz, out);
-  HALS_LAUNCH_CHECK();
-  return 0;
-}
-
-// Implicit feedback (Hu-Koren, c = alpha |r|): the tensor-core kernel rescales gathered rows by sqrt(c) and takes the
-// right-hand side from a rating column that holds (1 + c) / sqrt(c) where r > 0 and 0 elsewhere:
-//   sum (sqrt(c) y)(sqrt(c) y)^T = sum c y y^T,   sum (sqrt(c) y) (1 + c) / sqrt(c) = sum_{r>0} (1 + c) y.
-__global__ void pack_ratings_implicit_kernel(const float* __restrict__ vals, int64_t nnz, float alpha,
-                                             uint32_t* __restrict__ out_hl, float* __restrict__ out_scale) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= nnz) return;
-  const float r = vals[i];
-  const float c = alpha * fabsf(r);
-  const float sc = sqrtf(c);
-  const float rho = r > 0.f && c > 0.f ? (1.f + c) / sc : 0.f;
-  const __nv_bfloat16 rh = __float2bfloat16_rn(rho);
-  const __nv_bfloat16 rl = __float2bfloat16_rn(rho - __bfloat162float(rh));
-  out_hl[i] = (uint32_t)__bfloat16_as_ushort(rh) | ((uint32_t)__bfloat16_as_ushort(rl) << 16);
-  out_scale[i] = sc;
-}
-
-int als_pack_ratings_implicit(const float* vals, int64_t nnz, float alpha, uint32_t* out_hl, float* out_scale, cudaStream_t st) {
-  pack_ratings_implicit_kernel<<<(unsigned)((nnz + 255) / 256), 256, 0, st>>>(vals, nnz, alpha, out_hl, out_scale);
-  HALS_LAUNCH_CHECK();
-  return 0;
-}
-
-// ratings > 0 of every work item (one warp per item): the n of Spark's lambda * n in implicit mode
-__global__ void count_positive_kernel(const float* __restrict__ vals, const int64_t* __restrict__ item_begin,
-                                      const int32_t* __restrict__ item_len, int64_t n_items, int32_t* __restrict__ out) {
-  const int64_t it = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (it >= n_items) return;
-  const int64_t b = item_begin[it];
-  const int len = item_len[it];
-  int n = 0;
-  for (int t = lane; t < len; t += 32) n += vals[b + t] > 0.f;
-  for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
-  if (lane == 0) out[it] = n;
-}
-
-int als_count_positive(const float* vals, const int64_t* item_begin, const int32_t* item_len, int64_t n_items, int32_t* out,
-                       cudaStream_t st) {
-  count_positive_kernel<<<(unsigned)((n_items * 32 + 255) / 256), 256, 0, st>>>(vals, item_begin, item_len, n_items, out);
-  HALS_LAUNCH_CHECK();
-  return 0;
-}
-
-// src != nullptr: fp32 source factors, split into `split_buf` first (the stateless C-ABI call).
-// src == nullptr: `split_buf` already holds the split source ([n_src + 1][128] bf16, row n_src all zero) -- the
-// engine keeps the factors in this form across half-steps: every solved row is written as fp32 (dst) AND as its
-// bf16 hi|lo split (dst_hl, same row indexing as dst), so no split pass is needed and a sharded run all-gathers the
-// split rows in place.
 // Y^T Y ([64][64]) -> the one-warp solver's lane-tile order: tiles[lane][tri(q, c)] = (G[ti + 8q][tj + 8c],
 // G[ti + 4 + 8q][tj + 8c]), lane = 8 ti + tj.
 __global__ void gram_to_tiles64_kernel(const float* __restrict__ G, float* __restrict__ tiles) {
@@ -884,6 +703,11 @@ __global__ void gram_to_tiles64_kernel(const float* __restrict__ G, float* __res
         tiles[lane * 72 + ws64::tri(q, c) * 2 + h] = G[(ti + 4 * h + 8 * q) * ws64::K + tj + 8 * c];
 }
 
+// src != nullptr: fp32 source factors, split into `split_buf` first (the stateless C-ABI call).
+// src == nullptr: `split_buf` already holds the split source ([n_src + 1][128] bf16, row n_src all zero) -- the
+// engine keeps the factors in this form across half-steps: every solved row is written as fp32 (dst) AND as its
+// bf16 hi|lo split (dst_hl, same row indexing as dst), so no split pass is needed and a sharded run all-gathers the
+// split rows in place.
 // gram != nullptr selects implicit feedback (the plan must carry vals_scale / item_npos packed for the caller's alpha;
 // gram_tiles = 9,216 bytes of scratch).
 int als_half_step_ws64(const int32_t* colidx, const uint32_t* vals_hl, const float* src, int64_t n_src, float* dst,
@@ -893,9 +717,7 @@ int als_half_step_ws64(const int32_t* colidx, const uint32_t* vals_hl, const flo
   __nv_bfloat16* hl = reinterpret_cast<__nv_bfloat16*>(split_buf);
   HALS_REQUIRE(n_src < (int64_t)1 << 31, "at most 2^31 - 1 source rows");
   if (src != nullptr) {
-    const int64_t nthreads = n_src * (K / 8);
-    split_bf16_kernel<<<(unsigned)((nthreads + 255) / 256), 256, 0, st>>>(src, n_src, K, hl);
-    HALS_LAUNCH_CHECK();
+    if (int rc = als_launch_split_bf16(src, n_src, K, hl, st)) return rc;
     // row n_src of the split buffer (inside the workspace's slack): all zero, what the ragged tail of an item gathers
     HALS_CUDA(cudaMemsetAsync(hl + (size_t)n_src * 2 * K, 0, 4 * K, st));
   }
@@ -920,10 +742,8 @@ int als_half_step_ws64(const int32_t* colidx, const uint32_t* vals_hl, const flo
   HALS_LAUNCH_CHECK();
   if (plan->n_long_rows > 0) {
     if (int rc = als_launch_slot_group_sum(slots, plan, K * K + K + 4, st)) return rc;
-    // level strides of the slot pre-sums (als_tc.cu: kSlotGroup = 16)
     als_reduce_solve64_warp_kernel<<<(unsigned)plan->n_long_rows, 128, 0, st>>>(
-        slots, dst, reinterpret_cast<__nv_bfloat16*>(dst_hl), reg, plan->long_row, plan->long_slot0, plan->long_nseg, 16, 256,
-        gram);
+        slots, dst, reinterpret_cast<__nv_bfloat16*>(dst_hl), reg, plan->long_row, plan->long_slot0, plan->long_nseg, gram);
     HALS_LAUNCH_CHECK();
   }
   return 0;

@@ -2,7 +2,7 @@
 #include <cstdlib>
 #include <vector>
 
-#include "common.cuh"
+#include "als_prep.cuh"
 
 namespace hals {
 thread_local char g_last_error[512] = "";
@@ -18,14 +18,9 @@ int als_half_step_tc64(const int32_t* colidx, const float* vals, const float* sr
 int als_half_step_ws128(const int32_t* colidx, const uint32_t* vals_hl, const float* src, int64_t n_src, float* dst,
                         float reg, const hals_als_plan* plan, float* slots, void* split_buf, void* dst_hl,
                         const float* gram, float* gram_tiles, cudaStream_t st);
-int als_pack_ratings_implicit(const float* vals, int64_t nnz, float alpha, uint32_t* out_hl, float* out_scale, cudaStream_t st);
-int als_count_positive(const float* vals, const int64_t* item_begin, const int32_t* item_len, int64_t n_items, int32_t* out,
-                       cudaStream_t st);
 int als_half_step_ws64(const int32_t* colidx, const uint32_t* vals_hl, const float* src, int64_t n_src, float* dst,
                        float reg, const hals_als_plan* plan, float* slots, void* split_buf, void* dst_hl,
                        const float* gram, float* gram_tiles, cudaStream_t st);
-int als_launch_split_bf16(const float* src, int64_t n_src, int k, void* out, cudaStream_t st);
-int als_pack_ratings(const float* vals, int64_t nnz, uint32_t* out, cudaStream_t st);
 }  // namespace hals
 
 using namespace hals;
