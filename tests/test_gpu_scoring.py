@@ -42,9 +42,12 @@ def dense_blend(Ua, Ia, Ut, It, wa, wt):
 
 
 @pytest.mark.parametrize("U,I,ka,kt,k", [(130, 1000, 10, 50, 5), (64, 257, 128, 50, 100), (3, 5000, 64, 50, 10),
-                                         (1, 20000, 128, 50, 100), (200, 90, 16, 8, 200), (77, 640, 10, 50, 64)])
+                                         (1, 20000, 128, 50, 100), (200, 90, 16, 8, 200), (77, 640, 10, 50, 64)] +
+                         # either side of each candidate-capacity switch (topk_capacity: 64/65, 128/129), item-split
+                         [(150, 1800, 32, 16, k) for k in (64, 65, 128, 129, 256)])
 def test_blend_topk_matches_oracle(U, I, ka, kt, k):
     _, nat, scoring = _pkg()
+    assert int(nat.lib().hals_score_flag_counter_offset(U, I, ka, kt, k)) < 0, "expected the CUDA-core path"
     rng = np.random.default_rng(U + I)
     Ua, Ia = rng.normal(0, ka ** -0.5, (U, ka)).astype(np.float32), rng.normal(0, 1, (I, ka)).astype(np.float32)
     Ut, It = rng.normal(0, 1, (U, kt)).astype(np.float32), rng.normal(0, 1, (I, kt)).astype(np.float32)
@@ -58,7 +61,12 @@ def test_blend_topk_matches_oracle(U, I, ka, kt, k):
 
 
 @pytest.mark.parametrize("U,I,ka,kt,k", [(300, 20000, 128, 50, 100), (1000, 5000, 10, 50, 5), (130, 40000, 64, 50, 10),
-                                         (2000, 3000, 128, 50, 100), (5, 900000, 128, 50, 100), (257, 16500, 20, 50, 30)])
+                                         (2000, 3000, 128, 50, 100), (5, 900000, 128, 50, 100), (257, 16500, 20, 50, 30)] +
+                         # either side of make_plan's candidate-capacity switches (56/57: 128 -> 256 keys per stream;
+                         # 24/25 only differ in a two-part build), of the exact re-scoring's sort width (64/65,
+                         # 128/129, 256) and of topk_capacity in the merge; one user tile against 512 item tiles:
+                         # 64 splits, 512 columns per candidate stream
+                         [(64, 131072, 64, 50, k) for k in (1, 24, 25, 56, 57, 64, 65, 128, 129, 256)])
 def test_tensor_core_path_matches_oracle(U, I, ka, kt, k):
     """Shapes large enough for the tcgen05 path (TMA-staged bf16 operands, fused selection epilogue, exact
     fp32 re-scoring): the result must still be the exact fp32 answer."""
