@@ -1,4 +1,5 @@
 // C-ABI glue: error state, launch counter, host-side ALS planner, half-step dispatch.
+#include <cmath>
 #include <cstdlib>
 #include <vector>
 
@@ -163,9 +164,14 @@ extern "C" int hals_als_split_factors(const float* src, int64_t n_rows, int k, v
   return als_launch_split_bf16(src, n_rows, k, out_hl, (cudaStream_t)stream);
 }
 
+// Spark's regParam validator is gtEq(0): a negative reg can make A indefinite (silent NaN or garbage factors), a NaN
+// or infinite one poisons every row.  reg = 0 is accepted, as in Spark.
+static const char kRegCheck[] = "reg must be finite and >= 0";
+
 extern "C" int hals_als_half_step_split(const int32_t* colidx, int64_t m_dst, const void* src_hl, int64_t n_src,
                                         float* dst, void* dst_hl, int k, float reg, const hals_als_plan* plan,
                                         void* workspace, size_t workspace_bytes, void* stream) {
+  HALS_REQUIRE(reg >= 0.f && std::isfinite(reg), kRegCheck);
   HALS_REQUIRE(plan != nullptr, "null plan");
   HALS_REQUIRE(k == 64 || k == 128, "split-form half-steps exist for ranks 64 and 128");
   HALS_REQUIRE(m_dst >= 0 && n_src >= 0, "negative count");
@@ -213,6 +219,7 @@ static int als_half_step_impl(const int32_t* colidx, const float* vals, int64_t 
                               float* dst, int k, float reg, int implicit, float alpha, const float* gram,
                               const hals_als_plan* plan, void* workspace, size_t workspace_bytes, void* stream,
                               bool nonneg, int32_t* n_capped) {
+  HALS_REQUIRE(reg >= 0.f && std::isfinite(reg), kRegCheck);
   HALS_REQUIRE(plan != nullptr, "null plan");
   HALS_REQUIRE(k >= 1 && k <= 128, "rank must be in [1,128]");
   HALS_REQUIRE(m_dst >= 0, "negative row count");

@@ -54,6 +54,9 @@ int hals_max_rank(void);
  *   explicit:  A = sum_i y_i y_i^T,                b = sum_i r_ji y_i,          n = nnz_j
  *   implicit:  A = gram + sum_i c1 y_i y_i^T,      b = sum_{r>0} (1+c1) y_i,    n = #{r>0},  c1 = alpha*|r|
  *   A[d,d] += reg * n ;  dst_j = A^{-1} b (Cholesky).  Rows without ratings get 0.
+ * reg must be finite and >= 0 (Spark's regParam validator, gtEq(0)); anything else is HALS_ERR_INVALID before any
+ * CUDA call, here and in hals_als_half_step_split.  reg = 0 is accepted (A is then singular for a row with fewer
+ * ratings than k).
  *
  * Work decomposition is described by a plan built once per CSR matrix: rows longer than
  * `seg_len` ratings are cut into segments whose partial (A,b) go through `workspace` and

@@ -122,3 +122,23 @@ def test_compute_fails_loudly_without_gpu():
     assert pkg.ALSModel().initialize_spark() is False      # print + sentinel, like the reference
     with pytest.raises(nat.NativeError):
         pkg.TwoTowerModel(3, 3, 2, 2).build_model()
+
+
+def test_half_steps_reject_a_negative_or_non_finite_reg():
+    """Spark's regParam is >= 0: a negative reg can make A indefinite (silent NaN factors), a NaN one poisons every row.
+    Both entry points refuse them before any CUDA call (a zeroed plan, null pointers, no GPU needed); reg = 0 is
+    accepted as in Spark (here with no rows, so nothing runs)."""
+    L = nat.lib()
+    plan = nat.AlsPlan()
+    for reg in (-0.1, float("nan"), float("inf")):
+        for name, call in (
+            ("hals_als_half_step", lambda: L.hals_als_half_step(None, None, None, 0, None, 0, None, 64, reg, 0, 1.0,
+                                                                None, ctypes.byref(plan), None, 0, None)),
+            ("hals_als_half_step_split", lambda: L.hals_als_half_step_split(None, 0, None, 0, None, None, 64, reg,
+                                                                            ctypes.byref(plan), None, 0, None)),
+        ):
+            assert call() == 1, (name, reg)          # HALS_ERR_INVALID
+            assert b"reg must be finite and >= 0" in L.hals_last_error(), (name, reg, L.hals_last_error())
+    assert L.hals_als_half_step(None, None, None, 0, None, 0, None, 64, 0.0, 0, 1.0, None, ctypes.byref(plan), None, 0,
+                                None) == 0
+    assert L.hals_als_half_step_split(None, 0, None, 0, None, None, 64, 0.0, ctypes.byref(plan), None, 0, None) == 0

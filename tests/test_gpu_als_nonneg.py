@@ -89,7 +89,9 @@ def gpu_nonneg(rows, cols, vals, n_rows, src, reg, implicit=False, alpha=ALPHA, 
     return dst.cpu().numpy(), plan, (None if capped is None else int(capped.item()))
 
 
-def check_case(got, rows, cols, vals, n_rows, src, reg, implicit, alpha=ALPHA, coverage=True):
+def check_case(got, rows, cols, vals, n_rows, src, reg, implicit, alpha=ALPHA, coverage=True, forward=True):
+    """The KKT conditions per row, nonnegativity, zero empty rows; the rel-L2 forward tolerance unless forward=False
+    (ill-conditioned cases, where fp32 rounding alone moves x by ~kappa u: the KKT check is then the criterion)."""
     rp, ci, v = als_oracle.coo_to_csr(rows, cols, vals, n_rows)
     ids, A, b = nnls_oracle.normal_equations(rp, ci, v, src, reg, implicit, alpha)
     x, _ = nnls_oracle.nnls_batched(A, b)
@@ -103,7 +105,8 @@ def check_case(got, rows, cols, vals, n_rows, src, reg, implicit, alpha=ALPHA, c
     assert not np.isnan(got).any() and (got >= 0).all()
     empty = np.setdiff1d(np.arange(n_rows), ids)
     assert not got[empty].any(), "rows without ratings are zero"
-    assert rel_l2(got, want) <= REL[implicit], rel_l2(got, want)
+    if forward:
+        assert rel_l2(got, want) <= REL[implicit], rel_l2(got, want)
     g64 = got[ids].astype(np.float64)
     grad = np.einsum("rij,rj->ri", A, g64) - b
     tau = 1e-4 * (np.einsum("rij,rj->ri", np.abs(A), np.abs(g64)) + np.abs(b))
