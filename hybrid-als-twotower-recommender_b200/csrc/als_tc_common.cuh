@@ -54,14 +54,15 @@ __device__ __forceinline__ void sts128x2(uint32_t addr, f32x2 p0, f32x2 p1) {
   asm volatile("st.shared.v2.b64 [%0], {%1,%2};\n" ::"r"(addr), "l"(p0), "l"(p1) : "memory");
 }
 
-// Predicated (branch-free) shared stores: the pivot owner publishes without diverging its warp.
-__device__ __forceinline__ void sts128x2_if(bool pred, uint32_t addr, f32x2 p0, f32x2 p1) {
+// Predicated (branch-free) shared stores, pred = any non-zero word: the pivot owner publishes without diverging its
+// warp, and a role bit tests with one instruction.
+__device__ __forceinline__ void sts128x2_if(uint32_t pred, uint32_t addr, f32x2 p0, f32x2 p1) {
   asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %3, 0;\n\t@p st.shared.v2.b64 [%0], {%1,%2};\n\t}\n"
-               ::"r"(addr), "l"(p0), "l"(p1), "r"((uint32_t)pred) : "memory");
+               ::"r"(addr), "l"(p0), "l"(p1), "r"(pred) : "memory");
 }
-__device__ __forceinline__ void sts32_if(bool pred, uint32_t addr, float a) {
+__device__ __forceinline__ void sts32_if(uint32_t pred, uint32_t addr, float a) {
   asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p st.shared.f32 [%0], %1;\n\t}\n"
-               ::"r"(addr), "f"(a), "r"((uint32_t)pred) : "memory");
+               ::"r"(addr), "f"(a), "r"(pred) : "memory");
 }
 
 // Named barriers: 1 = the two solver warps, 2 = the two producer warps (0 is __syncthreads).

@@ -50,6 +50,8 @@ constexpr int kThreads = 512;
 constexpr int kWarpSolver = 0, kWarpGather = 9, kWarpMma = 11, kWarpDrain = 12;
 static_assert(kStages % 2 == 0, "the two gather warps own alternate stages");
 static_assert(kWarpSolver + kSolvers == kWarpGather && kWarpDrain + 4 == kThreads / 32 && kWarpDrain % 4 == 0, "role map");
+static_assert(kStageBytes % 512 == 0 && kSlotBytes % 512 == 0 && kScratchBytes % 512 == 0,
+              "a solver's scratch is 512-byte aligned: its elimination steps flip the column buffer by bit 8");
 
 struct Bars {
   uint64_t st_full[kStages], st_free[kStages];
@@ -307,81 +309,127 @@ __device__ __noinline__ void drain_role(uint32_t slots, uint32_t tmem, Bars* bar
 // lane then needs 8-JR packed row values, 8-JR column values and the pivot:  A[m][n] -= (A[m][j]/d) * A[n][j].
 // Finished columns stay in the registers as columns of L*D and feed the back substitution.
 // Right-hand side: b[ti + 8tj], b[ti + 4 + 8tj] live in lane (ti, tj) as one packed pair; z = L^-1 b is
-// published element by element (Y[j]) as the pivots pass.
+// published element by element (Y[j]) as the pivots pass.  A row's pair half is dead once its z is out, so the update
+// runs on both halves of every lane (no row mask): only rows below the pivot are published later.
+//
+// Published column: P[q / 2][ti][q % 2][half] (row ti + 4 half + 8 q).  The first layout, P[ti][q][half], put rows
+// ti and ti + 2 on the same banks: every column-value load and every publish was a 2-way conflict, and the solver
+// warps keep the SM's one shared-memory pipe 72 % busy (ncu, user half of c2) -- wavefronts are what this loop pays.
+// Step jm reads buffer jm % 2 and publishes column j + 1 into the other one: P is 512-byte aligned, so the lane's three
+// base addresses flip bit 8 after each step.
+struct Lane {
+  uint32_t pw, pl, pb;   // P + my rows (+ (q / 2) * 64 + (q % 2) * 8), + row n = tj + 8c of a column, + my rhs rows
+  uint32_t dsel;         // low 16 bits: byte selector of my diagonal-block pivot candidate (high half if tj >= 4);
+                         // bit kRoleOwn: set if I hold the pivot of the column I own (ti == tj % 4)
+  uint32_t roles;        // the role bytes; kRoleZ as in block JR == tj (elim_block clears it in the other blocks)
+};
+// Role bytes (bit jm = this lane's part in step jm of a block).  Each step shifts the word by one, so every test is
+// one AND with a constant bit.
+constexpr int kRoleLive = 0;    // tj > jm: my column of the diagonal block is not finished yet
+constexpr int kRoleZ = 8;       // ti == (jm + 1) % 4, jm < 7, in block JR == tj: I hold row j + 1 of the rhs
+constexpr int kRoleOwn = 16;    // tj == jm + 1: I publish column j + 1 (and 1/d of its pivot if dsel says so)
+constexpr int kRoleZhi = 24;    // jm >= 3: row j + 1 is the high half of its pair.  The same in every lane, and it
+                                // empties after the block's eight steps: it is also the loop counter.
+
+// Built once per system from %laneid, not from a lane index kept in a register: the compiler would hoist all of it out
+// of the solver's row loop and hold it (spilled) across the tile load and the back substitution.
+__device__ __forceinline__ Lane lane_setup(uint32_t P) {
+  uint32_t lane;
+  asm volatile("mov.u32 %0, %%laneid;\n" : "=r"(lane));
+  const uint32_t ti = lane >> 3, tj = lane & 7;
+  Lane L;
+  L.pw = P + ti * 16u;
+  L.pl = P + (tj & 3) * 16u + (tj >> 2) * 4u;
+  L.pb = L.pw + (tj >> 1) * 64u + (tj & 1) * 8u;
+  L.dsel = (tj & 4 ? 0x7654u : 0x3210u) | (ti == (tj & 3) ? 3u << kRoleOwn : 0u);
+  const uint32_t z = ti == 0 ? 0x08u : 0x11u << (ti - 1);       // steps jm with (jm + 1) % 4 == ti, jm < 7
+  L.roles = (((1u << tj) - 1u) << kRoleLive) | (z << kRoleZ) | (((1u << tj) >> 1) << kRoleOwn) | (0xf8u << kRoleZhi);
+  return L;
+}
+
+// pred ? a : b for a predicate that is a non-zero word (a role bit): one LOP3 into a predicate and one select
+__device__ __forceinline__ float sel_if(uint32_t pred, float a, float b) {
+  float r;
+  asm("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %1, 0;\n\tselp.f32 %0, %2, %3, p;\n\t}\n" : "=f"(r) : "r"(pred), "f"(a), "f"(b));
+  return r;
+}
+
 template <int JR>
-__device__ __forceinline__ void elim_block(f32x2 (&R)[36], f32x2& bb2, const uint32_t P, const uint32_t Y,
-                                           const uint32_t DI, const int ti, const int tj, const int lane) {
-  // Published column: P[q / 2][ti][q % 2][half] (row ti + 4 half + 8 q).  The first layout, P[ti][q][half], put rows
-  // ti and ti + 2 on the same banks: every column-value load and every publish was a 2-way conflict, and the solver
-  // warps keep the SM's one shared-memory pipe 72 % busy (ncu, user half of c2) -- wavefronts are what this loop pays.
-  const uint32_t oW = (uint32_t)ti * 16u;                                  // my rows: + (q / 2) * 64 + (q % 2) * 8
-  const uint32_t oL = (uint32_t)(tj & 3) * 16u + (uint32_t)(tj >> 2) * 4u; // row n = tj + 8c: + (c / 2) * 64 + (c % 2) * 8
-  const uint32_t oB = oW + (uint32_t)(tj >> 1) * 64u + (uint32_t)(tj & 1) * 8u;   // my right-hand-side rows (q = tj)
-  auto publish = [&](uint32_t Pn, bool own) {
-    if (JR & 1) sts64_if(own, Pn + oW + (JR >> 1) * 64 + 8, R[tri(JR, JR)]);
+__device__ __forceinline__ void publish_column(const f32x2 (&R)[36], uint32_t pw, uint32_t own) {
+  if (JR & 1) sts64_if(own, pw + (JR >> 1) * 64 + 8, R[tri(JR, JR)]);
 #pragma unroll
-    for (int q = (JR + 1) & ~1; q < 8; q += 2) sts128x2_if(own, Pn + oW + (q >> 1) * 64, R[tri(q, JR)], R[tri(q + 1, JR)]);
-  };
-  {   // column 8*JR goes out first (owners: tj == 0), into buffer 0; lane 0 holds its diagonal and publishes -1/d
-    publish(P, tj == 0);
-    sts32_if(ti == 0 && tj == JR, Y + (uint32_t)(8 * JR) * 4u, lo2(bb2));
-    sts32_if(lane == 0, DI + (uint32_t)(8 * JR) * 4u, -rcp_fast(lo2(R[tri(JR, JR)])));
+  for (int q = (JR + 1) & ~1; q < 8; q += 2) sts128x2_if(own, pw + (q >> 1) * 64, R[tri(q, JR)], R[tri(q + 1, JR)]);
+}
+
+// Step j = 8 JR + jm; yj = Y + 4 j, DI = Y + 256 holds 1/d.  The multipliers are +A[m][j]/d and the column values
+// enter negated (an operand modifier of FFMA2): x * (-y) rounds exactly like -(x * y), so every product and sum is
+// the one of A[m][n] += (A[m][j] * (-1/d)) * A[n][j].
+template <int JR>
+__device__ __forceinline__ void elim_step(f32x2 (&R)[36], f32x2& bb2, const Lane& L, const uint32_t yj, const uint32_t roles) {
+  f32x2 w[8];
+  float l[8];
+  if (JR & 1) w[JR] = lds64x2(L.pw + (JR >> 1) * 64 + 8);
+#pragma unroll
+  for (int q = (JR + 1) & ~1; q < 8; q += 2) lds128x2(L.pw + (q >> 1) * 64, w[q], w[q + 1]);
+  const float dinv = lds32(yj + 256);
+#pragma unroll
+  for (int c = JR; c < 8; ++c) l[c] = lds32(L.pl + (c >> 1) * 64 + (c & 1) * 8);
+  const float zj = lds32(yj);
+  const f32x2 wb = lds64x2(L.pb);
+  const f32x2 dinv2 = pack2(dinv, dinv);
+  const float lj = sel_if(roles & (1u << kRoleLive), l[JR], 0.f);   // columns <= j are finished
+  // the diagonal block first: it holds the next pivot, whose reciprocal then overlaps the rest of the column
+  // Rows <= j of the diagonal block are finished, but their multipliers are NOT zeroed: a finished row only owns
+  // entries of finished columns (l = 0 below: untouched) and of the upper triangle inside the diagonal block, which
+  // nothing ever reads (the column publish of a later pivot carries them as row multipliers of finished rows again;
+  // the back substitution reads the strict lower triangle only).  Each half of a packed pair is its own row, so a
+  // runaway value cannot leak into a live one.
+  w[JR] = fmul2(w[JR], dinv2);
+  R[tri(JR, JR)] = ffma2(w[JR], pack2(-lj, -lj), R[tri(JR, JR)]);
+  // only the owner of column j + 1 with ti == tj % 4 stores this: its pivot is half tj / 4 of the pair
+  const float dinv_n = rcp_fast(__uint_as_float(
+      __byte_perm(__float_as_uint(lo2(R[tri(JR, JR)])), __float_as_uint(hi2(R[tri(JR, JR)])), L.dsel)));
+#pragma unroll
+  for (int q = JR + 1; q < 8; ++q) {      // the block's own column, so that column j+1 can go out early
+    w[q] = fmul2(w[q], dinv2);
+    R[tri(q, JR)] = ffma2(w[q], pack2(-lj, -lj), R[tri(q, JR)]);
+  }
+  bb2 = ffma2(fmul2(wb, dinv2), pack2(-zj, -zj), bb2);
+  {   // publish column j + 1 into the other buffer (jm == 7: nobody owns "column 8" of the block -- no store, no branch)
+    const uint32_t own = roles & (1u << kRoleOwn);
+    publish_column<JR>(R, L.pw ^ 256u, own);
+    sts32_if(roles & (1u << kRoleZ), yj + 4, sel_if(roles & (1u << kRoleZhi), hi2(bb2), lo2(bb2)));
+    sts32_if(own & L.dsel, yj + 256 + 4, dinv_n);
     __syncwarp();
   }
-  const bool below = tj > JR;             // my right-hand-side rows are below this whole block
-#pragma unroll 1
-  for (int jm = 0; jm < 8; ++jm) {
-    const int j = 8 * JR + jm;
-    const uint32_t Pj = P + ((uint32_t)(jm & 1) << 8);
-    f32x2 w[8];
-    float l[8];
-    if (JR & 1) w[JR] = lds64x2(Pj + oW + (JR >> 1) * 64 + 8);
 #pragma unroll
-    for (int q = (JR + 1) & ~1; q < 8; q += 2) lds128x2(Pj + oW + (q >> 1) * 64, w[q], w[q + 1]);
-    const float ninv = lds32(DI + (uint32_t)j * 4u);
+  for (int c = JR + 1; c < 8; ++c) {
 #pragma unroll
-    for (int c = JR; c < 8; ++c) l[c] = lds32(Pj + oL + (c >> 1) * 64 + (c & 1) * 8);
-    const float zj = lds32(Y + (uint32_t)j * 4u);
-    const f32x2 wb = lds64x2(Pj + oB);
-    const f32x2 ninv2 = pack2(ninv, ninv);
-    const float lj = tj > jm ? l[JR] : 0.f;      // columns <= j are finished
-    const f32x2 lj2 = pack2(lj, lj);
-    // the diagonal block first: it holds the next pivot, whose reciprocal then overlaps the rest of the column
-    // Rows <= j of the diagonal block are finished, but their multipliers are NOT zeroed: a finished row only owns
-    // entries of finished columns (l = 0 below: untouched) and of the upper triangle inside the diagonal block, which
-    // nothing ever reads (the column publish of a later pivot carries them as row multipliers of finished rows again;
-    // the back substitution reads the strict lower triangle only).  Each half of a packed pair is its own row, so a
-    // runaway value cannot leak into a live one.
-    w[JR] = fmul2(w[JR], ninv2);
-    R[tri(JR, JR)] = ffma2(w[JR], lj2, R[tri(JR, JR)]);
-    const int jn = jm + 1;
-    const float ninv_n = -rcp_fast((jn & 4) ? hi2(R[tri(JR, JR)]) : lo2(R[tri(JR, JR)]));
-#pragma unroll
-    for (int q = JR + 1; q < 8; ++q) {      // the block's own column, so that column j+1 can go out early
-      w[q] = fmul2(w[q], ninv2);
-      R[tri(q, JR)] = ffma2(w[q], lj2, R[tri(q, JR)]);
-    }
-    {   // right-hand side rows below the pivot
-      const bool on = tj == JR;
-      const bool act_lo = below || (on && ti > jm), act_hi = below || (on && ti + 4 > jm);
-      const f32x2 mb = fmul2(wb, ninv2);
-      bb2 = ffma2(pack2(act_lo ? lo2(mb) : 0.f, act_hi ? hi2(mb) : 0.f), pack2(zj, zj), bb2);
-    }
-    {   // publish column j + 1 (jm == 7: nobody owns "column 8" of the block -- no store, no branch either)
-      const uint32_t Pn = P + ((uint32_t)(jn & 1) << 8);
-      const bool own = (tj == jn);
-      publish(Pn, own);
-      sts32_if(tj == JR && ti == (jn & 3) && jn < 8, Y + (uint32_t)(j + 1) * 4u, (jn & 4) ? hi2(bb2) : lo2(bb2));
-      sts32_if(own && ti == (jn & 3), DI + (uint32_t)(j + 1) * 4u, ninv_n);
-      __syncwarp();
-    }
-#pragma unroll
-    for (int c = JR + 1; c < 8; ++c) {
-      const f32x2 l2 = pack2(l[c], l[c]);
-#pragma unroll
-      for (int q = c; q < 8; ++q) R[tri(q, c)] = ffma2(w[q], l2, R[tri(q, c)]);
-    }
+    for (int q = c; q < 8; ++q) R[tri(q, c)] = ffma2(w[q], pack2(-l[c], -l[c]), R[tri(q, c)]);
   }
+}
+
+// yj: Y + 4 * 8 JR on entry, the next block's on return
+template <int JR>
+__device__ __forceinline__ void elim_block(f32x2 (&R)[36], f32x2& bb2, Lane& L, uint32_t& yj) {
+  // tj == JR <=> kRoleLive bits JR-1 set, JR clear
+  const bool zblk = (L.roles & (JR ? 3u << (JR - 1) : 1u)) == (JR ? 1u << (JR - 1) : 0u);
+  uint32_t roles = zblk ? L.roles : L.roles & ~(0xffu << kRoleZ);
+  {   // column 8*JR goes out first, into buffer 0: its owners are the lanes tj == 0 (no kRoleLive bit), lane 0 holds
+      // its pivot and publishes 1/d, lane (0, JR) holds row 8*JR of the rhs (the only kRoleZ bit 3 of the block)
+    const bool own0 = (L.roles & (1u << kRoleLive)) == 0;
+    publish_column<JR>(R, L.pw, own0);
+    sts32_if(roles & (1u << (kRoleZ + 3)), yj, lo2(bb2));
+    sts32_if(own0 && (L.dsel & (1u << kRoleOwn)), yj + 256, rcp_fast(lo2(R[tri(JR, JR)])));
+    __syncwarp();
+  }
+#pragma unroll 1
+  do {
+    elim_step<JR>(R, bb2, L, yj, roles);
+    L.pw ^= 256u; L.pl ^= 256u; L.pb ^= 256u;
+    yj += 4;
+    roles >>= 1;
+  } while (roles >= 1u << kRoleZhi);
 }
 
 // Back substitution L^T x = D^-1 z by blocks of 8 unknowns, last block first.  The part of the sums that reaches
@@ -414,7 +462,7 @@ __device__ __forceinline__ void back_block(const f32x2 (&R)[36], f32x2 (&x2)[8],
   }
 #pragma unroll
   for (int e = 7; e >= 0; --e) {
-    xb[e] = -r[e] * di[e];                 // DI holds -1/d
+    xb[e] = r[e] * di[e];                  // DI holds 1/d
     if (e > 0) {
       float t[8];
       const float4 a = lds128(T + (uint32_t)(e * 8) * 4u);
@@ -436,19 +484,20 @@ __device__ __forceinline__ void back_block(const f32x2 (&R)[36], f32x2 (&x2)[8],
   }
 }
 
-// One system, after its tile is loaded: eliminate (z = L^-1 b published in Y, -1/d in DI), then substitute back and
+// One system, after its tile is loaded: eliminate (z = L^-1 b published in Y, 1/d in DI), then substitute back and
 // store the row as fp32 and as the bf16 hi|lo split the NEXT half-step gathers (no separate split pass).
-// P | Y | DI | T | RH = the warp's kScratchBytes of shared memory.
-__device__ __forceinline__ void eliminate(f32x2 (&R)[36], f32x2& bb2, const uint32_t P, const uint32_t Y, const uint32_t DI,
-                                          int ti, int tj, int lane) {
-  elim_block<0>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<1>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<2>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<3>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<4>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<5>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<6>(R, bb2, P, Y, DI, ti, tj, lane);
-  elim_block<7>(R, bb2, P, Y, DI, ti, tj, lane);
+// P | Y | DI | T | RH = the warp's kScratchBytes of shared memory (DI = Y + 256: one address serves both).
+__device__ __forceinline__ void eliminate(f32x2 (&R)[36], f32x2& bb2, const uint32_t P, const uint32_t Y) {
+  Lane L = lane_setup(P);
+  uint32_t yj = Y;
+  elim_block<0>(R, bb2, L, yj);
+  elim_block<1>(R, bb2, L, yj);
+  elim_block<2>(R, bb2, L, yj);
+  elim_block<3>(R, bb2, L, yj);
+  elim_block<4>(R, bb2, L, yj);
+  elim_block<5>(R, bb2, L, yj);
+  elim_block<6>(R, bb2, L, yj);
+  elim_block<7>(R, bb2, L, yj);
   __syncwarp();                            // DI[63] / Y[63] visible to every lane
 }
 __device__ __forceinline__ void back_store(const f32x2 (&R)[36], const uint32_t Y, const uint32_t DI, const uint32_t T,
@@ -476,35 +525,50 @@ __device__ __forceinline__ void back_store(const f32x2 (&R)[36], const uint32_t 
   }
 }
 
-__device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars* bars, float* __restrict__ dst,
-                                         __nv_bfloat16* __restrict__ dst_hl, float* __restrict__ workspace, float reg,
-                                         const int32_t* __restrict__ item_row, const int32_t* __restrict__ item_len,
-                                         const int32_t* __restrict__ item_slot, const float* __restrict__ gram_tiles,
+// The solver's kernel arguments, in shared memory and loaded where they are used: held in registers across the
+// elimination, whose peak takes all 128, they were spilled.
+struct SolverArgs {
+  float* dst;
+  __nv_bfloat16* dst_hl;
+  float* workspace;
+  const float* gram_tiles;
+  const int32_t* item_row;
+  const int32_t* item_len;
+  const int32_t* item_slot;
+  float reg;
+};
+template <class T>
+__device__ __forceinline__ T* ld_arg(T* const& v) {          // volatile: not hoisted out of the row loop
+  uint64_t r;
+  asm volatile("ld.shared.u64 %0, [%1];\n" : "=l"(r) : "r"(umma::smem_u32(&v)));
+  return reinterpret_cast<T*>(r);
+}
+__device__ __forceinline__ float ld_arg(const float& v) { return lds32(umma::smem_u32(&v)); }
+
+__device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars* bars, const SolverArgs* args,
                                          const Range* rg, int nsolv, int w, int lane) {
   const int ti = lane >> 3, tj = lane & 7;
   const uint32_t P = scratch, Y = P + 512, DI = Y + 256, T = DI + 256, RH = T + 256;
-  const int64_t n_items = rg->item_hi;
+  // this CTA's items (a share of one plan, far below 2^32)
+  const uint32_t n_items = (uint32_t)(rg->item_hi - rg->item_lo);
 #ifdef HALS_WS_PROFILE
   long long w_slot = 0, t_load = 0, t_elim = 0, t_back = 0;
   int n_solved = 0;
 #endif
-  // rows i = w, w + kSolvers, ... of this CTA's item sequence; slot = i % kSlots
-  int64_t it = rg->item_lo + w;
-  int row_n = 0, len_n = 0, slot_n = -1;
-  if (it < n_items) { row_n = __ldg(item_row + it); len_n = __ldg(item_len + it); slot_n = __ldg(item_slot + it); }
-  uint32_t mine = 0;                     // rows this solver has taken
-  for (uint32_t i = (uint32_t)w; it < n_items; i += nsolv, it += nsolv, ++mine) {
-    const int row = row_n, len = len_n, wslot = slot_n;
-    {
-      const int64_t nx = it + nsolv;
-      if (nx < n_items) { row_n = __ldg(item_row + nx); len_n = __ldg(item_len + nx); slot_n = __ldg(item_slot + nx); }
-    }
+  // rows i = w, w + kSolvers, ... of this CTA's item sequence; slot = i % kSlots.  A row's metadata is loaded where it
+  // is needed, behind the wait for its slot or the back substitution (prefetched a row ahead, and held across the
+  // elimination, it took registers the elimination needs).
+  for (uint32_t mine = 0;; ++mine) {     // rows this solver has taken
+    const uint32_t i = (uint32_t)w + mine * (uint32_t)nsolv;
+    if (i >= n_items) break;
+    const int64_t it = rg->item_lo + i;
+    const int len = __ldg(ld_arg(args->item_len) + it), wslot = __ldg(ld_arg(args->item_slot) + it);
     const uint32_t sl = i % kSlots;
     { WS_T0(); umma::mbar_wait(&bars->sol_full[w], mine & 1); WS_ACC(w_slot); }
     const uint32_t S1 = slots + sl * kSlotBytes, S2 = S1 + 64 * kLd * 4, B1 = S2 + 64 * kLd * 4, B2 = B1 + 256;
     if (wslot >= 0) {
       // slice of a long row: park (A, b, n) in its workspace slot (layout of the SIMT path / reduce kernel)
-      float* W = workspace + (size_t)wslot * ((size_t)K * K + K + 4);
+      float* W = ld_arg(args->workspace) + (size_t)wslot * ((size_t)K * K + K + 4);
       for (int e = lane; e < K * K; e += 32) {
         const int m = e >> 6, n = e & 63;
         W[e] = lds32(S1 + (uint32_t)(m * kLd + n) * 4u) + lds32(S2 + (uint32_t)(m * kLd + n) * 4u) +
@@ -521,7 +585,7 @@ __device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars*
     f32x2 bb2;
     {
       WS_T0();
-      const float lam = reg * (float)len;
+      const float lam = ld_arg(args->reg) * (float)len;
       const uint32_t p1 = S1 + (uint32_t)(ti * kLd + tj) * 4u, p2 = S2 + (uint32_t)(ti * kLd + tj) * 4u;
       const uint32_t pt = S2 + (uint32_t)(tj * kLd + ti) * 4u;
 #pragma unroll
@@ -538,6 +602,7 @@ __device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars*
           R[tri(q, c)] = pack2(v[0], v[1]);
         }
       }
+      const float* gram_tiles = ld_arg(args->gram_tiles);
       if (gram_tiles != nullptr) {                           // implicit: + Y^T Y, already in this lane's tile order
         const float4* gp = reinterpret_cast<const float4*>(gram_tiles) + lane * 18;
 #pragma unroll
@@ -555,12 +620,13 @@ __device__ __noinline__ void solver_role(uint32_t slots, uint32_t scratch, Bars*
     }
     {
       WS_T0();
-      eliminate(R, bb2, P, Y, DI, ti, tj, lane);
+      eliminate(R, bb2, P, Y);
       WS_ACC(t_elim);
     }
     {
       WS_T0();
-      back_store(R, Y, DI, T, RH, ti, tj, lane, dst, dst_hl, row);
+      const int row = __ldg(ld_arg(args->item_row) + it);   // in flight during the back substitution
+      back_store(R, Y, DI, T, RH, ti, tj, lane, ld_arg(args->dst), ld_arg(args->dst_hl), row);
       WS_ACC(t_back);
     }
 #ifdef HALS_WS_PROFILE
@@ -585,6 +651,7 @@ als_ws64_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict__
   extern __shared__ uint8_t smem_dyn[];
   __shared__ Bars bars;
   __shared__ Range range;
+  __shared__ SolverArgs sargs;
   __shared__ uint32_t tmem_slot;
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -601,6 +668,7 @@ als_ws64_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict__
     umma::mbar_fence_init();
   }
   if (tid < 2) cta_range(&range, item_cost0, item_chunk0, n_items, tid);
+  if (tid == 64) sargs = SolverArgs{dst, dst_hl, workspace, gram_tiles, item_row, item_len, item_slot, reg};
   zero_r_blocks<K, kStages, kThreads>(base, tid);
   umma::fence_proxy_async();
   umma::fence_before_sync();
@@ -626,8 +694,8 @@ als_ws64_kernel(const int32_t* __restrict__ colidx, const uint32_t* __restrict__
   } else if (warp == kWarpMma) {
     mma_role(sbase, tmem, &bars, &range, chunk_cnt, implicit, lane);
   } else if (warp - kWarpSolver < nsolv) {
-    solver_role(slots, scratch + (uint32_t)(warp - kWarpSolver) * kScratchBytes, &bars, dst, dst_hl, workspace, reg, item_row,
-                item_len, item_slot, gram_tiles, &range, nsolv, warp - kWarpSolver, lane);
+    solver_role(slots, scratch + (uint32_t)(warp - kWarpSolver) * kScratchBytes, &bars, &sargs, &range, nsolv,
+                warp - kWarpSolver, lane);
   } else {
     scaler_role(sbase, &bars, &range, lane);
   }
@@ -654,7 +722,7 @@ als_reduce_solve64_warp_kernel(const float* __restrict__ workspace, float* __res
                                const float* __restrict__ gram) {
   constexpr int SF = K * K + K + 4;
   __shared__ __align__(16) float sA[SF];
-  __shared__ __align__(16) uint8_t sScratch[kScratchBytes];
+  __shared__ __align__(512) uint8_t sScratch[kScratchBytes];   // P flips buffers by bit 8
   const int tid = threadIdx.x, lane = tid & 31;
   const int row = long_row[blockIdx.x];
   const int s0 = long_slot0[blockIdx.x], ns = long_nseg[blockIdx.x];
@@ -687,7 +755,7 @@ als_reduce_solve64_warp_kernel(const float* __restrict__ workspace, float* __res
   }
   f32x2 bb2 = pack2(sA[K * K + ti + 8 * tj], sA[K * K + ti + 4 + 8 * tj]);
   const uint32_t P = umma::smem_u32(sScratch), Y = P + 512, DI = Y + 256, T = DI + 256, RH = T + 256;
-  eliminate(R, bb2, P, Y, DI, ti, tj, lane);
+  eliminate(R, bb2, P, Y);
   back_store(R, Y, DI, T, RH, ti, tj, lane, dst, dst_hl, row);
 }
 

@@ -25,9 +25,9 @@ __host__ __device__ constexpr int stage_bytes(int K) { return (K / 32 + 1) * kBl
 #define WS_ACC(v) do { } while (0)
 #endif
 
-__device__ __forceinline__ void sts64_if(bool pred, uint32_t addr, f32x2 p) {
+__device__ __forceinline__ void sts64_if(uint32_t pred, uint32_t addr, f32x2 p) {
   asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p st.shared.b64 [%0], %1;\n\t}\n"
-               ::"r"(addr), "l"(p), "r"((uint32_t)pred) : "memory");
+               ::"r"(addr), "l"(p), "r"(pred) : "memory");
 }
 __device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* mbar) {
   asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];\n" ::"r"(umma::smem_u32(mbar)) : "memory");
