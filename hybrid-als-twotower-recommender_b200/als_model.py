@@ -11,6 +11,10 @@ Additive (keyword-only) extensions, none of which changes the reference behaviou
   ALSModel(..., nonnegative=False)                         Spark's nonnegative: factors >= 0 (NNLS half-steps)
   train(data, init_user_factors=None)                      explicit initial factors for parity runs
   predict_for_users(user_ids, item_ids)                    dense [U,I] block of scores (device)
+  recommend_for_all_users(num_items, *, exclude=None, as_arrays=False)            Spark's recommendForAllUsers
+  recommend_for_all_items(num_users, *, exclude=None, as_arrays=False)            Spark's recommendForAllItems
+  recommend_for_user_subset(dataset, num_items, *, exclude=None, as_arrays=False) Spark's recommendForUserSubset
+  recommend_for_item_subset(dataset, num_users, *, exclude=None, as_arrays=False) Spark's recommendForItemSubset
 """
 from __future__ import annotations
 
@@ -56,11 +60,19 @@ class ALSFactors:
         return i if i < len(self.user_ids) and self.user_ids[i] == user_id else -1
 
     def item_rows(self, items):
-        items = np.asarray(items)
-        pos = np.searchsorted(self.item_ids, items)
-        pos = np.clip(pos, 0, max(len(self.item_ids) - 1, 0))
-        ok = (self.item_ids[pos] == items) if len(self.item_ids) else np.zeros(len(items), bool)
-        return np.where(ok, pos, -1)
+        return _rows_of(self.item_ids, items)
+
+
+def _rows_of(sorted_ids, ids):
+    """Row of each id in a sorted id table, -1 where it is absent."""
+    ids = np.asarray(ids)
+    pos = np.searchsorted(sorted_ids, ids)
+    pos = np.clip(pos, 0, max(len(sorted_ids) - 1, 0))
+    ok = (sorted_ids[pos] == ids) if len(sorted_ids) else np.zeros(len(ids), bool)
+    return np.where(ok, pos, -1)
+
+
+MAX_RECOMMENDATIONS = 256   # longest list recommend_for_* returns (the top-k limit of hals_score_topk; Spark has none)
 
 
 def read_spark_als_dir(model_path):
@@ -227,6 +239,86 @@ class ALSModel:
         out = out.view(len(urows), len(irows))
         bad = torch.from_numpy((urows < 0)[:, None] | (irows < 0)[None, :]).to(dev)
         return out.masked_fill(bad, float("nan"))
+
+    # -- Spark's ALSModel.recommendFor* (additive) ------------------------------------------------------------------
+    # rating = the fp32 dot product of the two factor rows (it agrees with predict_for_users to fp32 rounding; the
+    # summation orders differ).  A list is ordered by rating descending, then ascending raw id (Spark leaves the order
+    # of ties unspecified), and is min(num, candidates) long.  Only rows whose user_present / item_present is set take
+    # part, as queries or as candidates.  num must be an int in [1, MAX_RECOMMENDATIONS].
+    # exclude: optional DataFrame of userId / itemId pairs (e.g. the training frame): each list leaves its pairs out
+    # and fills up with the next best (the item direction applies the same pairs transposed); a kept rating is the
+    # one it has without `exclude`.
+    # Returns a pandas DataFrame, one row per query id in ascending order: (<query id column>, recommendations = list
+    # of (id, rating)); as_arrays=True returns numpy (query_ids int64 [Q], rec_ids int64 [Q, num] (-1 padded),
+    # ratings float32 [Q, num] (-inf padded)) instead -- a frame of 1e6 x 100 tuples costs more on the host than the
+    # GPU work.
+
+    def recommend_for_all_users(self, num_items, *, exclude=None, as_arrays=False):
+        """Top num_items items of every user: Spark's recommendForAllUsers (see the notes above)."""
+        return self._recommend(True, None, num_items, exclude, as_arrays)
+
+    def recommend_for_all_items(self, num_users, *, exclude=None, as_arrays=False):
+        """Top num_users users of every item: Spark's recommendForAllItems."""
+        return self._recommend(False, None, num_users, exclude, as_arrays)
+
+    def recommend_for_user_subset(self, dataset, num_items, *, exclude=None, as_arrays=False):
+        """recommend_for_all_users for the distinct dataset["userId"] known to the model (unknown ids are dropped, as
+        in Spark's inner join): Spark's recommendForUserSubset."""
+        return self._recommend(True, dataset["userId"].values, num_items, exclude, as_arrays)
+
+    def recommend_for_item_subset(self, dataset, num_users, *, exclude=None, as_arrays=False):
+        """recommend_for_all_items for the distinct dataset["itemId"] known to the model: Spark's recommendForItemSubset."""
+        return self._recommend(False, dataset["itemId"].values, num_users, exclude, as_arrays)
+
+    def _recommend(self, for_users, subset, num, exclude, as_arrays, slab=65536):
+        if isinstance(num, bool) or not isinstance(num, (int, np.integer)) or not 1 <= num <= MAX_RECOMMENDATIONS:
+            raise ValueError(f"the number of recommendations must be an int in [1, {MAX_RECOMMENDATIONS}], got {num!r}")
+        if self.model is None:
+            raise ValueError("no trained or loaded model: call train() or load_model() first")
+        import torch
+        from .scoring import HybridScorer, exclusion_lists_by_id
+        m, num = self.model, int(num)
+        q_col, c_col = ("userId", "itemId") if for_users else ("itemId", "userId")
+        q_ids, q_fac, q_present = (m.user_ids, m.user_factors, m.user_present) if for_users else \
+            (m.item_ids, m.item_factors, m.item_present)
+        c_ids, c_fac, c_present = (m.item_ids, m.item_factors, m.item_present) if for_users else \
+            (m.user_ids, m.user_factors, m.user_present)
+        q_ok = q_present.cpu().numpy()
+        if subset is None:
+            q_rows = np.flatnonzero(q_ok)
+        else:
+            q_rows = _rows_of(q_ids, np.unique(np.asarray(subset)))
+            q_rows = q_rows[q_rows >= 0]
+            q_rows = q_rows[q_ok[q_rows]]
+        c_rows = np.flatnonzero(c_present.cpu().numpy())
+        dev = c_fac.device
+
+        def take(fac, rows):      # the whole table when every row takes part (no copy)
+            return fac if len(rows) == fac.shape[0] else fac[torch.from_numpy(rows).to(dev)]
+
+        n_q, n_c = len(q_rows), len(c_rows)
+        rec = np.full((n_q, num), -1, np.int64)
+        ratings = np.full((n_q, num), -np.inf, np.float32)
+        if n_q and n_c:
+            sc = HybridScorer(take(q_fac, q_rows), take(c_fac, c_rows), None, None)
+            excl = None
+            if exclude is not None:
+                def t(a):
+                    return torch.from_numpy(np.ascontiguousarray(np.asarray(a, dtype=np.int64))).to(dev)
+                excl = exclusion_lists_by_id(t(q_ids[q_rows]), t(c_ids[c_rows]), t(exclude[q_col].values),
+                                             t(exclude[c_col].values))
+            for u0 in range(0, n_q, slab):      # one scorer (candidates, workspace) for every slab of queries
+                u1 = min(n_q, u0 + slab)
+                idx, s = sc.topk_dot(num, u0, u1, exclude=excl)
+                idx = idx.cpu().numpy()
+                rec[u0:u1] = np.where(idx >= 0, c_ids[c_rows[np.maximum(idx, 0)]], -1)
+                ratings[u0:u1] = s.cpu().numpy()
+        query_ids = np.asarray(q_ids[q_rows], np.int64)
+        if as_arrays:
+            return query_ids, rec, ratings
+        lens = (rec >= 0).sum(1)
+        lists = [list(zip(r[:n].tolist(), s[:n].tolist())) for r, s, n in zip(rec, ratings, lens)]
+        return pd.DataFrame({q_col: query_ids, "recommendations": pd.Series(lists, dtype=object)})
 
     def _fallback_scores(self, items):
         """Placeholder rating of every item in `items` (als_model.py:83-86): mean rating of its <= 3 cosine neighbours

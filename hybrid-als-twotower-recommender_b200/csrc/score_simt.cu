@@ -142,7 +142,8 @@ score_simt_kernel(ScoreArgs A, float* __restrict__ extrema_out, const float* __r
       const float inf = __int_as_float(0x7f800000);
       ex = make_float4(inf, -inf, inf, -inf);
     } else {
-      ex = (u0 + tid < n_rows) ? reinterpret_cast<const float4*>(extrema_in)[u] : make_float4(0, 1, 0, 1);
+      // padding rows, and every row in raw mode (extrema_in == NULL: hals_score_topk), take the identity coefficients
+      ex = (u0 + tid < n_rows && extrema_in) ? reinterpret_cast<const float4*>(extrema_in)[u] : make_float4(0, 1, 0, 1);
       const BlendCoef c = blend_coef(ex);
       ex = make_float4(c.min_a, c.sc_a, c.min_t, c.sc_t);
     }

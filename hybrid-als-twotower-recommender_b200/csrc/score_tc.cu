@@ -12,6 +12,7 @@
 //           = blend - gamma_u; per-row threshold filter keeps the best CAP/2..CAP candidates
 //                                                      -> exact fp32 blend of the candidates,
 //                                                         sort, top-k (same code as the SIMT path)
+// hals_score_topk (ALS top-k by raw dot product) is pass 2 alone: no scaling, so no extrema are needed (blend_topk).
 // Each user carries a rigorous bound eps_u on |bf16 score - fp32 score| (2^-8 |u| max|i|, Cauchy-
 // Schwarz).  A result is accepted only if the exact k-th score clears (candidate threshold +
 // eps_u), i.e. no rejected item could belong to the answer; otherwise the user is flagged and
@@ -577,7 +578,8 @@ __global__ void score_exact_extrema_kernel(ExactArgs E, const float* __restrict_
 // Pass 2: candidates (bf16 score keys) -> exact fp32 blend keys, in place.  One warp per candidate stream
 // (stream, user): the user's two vectors stay in registers, every candidate's item rows are read with
 // coalesced 128-byte warp loads and reduced with shuffles (fp32; the summation order differs from the
-// CUDA-core path's sequential fmaf only in the last bits).
+// CUDA-core path's sequential fmaf only in the last bits).  extrema == NULL: raw mode (hals_score_topk, kt = 0,
+// w = (1, 0)) with the identity coefficients (0, 1, 0, 1), so the key is the ALS dot product itself.
 __global__ void score_exact_blend_kernel(ExactArgs E, const float* __restrict__ extrema, float w_als, float w_tt,
                                          int32_t item_offset, uint64_t* __restrict__ cand, const int32_t* __restrict__ cand_cnt,
                                          int cap, int sortn) {
@@ -593,7 +595,7 @@ __global__ void score_exact_blend_kernel(ExactArgs E, const float* __restrict__ 
   for (int q = 0; q < 4; ++q) ua[q] = (lane + 32 * q < E.ka) ? E.Ua[u * E.ua_stride + lane + 32 * q] : 0.f;
 #pragma unroll
   for (int q = 0; q < 2; ++q) ut[q] = (lane + 32 * q < E.kt) ? E.Ut[u * E.ut_stride + lane + 32 * q] : 0.f;
-  const float4 ex = reinterpret_cast<const float4*>(extrema)[u];
+  const float4 ex = extrema ? reinterpret_cast<const float4*>(extrema)[u] : make_float4(0.f, 1.f, 0.f, 1.f);
   const float ra = ex.y - ex.x, rt = ex.w - ex.z;
   const float sca = (ra != 0.f) ? 1.f / ra : 1.f, sct = (rt != 0.f) ? 1.f / rt : 1.f;
   uint64_t* buf = cand + (size_t)row * cap;
@@ -643,7 +645,8 @@ __global__ void score_select_kernel(int stride /* key slots per stream */, uint6
 
 // Pass 2 verification, after the cross-split merge: every item a split rejected had bf16 (blend - gamma) <= thr_s,
 // hence exact blend <= thr_s + gamma + eps.  The final list is provably the exact top-k when its k-th score
-// clears that bound for every split; otherwise the user is flagged for the exact re-run.
+// clears that bound for every split; otherwise the user is flagged for the exact re-run.  Raw mode (extrema == NULL):
+// the identity coefficients give alpha = w_als = 1 and gamma = 0 -- the accumulator is the bf16 dot product itself.
 __global__ void score_verify_kernel(const float* __restrict__ cand_thr, const float* __restrict__ extrema,
                                     const float2* __restrict__ unorm_scaled, const unsigned int* __restrict__ inorm_bits,
                                     float w_als, float w_tt, int64_t n_users, int n_splits, int topk,
@@ -654,7 +657,7 @@ __global__ void score_verify_kernel(const float* __restrict__ cand_thr, const fl
   float thr = ninf;
   for (int s = 0; s < n_splits; ++s) thr = fmaxf(thr, cand_thr[(size_t)s * n_users + u]);
   if (!(thr > ninf)) return;                            // nothing was ever rejected
-  const float4 ex = reinterpret_cast<const float4*>(extrema)[u];
+  const float4 ex = extrema ? reinterpret_cast<const float4*>(extrema)[u] : make_float4(0.f, 1.f, 0.f, 1.f);
   const float ra = ex.y - ex.x, rt = ex.w - ex.z;
   const float al = (ra != 0.f) ? w_als / ra : 0.f, be = (rt != 0.f) ? w_tt / rt : 0.f;
   const float gamma = -(al * ex.x + be * ex.z);
@@ -857,14 +860,16 @@ extern "C" int hals_score_extrema(const float* Ua, int64_t ua_stride, const floa
   return score_extrema_simt(O, n_users, n_items, extrema, list, fcount, st);   // exact re-run of unproven users
 }
 
-// The body of hals_score_blend_topk and hals_score_blend_topk_excluding (excl_rowptr == NULL: no exclusion).
+// The body of hals_score_blend_topk, hals_score_blend_topk_excluding (excl_rowptr == NULL: no exclusion) and
+// hals_score_topk (raw mode: extrema == NULL, kt = 0, w = (1, 0); the kernels that read extrema then use the identity
+// coefficients (0, 1, 0, 1), so every score is the plain dot product and no extrema pass is needed).
 static int blend_topk(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride, int ka, const float* Ut,
                       int64_t ut_stride, const float* It, int64_t it_stride, int kt, int64_t n_users, int64_t n_items,
                       const float* extrema, float w_als, float w_tt, int topk, int32_t item_offset, int32_t* out_idx,
                       float* out_score, const int64_t* excl_rowptr, const int32_t* excl_items, void* workspace,
                       size_t workspace_bytes, void* stream) {
   if (int rc = check_score_args(Ua, Ia, ka, Ut, It, kt, n_users, n_items)) return rc;
-  HALS_REQUIRE(extrema && out_idx && out_score && workspace, "null pointer");
+  HALS_REQUIRE(out_idx && out_score && workspace, "null pointer");
   HALS_REQUIRE(topk >= 1 && topk <= 256, "topk must be in [1,256]");
   const TcPlan p = make_plan(n_users, n_items, ka, kt, topk);
   if (workspace_bytes < p.total) return fail(HALS_ERR_WORKSPACE, "%s: workspace too small%s", __func__);
@@ -937,6 +942,7 @@ extern "C" int hals_score_blend_topk(const float* Ua, int64_t ua_stride, const f
                                      const float* extrema, float w_als, float w_tt, int topk,
                                      int32_t item_offset, int32_t* out_idx, float* out_score,
                                      void* workspace, size_t workspace_bytes, void* stream) {
+  HALS_REQUIRE(extrema, "null pointer");
   return blend_topk(Ua, ua_stride, Ia, ia_stride, ka, Ut, ut_stride, It, it_stride, kt, n_users, n_items, extrema, w_als,
                     w_tt, topk, item_offset, out_idx, out_score, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
@@ -949,6 +955,21 @@ extern "C" int hals_score_blend_topk_excluding(const float* Ua, int64_t ua_strid
                                                const int64_t* excl_rowptr, const int32_t* excl_items,
                                                void* workspace, size_t workspace_bytes, void* stream) {
   HALS_REQUIRE((excl_rowptr == nullptr) == (excl_items == nullptr), "excl_rowptr and excl_items must both be set or both NULL");
+  HALS_REQUIRE(extrema, "null pointer");
   return blend_topk(Ua, ua_stride, Ia, ia_stride, ka, Ut, ut_stride, It, it_stride, kt, n_users, n_items, extrema, w_als,
                     w_tt, topk, item_offset, out_idx, out_score, excl_rowptr, excl_items, workspace, workspace_bytes, stream);
+}
+
+extern "C" int hals_score_topk(const float* Q, int64_t q_stride, const float* C, int64_t c_stride, int k, int64_t n_q,
+                               int64_t n_c, int topk, int32_t c_offset, const int64_t* excl_rowptr,
+                               const int32_t* excl_items, int32_t* out_idx, float* out_score, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+  // every argument check comes before make_plan, whose SM count query is the first CUDA call
+  HALS_REQUIRE(k >= 1 && k <= 128, "k (the factor rank) must be in [1,128]");
+  HALS_REQUIRE(topk >= 1 && topk <= 256, "topk must be in [1,256]");
+  HALS_REQUIRE(n_q >= 0 && n_c >= 0, "negative size");
+  HALS_REQUIRE(Q && C && out_idx && out_score && workspace, "null pointer");
+  HALS_REQUIRE((excl_rowptr == nullptr) == (excl_items == nullptr), "excl_rowptr and excl_items must both be set or both NULL");
+  return blend_topk(Q, q_stride, C, c_stride, k, nullptr, 0, nullptr, 0, 0, n_q, n_c, nullptr, 1.f, 0.f, topk, c_offset,
+                    out_idx, out_score, excl_rowptr, excl_items, workspace, workspace_bytes, stream);
 }

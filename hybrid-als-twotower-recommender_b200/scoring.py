@@ -5,6 +5,9 @@ ALSModel.predict_for_user + TwoTowerModel.predict_for_user + adaptive_fusion + s
   pass 1  hals_score_extrema     per-user (min,max) of both models      [+ min/max all-reduce]
   pass 2  hals_score_blend_topk  blend + per-user top-k, scores never stored
           [+ all-to-all of the per-shard lists and hals_topk_merge when item-sharded]
+
+ALS-only top-k by raw dot product (HybridScorer.topk_dot, behind ALSModel.recommend_for_*) needs no extrema: it is
+pass 2 alone, hals_score_topk.
 """
 from __future__ import annotations
 
@@ -129,16 +132,17 @@ class HybridScorer:
         it = (None, 0) if self.It is None else (nat.ptr(self.It), self.It.stride(0))
         return ua, uas, ia[0], ia[1], self.ka, ut, uts, it[0], it[1], self.kt
 
-    def _workspace(self, n_users: int, k: int) -> torch.Tensor:
-        need = int(nat.lib().hals_score_workspace_bytes(n_users, self.n_items, self.ka, self.kt, k))
+    def _workspace(self, n_users: int, k: int, kt: int | None = None) -> torch.Tensor:
+        kt = self.kt if kt is None else kt
+        need = int(nat.lib().hals_score_workspace_bytes(n_users, self.n_items, self.ka, kt, k))
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         return self._ws
 
-    def flagged_users(self, n_users: int, k: int) -> int:
+    def flagged_users(self, n_users: int, k: int, dot: bool = False) -> int:
         """Users of the last call (same n_users, k) that the tensor-core path re-ran exactly; -1 if the call
-        took the CUDA-core path."""
-        off = int(nat.lib().hals_score_flag_counter_offset(n_users, self.n_items, self.ka, self.kt, k))
+        took the CUDA-core path.  dot=True: the last call was topk_dot."""
+        off = int(nat.lib().hals_score_flag_counter_offset(n_users, self.n_items, self.ka, 0 if dot else self.kt, k))
         if off < 0 or self._ws is None:
             return -1
         return int(self._ws[off:off + 4].view(torch.int32).item())
@@ -170,17 +174,21 @@ class HybridScorer:
         if exclude is None:
             nat.check(L.hals_score_blend_topk(*head, *tail), "hals_score_blend_topk")
         else:
-            rowptr, items = exclude
-            if rowptr.dtype != torch.int64 or items.dtype != torch.int32 or rowptr.numel() != self.n_users + 1:
-                raise ValueError("exclude must be (rowptr int64 [n_users+1], items int32) over the scorer's users")
-            if rowptr.device != self.device or items.device != self.device:
-                raise ValueError("exclude must live on the scorer's device")
-            rowptr, items = rowptr.contiguous(), items.contiguous()
-            if items.numel() == 0:            # a valid pointer for an empty list set
-                items = torch.zeros(1, dtype=torch.int32, device=self.device)
+            rowptr, items = self._check_exclude(exclude)
             nat.check(L.hals_score_blend_topk_excluding(*head, nat.ptr(rowptr[u0:]), nat.ptr(items), *tail),
                       "hals_score_blend_topk_excluding")
         return idx, sc
+
+    def _check_exclude(self, exclude):
+        rowptr, items = exclude
+        if rowptr.dtype != torch.int64 or items.dtype != torch.int32 or rowptr.numel() != self.n_users + 1:
+            raise ValueError("exclude must be (rowptr int64 [n_users+1], items int32) over the scorer's users")
+        if rowptr.device != self.device or items.device != self.device:
+            raise ValueError("exclude must live on the scorer's device")
+        rowptr, items = rowptr.contiguous(), items.contiguous()
+        if items.numel() == 0:            # a valid pointer for an empty list set
+            items = torch.zeros(1, dtype=torch.int32, device=self.device)
+        return rowptr, items
 
     def recommend(self, k: int, w_als: float, w_tt: float, u0: int = 0, u1: int | None = None, exclude=None):
         """Final top-k for users [u0,u1).  Item-sharded runs return, on every rank, the merged
@@ -189,6 +197,29 @@ class HybridScorer:
         u1 = self.n_users if u1 is None else u1
         ex = self.extrema(u0, u1)
         idx, sc = self.topk_local(ex, k, w_als, w_tt, u0, u1, exclude=exclude)
+        return exchange_topk(idx, sc, self.rank, self.world, merge_lists)
+
+    def topk_dot(self, k: int, u0: int = 0, u1: int | None = None, exclude=None):
+        """The raw counterpart of `recommend`: for users [u0,u1) the k items with the largest ALS dot product
+        <Ua[u], Ia[i]> (fp32; score descending, then lower item index; padded with -1 / -inf), in one pass over the
+        items (hals_score_topk: no extrema, no scaling).  The tower operands are ignored.  exclude and the item-sharded
+        result: as for `recommend`."""
+        if self.Ua is None or self.Ia is None:
+            raise ValueError("topk_dot needs the ALS operands (Ua, Ia)")
+        L = nat.lib()
+        u1 = self.n_users if u1 is None else u1
+        n = u1 - u0
+        self._workspace(n, k, kt=0)
+        idx = torch.empty((n, k), dtype=torch.int32, device=self.device)
+        sc = torch.empty((n, k), dtype=torch.float32, device=self.device)
+        xr = xi = None
+        if exclude is not None:
+            xr, xi = self._check_exclude(exclude)
+            xr = xr[u0:]
+        nat.check(L.hals_score_topk(nat.ptr(self.Ua[u0:u1]), self.Ua.stride(0), nat.ptr(self.Ia), self.Ia.stride(0),
+                                    self.ka, n, self.n_items, int(k), self.item_offset, nat.ptr(xr), nat.ptr(xi),
+                                    nat.ptr(idx), nat.ptr(sc), nat.ptr(self._ws), self._ws.numel(),
+                                    nat.current_stream()), "hals_score_topk")
         return exchange_topk(idx, sc, self.rank, self.world, merge_lists)
 
     def user_slice(self, u0, u1):

@@ -299,6 +299,25 @@ int hals_score_blend_topk_excluding(const float* Ua, int64_t ua_stride, const fl
                                     int32_t* out_idx, float* out_score, const int64_t* excl_rowptr /* [n_users+1] */,
                                     const int32_t* excl_items, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ALS top-k by raw dot product (Spark's ALSModel.recommendForAllUsers / recommendForAllItems and the subset forms;
+ * both directions are this one call, with the roles of the two factor tables swapped).  Q [n_q, k] and C [n_c, k] are
+ * fp32 row-major with the given row strides.  For every query row q: the topk columns c not in X_q with the largest
+ * <Q[q], C[c]>, fp32, ordered score descending then column index ascending, indices + c_offset, padded with -1 / -inf
+ * when fewer remain.  One pass over C: the tensor-core kernel of hals_score_blend_topk's pass 2 with the plain dot
+ * product as its score (no extrema, no scaling), candidates re-scored in fp32, rows it cannot prove exact re-run on
+ * the exact CUDA-core kernel; small calls run on that kernel alone.  The summation order differs between the two
+ * routes, so a score agrees with hals_als_predict to fp32 rounding, not bit for bit.
+ * k in [1,128]; topk in [1,256].  Exclusion CSR exactly as in hals_score_blend_topk_excluding (rows = query rows, ids
+ * in the global numbering local index + c_offset; both NULL = none, one NULL = HALS_ERR_INVALID); a kept column's score
+ * is bit-identical to the call without exclusions whenever the row takes the same route in both calls.  Every
+ * argument is checked before the first CUDA call.
+ * Workspace: hals_score_workspace_bytes(n_q, n_c, k, 0, topk); hals_score_flag_counter_offset(n_q, n_c, k, 0, topk)
+ * reports the route and the exactly re-run rows, as for the hybrid call. */
+int hals_score_topk(const float* Q, int64_t q_stride, const float* C, int64_t c_stride, int k, int64_t n_q, int64_t n_c,
+                    int topk, int32_t c_offset, const int64_t* excl_rowptr /* [n_q+1] */, const int32_t* excl_items,
+                    int32_t* out_idx /* [n_q,topk] */, float* out_score /* [n_q,topk] */, void* workspace,
+                    size_t workspace_bytes, void* stream);
+
 int hals_topk_merge(const int32_t* part_idx, const float* part_score, int n_parts,
                     int64_t n_users, int topk, int32_t* out_idx, float* out_score, void* stream);
 
