@@ -75,6 +75,7 @@ SIGNATURES = {
     "hals_als_sse_workspace_bytes": (c_sz, []),
     "hals_als_sse": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "hals_f1_at_k": (ctypes.c_int, [c_vp, c_i64, ctypes.c_int, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "hals_ranking_metrics": (ctypes.c_int, [c_vp, c_i64, ctypes.c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "hals_similar_items": (ctypes.c_int, [c_vp, ctypes.c_int, c_vp, c_i64, c_vp, c_i64, ctypes.c_double, c_vp, c_vp, c_vp]),
     "hals_tower_user": (ctypes.c_int, [ctypes.POINTER(TowerWeights), c_vp, c_i64, c_vp, c_i64, c_vp]),
     "hals_tower_item": (ctypes.c_int, [ctypes.POINTER(TowerWeights), c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp]),

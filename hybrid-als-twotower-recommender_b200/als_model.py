@@ -15,6 +15,9 @@ Additive (keyword-only) extensions, none of which changes the reference behaviou
   recommend_for_all_items(num_users, *, exclude=None, as_arrays=False)            Spark's recommendForAllItems
   recommend_for_user_subset(dataset, num_items, *, exclude=None, as_arrays=False) Spark's recommendForUserSubset
   recommend_for_item_subset(dataset, num_users, *, exclude=None, as_arrays=False) Spark's recommendForItemSubset
+  transform(dataset)                                       Spark's transform, honouring cold_start_strategy
+  evaluate_regression(dataset, metric_name="rmse")         RegressionEvaluator on transform(dataset)
+  evaluate_ranking(dataset, k=10, *, exclude=None)         RankingEvaluator on recommendForAllUsers(k) (hals_ranking_metrics)
 """
 from __future__ import annotations
 
@@ -70,6 +73,12 @@ def _rows_of(sorted_ids, ids):
     pos = np.clip(pos, 0, max(len(sorted_ids) - 1, 0))
     ok = (sorted_ids[pos] == ids) if len(sorted_ids) else np.zeros(len(ids), bool)
     return np.where(ok, pos, -1)
+
+
+def _on(values, dev, dtype=np.int64):
+    """Host values (numpy / pandas column) as a contiguous torch tensor of `dtype` on `dev`."""
+    import torch
+    return torch.from_numpy(np.ascontiguousarray(np.asarray(values, dtype=dtype))).to(dev)
 
 
 MAX_RECOMMENDATIONS = 256   # longest list recommend_for_* returns (the top-k limit of hals_score_topk; Spark has none)
@@ -271,10 +280,27 @@ class ALSModel:
         return self._recommend(False, dataset["itemId"].values, num_users, exclude, as_arrays)
 
     def _recommend(self, for_users, subset, num, exclude, as_arrays, slab=65536):
-        if isinstance(num, bool) or not isinstance(num, (int, np.integer)) or not 1 <= num <= MAX_RECOMMENDATIONS:
-            raise ValueError(f"the number of recommendations must be an int in [1, {MAX_RECOMMENDATIONS}], got {num!r}")
-        if self.model is None:
-            raise ValueError("no trained or loaded model: call train() or load_model() first")
+        q_col = "userId" if for_users else "itemId"
+        query_ids, cand_ids, slabs = self._topk_slabs(for_users, subset, num, exclude, slab)
+        rec = np.full((len(query_ids), num), -1, np.int64)
+        ratings = np.full((len(query_ids), num), -np.inf, np.float32)
+        for u0, u1, idx, s in slabs:
+            idx = idx.cpu().numpy()
+            rec[u0:u1] = np.where(idx >= 0, cand_ids[np.maximum(idx, 0)], -1)
+            ratings[u0:u1] = s.cpu().numpy()
+        if as_arrays:
+            return query_ids, rec, ratings
+        lens = (rec >= 0).sum(1)
+        lists = [list(zip(r[:n].tolist(), s[:n].tolist())) for r, s, n in zip(rec, ratings, lens)]
+        return pd.DataFrame({q_col: query_ids, "recommendations": pd.Series(lists, dtype=object)})
+
+    def _topk_slabs(self, for_users, subset, num, exclude, slab):
+        """What recommend_for_* and evaluate_ranking share: check num and the model, select the query rows (present;
+        the distinct known ids of `subset` when it is given) and the candidate rows (present).  Returns (query raw ids
+        int64 [n_q] ascending, candidate raw ids [n_c] ascending, slabs); iterating `slabs` runs the top-k slab by slab
+        and yields (u0, u1, idx, scores): device tensors [u1-u0, num] of candidate positions (-1 padded) and fp32
+        ratings (-inf padded) of query rows [u0, u1)."""
+        self._check_topk(num)
         import torch
         from .scoring import HybridScorer, exclusion_lists_by_id
         m, num = self.model, int(num)
@@ -296,29 +322,123 @@ class ALSModel:
         def take(fac, rows):      # the whole table when every row takes part (no copy)
             return fac if len(rows) == fac.shape[0] else fac[torch.from_numpy(rows).to(dev)]
 
-        n_q, n_c = len(q_rows), len(c_rows)
-        rec = np.full((n_q, num), -1, np.int64)
-        ratings = np.full((n_q, num), -np.inf, np.float32)
-        if n_q and n_c:
+        def slabs():
+            n_q, n_c = len(q_rows), len(c_rows)
+            if not (n_q and n_c):
+                return
             sc = HybridScorer(take(q_fac, q_rows), take(c_fac, c_rows), None, None)
             excl = None
             if exclude is not None:
-                def t(a):
-                    return torch.from_numpy(np.ascontiguousarray(np.asarray(a, dtype=np.int64))).to(dev)
-                excl = exclusion_lists_by_id(t(q_ids[q_rows]), t(c_ids[c_rows]), t(exclude[q_col].values),
-                                             t(exclude[c_col].values))
+                excl = exclusion_lists_by_id(_on(q_ids[q_rows], dev), _on(c_ids[c_rows], dev),
+                                             _on(exclude[q_col].values, dev), _on(exclude[c_col].values, dev))
             for u0 in range(0, n_q, slab):      # one scorer (candidates, workspace) for every slab of queries
                 u1 = min(n_q, u0 + slab)
-                idx, s = sc.topk_dot(num, u0, u1, exclude=excl)
-                idx = idx.cpu().numpy()
-                rec[u0:u1] = np.where(idx >= 0, c_ids[c_rows[np.maximum(idx, 0)]], -1)
-                ratings[u0:u1] = s.cpu().numpy()
-        query_ids = np.asarray(q_ids[q_rows], np.int64)
-        if as_arrays:
-            return query_ids, rec, ratings
-        lens = (rec >= 0).sum(1)
-        lists = [list(zip(r[:n].tolist(), s[:n].tolist())) for r, s, n in zip(rec, ratings, lens)]
-        return pd.DataFrame({q_col: query_ids, "recommendations": pd.Series(lists, dtype=object)})
+                yield (u0, u1, *sc.topk_dot(num, u0, u1, exclude=excl))
+
+        return np.asarray(q_ids[q_rows], np.int64), c_ids[c_rows], slabs()
+
+    # -- Spark's ALSModel.transform, RegressionEvaluator and RankingEvaluator (additive) --------------------------------
+
+    def transform(self, dataset):
+        """Spark's ALSModel.transform: a copy of `dataset` with a float32 "prediction" column, the fp32 dot product of
+        the user's and the item's factors (hals_als_predict), NaN where the user or the item is unknown or not present.
+        cold_start_strategy "drop" (the default) removes the NaN rows and keeps the index of the others; "nan" keeps
+        them.  Any other strategy raises ValueError."""
+        pred = self._predict_frame(dataset).cpu().numpy()
+        out = dataset.copy()
+        out["prediction"] = pred
+        return out[~np.isnan(pred)] if self._drop_cold() else out
+
+    def evaluate_regression(self, dataset, metric_name="rmse"):
+        """Spark's RegressionEvaluator(metricName=...).evaluate(model.transform(dataset)), label column
+        "average_review_rating": "rmse", "mse", "mae" or "r2" (1 - SS_res / SS_tot).  Sums in fp64 on the device.
+        NaN when a NaN prediction remains (cold_start_strategy "nan") or when no row is left."""
+        if metric_name not in ("rmse", "mse", "mae", "r2"):
+            raise ValueError(f"metric_name must be one of 'rmse', 'mse', 'mae', 'r2', got {metric_name!r}")
+        import torch
+        p = self._predict_frame(dataset)
+        y = _on(dataset["average_review_rating"].values, p.device, np.float64)
+        p = p.double()
+        if self._drop_cold():
+            keep = ~torch.isnan(p)
+            p, y = p[keep], y[keep]
+        if p.numel() == 0:
+            return float("nan")
+        err = y - p
+        if metric_name == "mae":
+            v = err.abs().mean()
+        elif metric_name == "r2":
+            v = 1.0 - (err * err).sum() / ((y - y.mean()) ** 2).sum()
+        else:
+            v = (err * err).mean()
+            v = v.sqrt() if metric_name == "rmse" else v
+        return float(v.item())
+
+    def evaluate_ranking(self, dataset, k=10, *, exclude=None):
+        """recommendForAllUsers(k) joined with `dataset`'s (userId, itemId) pairs as each user's relevant items, then
+        Spark's RankingEvaluator: a dict of the means over the users of precisionAtK, recallAtK, ndcgAtK,
+        meanAveragePrecisionAtK and meanAveragePrecision (see hals_ranking_metrics), plus numUsers (the users
+        evaluated) and numColdUsers (distinct users of `dataset` that are unknown or not present: like Spark's inner
+        join, they are not in the means).  Every pair counts as relevant; a rating threshold is the caller's filter on
+        `dataset`.  A relevant item the model cannot recommend still counts in the user's label set.
+        k: an int in [1, MAX_RECOMMENDATIONS]; exclude: as for recommend_for_all_users (e.g. the training frame).
+        The lists and per-user metrics stay on the device and are reduced once; of the results only the five means come
+        back.  The id joins (test users, label and exclusion lists) still synchronise with the host for their sizes."""
+        return self._evaluate_ranking(dataset, k, exclude)
+
+    def _evaluate_ranking(self, dataset, k, exclude, slab=65536):
+        self._check_topk(k)
+        import torch
+        from .evaluation import RANKING_METRICS, ranking_metrics_batch
+        from .scoring import label_lists_by_id
+        dev = self.model.item_factors.device
+        users, items = _on(dataset["userId"].values, dev), _on(dataset["itemId"].values, dev)
+        distinct = torch.unique(users).cpu().numpy()   # the test users, deduplicated on the device
+        query_ids, cand_ids, slabs = self._topk_slabs(True, distinct, k, exclude, slab)
+        n_q = len(query_ids)
+        per_row = torch.zeros((n_q, 5), dtype=torch.float64, device=dev)
+        if n_q:
+            rowptr, labels = label_lists_by_id(_on(query_ids, dev), _on(cand_ids, dev), users, items)
+            for u0, u1, idx, _ in slabs:
+                per_row[u0:u1] = ranking_metrics_batch(idx, (rowptr[u0:u1 + 1], labels), k)
+        means = per_row.mean(0).cpu().tolist()          # NaN when no user is left, as Spark's mean of nothing
+        res = dict(zip(RANKING_METRICS, means))
+        res["numUsers"] = n_q
+        res["numColdUsers"] = len(distinct) - n_q
+        return res
+
+    def _check_topk(self, num):
+        """The argument checks of recommend_for_* and evaluate_ranking, made before any device work."""
+        if isinstance(num, bool) or not isinstance(num, (int, np.integer)) or not 1 <= num <= MAX_RECOMMENDATIONS:
+            raise ValueError(f"the number of recommendations must be an int in [1, {MAX_RECOMMENDATIONS}], got {num!r}")
+        if self.model is None:
+            raise ValueError("no trained or loaded model: call train() or load_model() first")
+
+    def _drop_cold(self):
+        s = self.cold_start_strategy
+        if not isinstance(s, str) or s.lower() not in ("drop", "nan"):
+            raise ValueError(f"cold_start_strategy must be 'drop' or 'nan', got {s!r}")
+        return s.lower() == "drop"
+
+    def _predict_frame(self, dataset):
+        """fp32 device tensor of the predictions of dataset's (userId, itemId) rows, NaN for unknown / absent ids."""
+        self._drop_cold()
+        if self.model is None:
+            raise ValueError("no trained or loaded model: call train() or load_model() first")
+        import torch
+        from . import _native as nat
+        m = self.model
+        dev = m.item_factors.device
+        urows = _on(_rows_of(m.user_ids, dataset["userId"].values), dev)
+        irows = _on(_rows_of(m.item_ids, dataset["itemId"].values), dev)
+        out = torch.empty(urows.numel(), dtype=torch.float32, device=dev)
+        if out.numel():
+            X, Y = m.user_factors.contiguous(), m.item_factors.contiguous()
+            uu, ii = urows.clamp(min=0).to(torch.int32), irows.clamp(min=0).to(torch.int32)
+            nat.check(nat.lib().hals_als_predict(nat.ptr(X), nat.ptr(Y), m.rank, nat.ptr(uu), nat.ptr(ii), out.numel(),
+                                                 nat.ptr(m.user_present), nat.ptr(m.item_present), nat.ptr(out),
+                                                 nat.current_stream()), "hals_als_predict")
+        return out.masked_fill((urows < 0) | (irows < 0), float("nan"))
 
     def _fallback_scores(self, items):
         """Placeholder rating of every item in `items` (als_model.py:83-86): mean rating of its <= 3 cosine neighbours

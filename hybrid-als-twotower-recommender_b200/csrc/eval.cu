@@ -6,10 +6,81 @@
 //                       with similarity > 0.5, mean of their ratings or the global mean (O(items) sklearn calls per
 //                       cold item in the reference)
 // Both are exact restatements (integer set arithmetic; fp64 cosine, ties to the lower item position = the stable
-// sort over the dict order the reference uses).
+// sort over the dict order the reference uses).  Beside them:
+//   hals_ranking_metrics  Spark's RankingMetrics per row (precision@k, recall@k, NDCG@k, AP@k, AP), behind
+//                         ALSModel.evaluate_ranking
 #include "common.cuh"
 
 namespace hals {
+
+// One warp per row.  The list is read in 32-entry chunks: lane j holds entry base + j, binary-searches it in the row's
+// sorted labels, and a ballot gives each hit its rank among the hits so far (the running count carried across
+// chunks is what AP needs).  Each lane sums its own positions in fp64; the butterfly reduction at the end runs in a
+// fixed order, so the result is bitwise reproducible.  No atomics, no workspace.
+__global__ void ranking_metrics_kernel(const int32_t* __restrict__ pred, int64_t pred_stride, int k, int64_t n_rows,
+                                       const int64_t* __restrict__ rowptr, const int32_t* __restrict__ labels,
+                                       double* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (r >= n_rows) return;                                // warp-uniform
+  const int64_t lo = rowptr[r], na = rowptr[r + 1] - lo;
+  const int32_t* a = labels + lo;
+  // |L|: distinct labels (sorted, so a label counts where it differs from its predecessor; Spark builds lab.toSet)
+  int64_t distinct = 0;
+  for (int64_t j = lane; j < na; j += 32) distinct += (j == 0 || a[j] != a[j - 1]) ? 1 : 0;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) distinct += __shfl_xor_sync(0xffffffffu, distinct, o);
+  double* o5 = out + r * 5;
+  if (distinct == 0) {                                    // Spark returns 0 for every metric of an empty label set
+    if (lane < 5) o5[lane] = 0.0;
+    return;
+  }
+  const int32_t* p = pred + r * pred_stride;
+  const unsigned below = (1u << lane) - 1u;
+  int carried = 0;                                        // hits before the current chunk
+  double dcg = 0.0, ap = 0.0, idcg = 0.0;
+  for (int64_t base = 0; base < k; base += 32) {
+    const int64_t e = base + lane;
+    const int32_t item = e < k ? p[e] : -1;
+    // the list ends at its first negative entry (the top-k kernels pad with -1) or at k
+    const unsigned ended = __ballot_sync(0xffffffffu, item < 0);
+    const bool valid = (ended & (below | (1u << lane))) == 0;
+    bool hit = false;
+    if (valid) {
+      int64_t l = 0, h = na;                              // lower bound in the sorted labels
+      while (l < h) {
+        const int64_t m = (l + h) >> 1;
+        if (a[m] < item) l = m + 1; else h = m;
+      }
+      hit = l < na && a[l] == item;
+    }
+    const unsigned hits = __ballot_sync(0xffffffffu, hit);
+    if (hit) {
+      const double g = 1.0 / log2((double)(e + 2));
+      dcg += g;
+      ap += (double)(carried + __popc(hits & below) + 1) / (double)(e + 1);
+    }
+    carried += __popc(hits);
+    if (ended) break;                                     // warp-uniform
+  }
+  // ideal DCG: a hit at each of the first min(|L|, k) positions
+  const int64_t n_ideal = distinct < (int64_t)k ? distinct : (int64_t)k;
+  for (int64_t i = lane; i < n_ideal; i += 32) idcg += 1.0 / log2((double)(i + 2));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    dcg += __shfl_xor_sync(0xffffffffu, dcg, o);
+    ap += __shfl_xor_sync(0xffffffffu, ap, o);
+    idcg += __shfl_xor_sync(0xffffffffu, idcg, o);
+  }
+  if (lane == 0) {
+    const double nl = (double)distinct;
+    o5[0] = (double)carried / (double)k;
+    o5[1] = (double)carried / nl;
+    o5[2] = dcg / idcg;
+    o5[3] = ap / (double)n_ideal;
+    o5[4] = ap / nl;
+  }
+}
 
 // one warp per user: predicted[u][0..k) (first k valid entries of a score-sorted list) vs the sorted item list
 // actual_items[rowptr[u] .. rowptr[u+1])
@@ -118,6 +189,23 @@ extern "C" int hals_f1_at_k(const int32_t* pred_idx, int64_t pred_stride, int k,
   if (n_users == 0) return 0;
   f1_at_k_kernel<<<(unsigned)((n_users + 7) / 8), 256, 0, (cudaStream_t)stream>>>(pred_idx, pred_stride, k, actual_rowptr,
                                                                                  actual_items, n_users, f1, true_positives);
+  HALS_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int hals_ranking_metrics(const int32_t* pred_idx, int64_t pred_stride, int k, int64_t n_rows,
+                                    const int64_t* label_rowptr, const int32_t* label_items, double* out,
+                                    void* stream) {
+  HALS_REQUIRE(pred_idx, "pred_idx is null");
+  HALS_REQUIRE(label_rowptr, "label_rowptr is null");
+  HALS_REQUIRE(label_items, "label_items is null");
+  HALS_REQUIRE(out, "out is null");
+  HALS_REQUIRE(k >= 1, "k must be >= 1");
+  HALS_REQUIRE(pred_stride >= k, "pred_stride must be >= k");
+  HALS_REQUIRE(n_rows >= 0, "n_rows must be >= 0");
+  if (n_rows == 0) return 0;
+  ranking_metrics_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
+      pred_idx, pred_stride, k, n_rows, label_rowptr, label_items, out);
   HALS_LAUNCH_CHECK();
   return 0;
 }

@@ -26,3 +26,37 @@ def f1_at_k_batch(pred_idx, actual_lists, k=10):
     nat.check(nat.lib().hals_f1_at_k(nat.ptr(pred_idx), pred_idx.stride(0), int(k), nat.ptr(rp), nat.ptr(it), U,
                                      nat.ptr(out), None, nat.current_stream()), "hals_f1_at_k")
     return out
+
+
+RANKING_METRICS = ("precisionAtK", "recallAtK", "ndcgAtK", "meanAveragePrecisionAtK", "meanAveragePrecision")
+
+
+def ranking_metrics_batch(pred_idx, labels, k):
+    """Spark's RankingMetrics of every row in one launch (hals_ranking_metrics); the columns are RANKING_METRICS.
+
+    pred_idx: int32 device tensor [n, >=k] of ranked ids, each list cut at its first negative entry (the -1 padding of
+    the top-k kernels) and never repeating an id; labels: device CSR (rowptr int64 [n+1], items int32) of each row's
+    relevant ids, ascending within a row, repeats allowed (scoring.label_lists_by_id builds it from raw id pairs).
+    Returns a float64 device tensor [n, 5]."""
+    import torch
+    from . import _native as nat
+    rowptr, items = labels
+    n = int(pred_idx.shape[0])
+    if pred_idx.dtype != torch.int32 or pred_idx.dim() != 2 or not 1 <= int(k) <= pred_idx.shape[1]:
+        raise ValueError("pred_idx must be an int32 [n, >= k] tensor and k >= 1")
+    if rowptr.dtype != torch.int64 or items.dtype != torch.int32 or rowptr.numel() != n + 1:
+        raise ValueError("labels must be (rowptr int64 [n+1], items int32)")
+    dev = pred_idx.device
+    if rowptr.device != dev or items.device != dev:
+        raise ValueError("pred_idx and labels must live on the same device")
+    out = torch.empty((n, 5), dtype=torch.float64, device=dev)
+    if n == 0:
+        return out
+    if pred_idx.stride(1) != 1:
+        pred_idx = pred_idx.contiguous()
+    rowptr = rowptr.contiguous()
+    items = items.contiguous() if items.numel() else torch.zeros(1, dtype=torch.int32, device=dev)  # a valid pointer
+    nat.check(nat.lib().hals_ranking_metrics(nat.ptr(pred_idx), pred_idx.stride(0), int(k), n, nat.ptr(rowptr),
+                                             nat.ptr(items), nat.ptr(out), nat.current_stream()),
+              "hals_ranking_metrics")
+    return out

@@ -104,6 +104,18 @@ def exclusion_lists_by_id(user_ids: torch.Tensor, item_ids: torch.Tensor, pair_u
     return exclusion_lists(rows[q2], cols, user_ids.numel())
 
 
+def label_lists_by_id(user_ids: torch.Tensor, item_ids: torch.Tensor, pair_users: torch.Tensor,
+                      pair_items: torch.Tensor):
+    """Label CSR of a ranking evaluation (hals_ranking_metrics) from (raw user id, raw item id) pairs, in the format of
+    exclusion_lists_by_id: row r = user_ids[r], items = positions among the candidates item_ids, ascending within a row,
+    duplicates kept.  An item that is not a candidate (unknown to the model, or not present) still belongs to the
+    label set: it gets the position len(item_ids) + its rank among the distinct such ids, which no prediction matches.
+    Pairs whose user is not a row are ignored."""
+    distinct = torch.unique(pair_items.reshape(-1))
+    extra = distinct[~torch.isin(distinct, item_ids.reshape(-1))]
+    return exclusion_lists_by_id(user_ids, torch.cat([item_ids.reshape(-1), extra]), pair_users, pair_items)
+
+
 def shard_items(n_items: int, rank: int, world: int):
     """Contiguous equal item shards (item-sharded scoring): [begin, end) of this rank."""
     per = (n_items + world - 1) // world

@@ -202,6 +202,26 @@ int hals_similar_items(const double* features /* [n_items, n_features] */, int n
                        const double* ratings /* [n_items] */, int64_t n_items, const int32_t* queries,
                        int64_t n_queries, double global_mean, double* out, int32_t* out_neighbours, void* stream);
 
+/* hals_ranking_metrics: Spark's RankingMetrics (3.x: countRelevantItemRatio, averagePrecision, ndcgAt, binary
+ * relevance) for every row at once -- ALSModel.evaluate_ranking.
+ *   - the predicted list of row r is pred_idx[r*pred_stride .. r*pred_stride + k), cut at its first negative entry (the
+ *     -1 padding of the top-k kernels); n = its length.  PRECONDITION: a list never repeats an item (the top-k
+ *     kernels guarantee it); not checked on the device;
+ *   - the labels L of row r are label_items[label_rowptr[r] .. label_rowptr[r+1]).  PRECONDITION: sorted ascending
+ *     within a row; not checked on the device.  They may repeat: a repeat counts once (Spark's lab.toSet);
+ *   - out[r*5 + 0..4] (fp64), with hit(i) = pred[i] in L and every metric 0 when L is empty:
+ *       0 precision@k  #{i < n : hit(i)} / k      (k even when n < k)
+ *       1 recall@k     #{i < n : hit(i)} / |L|
+ *       2 NDCG@k       DCG / IDCG, DCG = sum_{i<n, hit(i)} 1/log2(i+2), IDCG = sum_{i<min(|L|,k)} 1/log2(i+2)
+ *       3 AP@k         sum_{i<n, hit(i)} (#hits in 0..i)/(i+1)  /  min(|L|, k)
+ *       4 AP           the same sum / |L|  (Spark's meanAveragePrecision when the list is the top-k list)
+ *   - one warp per row, no atomics, no workspace; the reductions run in a fixed order (bitwise reproducible);
+ *   - null pointers, k < 1, pred_stride < k, n_rows < 0: HALS_ERR_INVALID before any CUDA call; n_rows == 0 launches
+ *     nothing. */
+int hals_ranking_metrics(const int32_t* pred_idx, int64_t pred_stride, int k, int64_t n_rows,
+                         const int64_t* label_rowptr /* [n_rows+1] */, const int32_t* label_items,
+                         double* out /* [n_rows, 5] */, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * Two-tower forward.  Replaces the Keras graph built at src/two_tower_model.py:38-89 as
  * evaluated by Model.predict at src/two_tower_model.py:145.
