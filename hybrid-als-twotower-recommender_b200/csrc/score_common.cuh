@@ -1,5 +1,5 @@
 // Interfaces between the exact SIMT scoring path (score_simt.cu) and the tensor-core path / public
-// dispatch (score_tc.cu).
+// dispatch (score_tc.cu), and the min-max blend every hybrid kernel applies (score_simt.cu, score_lists.cu).
 #pragma once
 #include "common.cuh"
 
@@ -9,6 +9,19 @@ struct ScoreOperands {
   const float* Ua; int64_t ua_stride; const float* Ia; int64_t ia_stride; int ka;
   const float* Ut; int64_t ut_stride; const float* It; int64_t it_stride; int kt;
 };
+
+// blend coefficients of one user from its extrema (sklearn MinMaxScaler: zero range -> scale 1)
+struct BlendCoef { float min_a, sc_a, min_t, sc_t; };
+__device__ __forceinline__ BlendCoef blend_coef(const float4 ex) {
+  BlendCoef c;
+  const float ra = ex.y - ex.x, rt = ex.w - ex.z;
+  c.min_a = ex.x; c.sc_a = (ra != 0.f) ? 1.f / ra : 1.f;
+  c.min_t = ex.z; c.sc_t = (rt != 0.f) ? 1.f / rt : 1.f;
+  return c;
+}
+__device__ __forceinline__ float blend_value(const BlendCoef& c, float wa, float wt, float sa, float st) {
+  return fmaf(wa, (sa - c.min_a) * c.sc_a, wt * ((st - c.min_t) * c.sc_t));
+}
 
 size_t score_simt_workspace_bytes(int64_t n_users, int64_t n_items, int topk);
 size_t score_simt_list_workspace_bytes(int64_t n_users, int64_t n_items, int topk);

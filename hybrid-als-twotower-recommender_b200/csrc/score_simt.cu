@@ -66,19 +66,6 @@ __global__ void extrema_init_kernel(float* extrema, int64_t n_users) {
   }
 }
 
-// blend coefficients of one user from its extrema (sklearn MinMaxScaler: zero range -> scale 1)
-struct BlendCoef { float min_a, sc_a, min_t, sc_t; };
-__device__ __forceinline__ BlendCoef blend_coef(const float4 ex) {
-  BlendCoef c;
-  const float ra = ex.y - ex.x, rt = ex.w - ex.z;
-  c.min_a = ex.x; c.sc_a = (ra != 0.f) ? 1.f / ra : 1.f;
-  c.min_t = ex.z; c.sc_t = (rt != 0.f) ? 1.f / rt : 1.f;
-  return c;
-}
-__device__ __forceinline__ float blend_value(const BlendCoef& c, float wa, float wt, float sa, float st) {
-  return fmaf(wa, (sa - c.min_a) * c.sc_a, wt * ((st - c.min_t) * c.sc_t));
-}
-
 // true when the ascending list items[lo, hi) holds v
 __device__ __forceinline__ bool sorted_contains(const int32_t* __restrict__ items, int64_t lo, int64_t hi, int32_t v) {
   const int64_t end = hi;

@@ -231,6 +231,140 @@ class HybridRecommendationSystem:
             self.als_f1_score, self.twotower_f1_score = float(f_als[-1]), float(f_tt[-1])
         return f_als, f_tt
 
+    def get_hybrid_recommendations_batch(self, user_ids, item_features, candidates=None, actual_ratings_by_user=None,
+                                         top_k=5, *, as_arrays=False):
+        """What a loop of get_hybrid_recommendations(u, items_u, actual_u, top_k) over `user_ids` (in order) returns,
+        in a few launches (hals_score_blend_topk_lists) instead of several per user.
+
+        item_features: the candidate universe, one row per itemId with the tower's feature columns (itemId,
+        manufacturer_id, category_id, price, average_review_rating).  candidates: per user, the loop's `all_items`:
+        a list aligned with user_ids of id sequences (or DataFrames), or a 2-D int array [len(user_ids), L] padded with
+        -1 (e.g. the ids of ALSModel.recommend_for_all_users(N, as_arrays=True)); None = every universe item for every
+        user.  A list keeps the first occurrence of a repeated id; an id missing from item_features raises ValueError.
+        Each user's scores are min-max scaled over that user's own list, and users or items unknown to ALS take the
+        content-similarity placeholder, as in predict_for_user.
+
+        actual_ratings_by_user: None, or a sequence aligned with user_ids of dicts of rated ids (or None).  A non-empty
+        entry of a user with a non-empty list sets that user's weights from its own F1@10 pair
+        (evaluate_individual_models on its list); any other user keeps the weights of the nearest earlier user that
+        had one, or the current als_f1_score / twotower_f1_score.  Afterwards those two attributes hold what the loop
+        leaves.  Nothing is printed.
+
+        Returns a list of per-user lists of (item_id, score), best first, as the loop does; as_arrays=True returns
+        (ids int64 [U, top_k] padded with -1, scores float32 [U, top_k] padded with -inf) instead.  Every score is
+        bit-identical to the loop's.  Two differences from the loop: items of exactly equal score are ordered by their
+        position in the user's list (the loop orders them by Python set iteration, which is unspecified), and the F1
+        ranking compares a cold id's placeholder as fp32 where the loop compares the float64 value."""
+        import torch
+        from .scoring import blend_topk_lists, candidate_lists, sticky_weights
+        if not self.models_loaded:
+            raise ValueError("Models not loaded. Call load_models() first.")
+        if isinstance(top_k, bool) or not isinstance(top_k, (int, np.integer)) or not 1 <= top_k <= 256:
+            raise ValueError(f"top_k must be an int in [1, 256], got {top_k!r}")
+        user_ids = list(user_ids)
+        U = len(user_ids)
+        if actual_ratings_by_user is not None and len(actual_ratings_by_user) != U:
+            raise ValueError("actual_ratings_by_user must be aligned with user_ids")
+        m = self.als_model.model
+        dev = m.item_factors.device
+        universe = np.asarray(item_features["itemId"].values, dtype=np.int64)
+        rowptr, cand = candidate_lists(candidates, universe, U, dev)      # raises on unknown ids before any launch
+
+        urows = np.array([m.user_row(u) for u in user_ids], dtype=np.int64)
+        irows = m.item_rows(universe) if len(universe) else np.zeros(0, np.int64)
+        user_known = torch.from_numpy(urows >= 0).to(dev)
+        item_known = torch.from_numpy(irows >= 0).to(dev)
+        Ua = m.user_factors[torch.from_numpy(np.maximum(urows, 0)).to(dev)]
+        Ia = m.item_factors[torch.from_numpy(np.maximum(irows, 0)).to(dev)]
+        Ut = self.twotower_model.user_vectors(user_ids)
+        It = self.twotower_model.item_vectors(item_features)
+        # placeholders for the universe items some list scores with them: cold items, and every item of a cold user's list
+        need = ~item_known
+        cold_users = torch.nonzero(~user_known).reshape(-1)
+        if cold_users.numel():
+            lens = rowptr[1:] - rowptr[:-1]
+            n = lens[cold_users]
+            start = torch.repeat_interleave(rowptr[:-1][cold_users] - (torch.cumsum(n, 0) - n), n)
+            need[cand[start + torch.arange(int(n.sum()), device=dev)].long()] = True
+        fallback = torch.zeros(len(universe), dtype=torch.float32, device=dev)
+        need_rows = torch.nonzero(need).reshape(-1)
+        if need_rows.numel():
+            ph = self.als_model._fallback_scores(universe[need_rows.cpu().numpy()].tolist())
+            fallback[need_rows] = torch.tensor(ph, dtype=torch.float64, device=dev).float()
+        known = dict(user_known=user_known, item_known=item_known, als_fallback=fallback)
+
+        # weights: the F1@10 pair of every user with ratings, carried forward to the users without
+        # a user with an empty list changes nothing: the loop's tower prediction fails on it before any F1 is taken
+        lens = (rowptr[1:] - rowptr[:-1]).cpu().numpy()
+        rated = [j for j in range(U) if actual_ratings_by_user is not None and actual_ratings_by_user[j] is not None
+                 and len(actual_ratings_by_user[j]) > 0 and lens[j] > 0]
+        fa = ft = np.zeros(0)
+        if rated:
+            fa, ft = self._list_f1(rated, [actual_ratings_by_user[j] for j in rated], universe, rowptr, cand,
+                                   Ua, Ia, Ut, It, known)
+        w, (self.als_f1_score, self.twotower_f1_score) = sticky_weights(
+            U, rated, fa, ft, (self.als_f1_score, self.twotower_f1_score))
+        w = torch.from_numpy(w).to(dev)
+        pos, score = blend_topk_lists(Ua, Ia, Ut, It, rowptr, cand, top_k, row_weights=w, **known)
+        univ_d = torch.from_numpy(universe).to(dev)
+        ids = torch.where(pos >= 0, univ_d[cand[pos.clamp(min=0).long()].long()], -1).cpu().numpy()
+        score = score.cpu().numpy()
+        if as_arrays:
+            return ids, score
+        n_ok = (ids >= 0).sum(1)
+        return [list(zip(i[:n].tolist(), s[:n].astype(np.float64).tolist())) for i, s, n in zip(ids, score, n_ok)]
+
+    @staticmethod
+    def _list_f1(rows, actuals, universe, rowptr, cand, Ua, Ia, Ut, It, known):
+        """F1@10 of each model for the users `rows` over their own lists (compute_f1_score: each model's top 10 by raw
+        score, ties by list position, against the rated ids; a rated id outside the list still counts in |actual|).
+        The true positives come from hals_f1_at_k; F1 itself is computed in float64 as compute_f1_score computes it."""
+        import torch
+        from . import _native as nat
+        from .scoring import blend_topk_lists
+        dev = cand.device
+        k = 10
+        r = torch.tensor(rows, dtype=torch.int64, device=dev)
+        if len(rows) < rowptr.numel() - 1:                 # the lists of these rows alone
+            lens = (rowptr[1:] - rowptr[:-1])[r]
+            sub_ptr = torch.zeros(len(rows) + 1, dtype=torch.int64, device=dev)
+            sub_ptr[1:] = torch.cumsum(lens, 0)
+            src = torch.repeat_interleave(rowptr[:-1][r] - sub_ptr[:-1], lens) + torch.arange(int(sub_ptr[-1]), device=dev)
+            rowptr, cand = sub_ptr, cand[src]
+            Ua, Ut = Ua[r], Ut[r]
+            known = dict(known, user_known=known["user_known"][r])
+        ia, _ = blend_topk_lists(Ua, Ia, None, None, rowptr, cand, k, w_als=1.0, raw=True, **known)
+        it, _ = blend_topk_lists(None, None, Ut, It, rowptr, cand, k, w_tt=1.0, raw=True)
+        # predicted and rated items as universe rows; a rated id outside the universe gets a row no prediction has
+        order = np.argsort(universe, kind="stable")
+        srt = universe[order]
+        lists, n_actual = [], np.empty(len(rows), np.int64)
+        for j, a in enumerate(actuals):
+            ids = np.unique(np.asarray(list(a.keys() if hasattr(a, "keys") else a), dtype=np.int64))
+            p = np.clip(np.searchsorted(srt, ids), 0, max(len(srt) - 1, 0))
+            ok = srt[p] == ids if len(srt) else np.zeros(len(ids), bool)
+            lists.append(np.concatenate([order[p[ok]], len(universe) + np.arange(int((~ok).sum()))]).astype(np.int32))
+            n_actual[j] = len(ids)
+        a_ptr = np.zeros(len(rows) + 1, np.int64)
+        a_ptr[1:] = np.cumsum([len(x) for x in lists])
+        a_items = np.concatenate([np.sort(x) for x in lists])
+        a_ptr_d = torch.from_numpy(a_ptr).to(dev)
+        a_items_d = torch.from_numpy(a_items if len(a_items) else np.zeros(1, np.int32)).to(dev)
+        tps = []
+        for pred in (ia, it):
+            pred = torch.where(pred >= 0, cand[pred.clamp(min=0).long()], -1).to(torch.int32).contiguous()
+            f1 = torch.empty(len(rows), dtype=torch.float32, device=dev)
+            tp = torch.empty(len(rows), dtype=torch.int32, device=dev)
+            nat.check(nat.lib().hals_f1_at_k(nat.ptr(pred), pred.stride(0), k, nat.ptr(a_ptr_d), nat.ptr(a_items_d),
+                                             len(rows), nat.ptr(f1), nat.ptr(tp), nat.current_stream()), "hals_f1_at_k")
+            tps.append(tp.cpu().numpy().astype(np.float64))
+        out = []
+        for tp in tps:                                     # compute_f1_score's arithmetic, in float64
+            p, rc = tp / k, tp / n_actual
+            with np.errstate(invalid="ignore", divide="ignore"):
+                out.append(np.where(p + rc > 0, 2 * (p * rc) / (p + rc), 0.0))
+        return out[0], out[1]
+
     def cleanup(self):
         if self.als_model:
             self.als_model.stop_spark()

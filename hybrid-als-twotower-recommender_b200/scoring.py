@@ -26,6 +26,28 @@ def fusion_weights(als_f1: float, tt_f1: float):
     return (0.8, 0.2) if als_f1 > tt_f1 else (0.2, 0.8)
 
 
+def sticky_weights(n_users: int, rated, als_f1, tt_f1, f1_init):
+    """The weights a loop of get_hybrid_recommendations gives each of n_users users: users `rated` (ascending) have
+    their own F1 pair (als_f1[j], tt_f1[j] for rated[j]) and set the sticky F1 scalars; every other user keeps the pair
+    of the nearest earlier rated user, or f1_init before the first.  Returns (float32 [n_users, 2] of fusion_weights,
+    the F1 pair the loop leaves)."""
+    import numpy as np
+    fa = np.full(n_users, f1_init[0], np.float64)
+    ft = np.full(n_users, f1_init[1], np.float64)
+    if len(rated):
+        src = np.full(n_users, -1, np.int64)
+        src[list(rated)] = np.arange(len(rated))
+        src = np.maximum.accumulate(src)
+        have = src >= 0
+        fa[have] = np.asarray(als_f1, np.float64)[src[have]]
+        ft[have] = np.asarray(tt_f1, np.float64)[src[have]]
+    better = fa > ft
+    hi, lo = fusion_weights(1.0, 0.0)
+    w = np.stack([np.where(better, hi, lo), np.where(better, lo, hi)], 1).astype(np.float32).reshape(n_users, 2)
+    last = (float(als_f1[-1]), float(tt_f1[-1])) if len(rated) else (float(f1_init[0]), float(f1_init[1]))
+    return w, last
+
+
 def merge_lists(part_idx: torch.Tensor, part_score: torch.Tensor):
     """[P, U, k] partial lists -> [U, k] (score desc, index asc)."""
     L = nat.lib()
@@ -114,6 +136,115 @@ def label_lists_by_id(user_ids: torch.Tensor, item_ids: torch.Tensor, pair_users
     distinct = torch.unique(pair_items.reshape(-1))
     extra = distinct[~torch.isin(distinct, item_ids.reshape(-1))]
     return exclusion_lists_by_id(user_ids, torch.cat([item_ids.reshape(-1), extra]), pair_users, pair_items)
+
+
+def candidate_lists(candidates, universe_ids, n_rows: int, device):
+    """Per-row candidate lists -> the CSR of hals_score_blend_topk_lists: (rowptr int64 [n_rows+1], cand int32), cand
+    holding ROWS of the universe (positions in `universe_ids`, which must not repeat an id).
+
+    candidates: None (every universe item, in universe order, for every row); a 2-D integer array [n_rows, L] whose -1
+    entries are padding (what ALSModel.recommend_for_all_users(..., as_arrays=True) returns); or a sequence of n_rows
+    id sequences (a DataFrame stands for its itemId column).  Each list keeps the first occurrence of a repeated id.
+    An id that is not in the universe raises ValueError.  The join and the deduplication run on `device`."""
+    import numpy as np
+    univ_h = np.array(universe_ids, dtype=np.int64)
+    n_univ = len(univ_h)
+    if len(np.unique(univ_h)) != n_univ:
+        raise ValueError("item_features must list each itemId once")
+    if candidates is None:
+        rowptr = torch.arange(n_rows + 1, dtype=torch.int64, device=device) * n_univ
+        return rowptr, torch.arange(n_univ, dtype=torch.int32, device=device).repeat(n_rows)
+    if isinstance(candidates, (np.ndarray, torch.Tensor)) and candidates.ndim == 2:
+        if candidates.shape[0] != n_rows:
+            raise ValueError(f"candidates has {candidates.shape[0]} rows for {n_rows} users")
+        ids = torch.as_tensor(np.asarray(candidates) if isinstance(candidates, np.ndarray) else candidates,
+                              device=device).to(torch.int64)
+        rows = torch.arange(n_rows, device=device).repeat_interleave(ids.shape[1])
+        ids = ids.reshape(-1)
+        real = ids != -1
+        ids, rows = ids[real], rows[real]
+    else:
+        lists = list(candidates)
+        if len(lists) != n_rows:
+            raise ValueError(f"candidates has {len(lists)} lists for {n_rows} users")
+        lists = [np.asarray(c["itemId"].values if hasattr(c, "columns") else list(c), dtype=np.int64).reshape(-1)
+                 for c in lists]
+        lens = np.fromiter((len(c) for c in lists), dtype=np.int64, count=n_rows)
+        flat = np.concatenate(lists) if lens.sum() else np.zeros(0, np.int64)
+        ids = torch.from_numpy(flat).to(device)
+        rows = torch.repeat_interleave(torch.arange(n_rows, device=device), torch.from_numpy(lens).to(device))
+    univ = torch.from_numpy(univ_h).to(device)
+    srt, order = torch.sort(univ)
+    pos = torch.searchsorted(srt, ids).clamp(max=max(n_univ - 1, 0))
+    ok = srt[pos] == ids if n_univ else torch.zeros_like(ids, dtype=torch.bool)
+    if not bool(ok.all()):
+        raise ValueError(f"candidate ids missing from item_features: {ids[~ok][:5].tolist()}")
+    urow = order[pos]
+    # first occurrence of each (row, item): a stable sort keeps equal keys in list order
+    sk, so = torch.sort(rows * max(n_univ, 1) + urow, stable=True)
+    first = torch.ones_like(sk, dtype=torch.bool)
+    first[1:] = sk[1:] != sk[:-1]
+    keep = torch.empty_like(first)
+    keep[so] = first
+    rows, urow = rows[keep], urow[keep]
+    rowptr = torch.zeros(n_rows + 1, dtype=torch.int64, device=device)
+    rowptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n_rows), 0)
+    return rowptr, urow.to(torch.int32)
+
+
+def blend_topk_lists(Ua, Ia, Ut, It, rowptr, cand, topk: int, *, w_als: float = 0.0, w_tt: float = 0.0,
+                     row_weights=None, raw: bool = False, user_known=None, item_known=None, als_fallback=None):
+    """hals_score_blend_topk_lists: per-row candidate lists (see candidate_lists), each row min-max blended over its
+    own list (raw=True: w_als*s_als + w_tt*s_tt) and cut to its best `topk`.  Ua [n_rows, ka] / Ut [n_rows, kt] are the
+    rows' user operands, Ia [n, ka] / It [n, kt] the candidate rows' (one model may be None); user_known [n_rows] /
+    item_known [n] (bool or uint8) mark ids known to ALS, the others take als_fallback [n] as their ALS score;
+    row_weights [n_rows, 2] overrides (w_als, w_tt) row by row.  Returns (positions into cand int32, scores float32),
+    both [n_rows, topk], padded with -1 / -inf; ties go to the lower position."""
+    L = nat.lib()
+    ref_u = Ua if Ua is not None else Ut
+    ref_i = Ia if Ia is not None else It
+    if ref_u is None or ref_i is None:
+        raise ValueError("need the operands of at least one model")
+    Ua, Ia, Ut, It = (None if t is None else t.contiguous() for t in (Ua, Ia, Ut, It))
+    n_rows, n_cand_rows = int(ref_u.shape[0]), int(ref_i.shape[0])
+    ka = 0 if Ua is None else int(Ua.shape[1])
+    kt = 0 if Ut is None else int(Ut.shape[1])
+    dev = ref_u.device
+    if (Ua is None) != (Ia is None) or (Ut is None) != (It is None):
+        raise ValueError("each model needs both its user and its item operand")
+    for t, rows, k in ((Ua, n_rows, ka), (Ut, n_rows, kt), (Ia, n_cand_rows, ka), (It, n_cand_rows, kt)):
+        if t is not None and (t.dtype != torch.float32 or t.dim() != 2 or tuple(t.shape) != (rows, k) or t.device != dev):
+            raise ValueError("operands must be float32 [n_rows, k] (users) and [n, k] (items) on one device")
+    if rowptr.dtype != torch.int64 or rowptr.numel() != n_rows + 1 or cand.dtype != torch.int32:
+        raise ValueError("candidate lists must be (rowptr int64 [n_rows+1], cand int32)")
+
+    def vec(t, n, dtype, what):
+        if t is None:
+            return None
+        t = t.to(dtype) if t.dtype == torch.bool else t
+        if t.dtype != dtype or t.numel() != n or t.device != dev:
+            raise ValueError(f"{what} must be {dtype} [{n}] on the operands' device")
+        return t.contiguous()
+    user_known = vec(user_known, n_rows, torch.uint8, "user_known")
+    item_known = vec(item_known, n_cand_rows, torch.uint8, "item_known")
+    als_fallback = vec(als_fallback, n_cand_rows, torch.float32, "als_fallback")
+    row_weights = vec(row_weights, 2 * n_rows, torch.float32, "row_weights")
+    rowptr, cand = rowptr.contiguous(), cand.contiguous()
+    if cand.numel() == 0:                   # a valid pointer for an empty list set
+        cand = torch.zeros(1, dtype=torch.int32, device=dev)
+    n_total = int(rowptr[-1].item()) if n_rows else 0
+    ws = torch.empty(int(L.hals_score_lists_workspace_bytes(n_total, int(topk))), dtype=torch.uint8, device=dev)
+    pos = torch.empty((n_rows, int(topk)), dtype=torch.int32, device=dev)
+    score = torch.empty((n_rows, int(topk)), dtype=torch.float32, device=dev)
+
+    def op(t):
+        return (None, 0) if t is None else (nat.ptr(t), t.stride(0))
+    nat.check(L.hals_score_blend_topk_lists(*op(Ua), *op(Ia), ka, *op(Ut), *op(It), kt, n_rows, n_total,
+                                            nat.ptr(rowptr), nat.ptr(cand), nat.ptr(user_known), nat.ptr(item_known),
+                                            nat.ptr(als_fallback), nat.ptr(row_weights), float(w_als), float(w_tt),
+                                            int(bool(raw)), int(topk), nat.ptr(pos), nat.ptr(score), nat.ptr(ws),
+                                            ws.numel(), nat.current_stream()), "hals_score_blend_topk_lists")
+    return pos, score
 
 
 def shard_items(n_items: int, rank: int, world: int):

@@ -338,6 +338,37 @@ int hals_score_topk(const float* Q, int64_t q_stride, const float* C, int64_t c_
                     int32_t* out_idx /* [n_q,topk] */, float* out_score /* [n_q,topk] */, void* workspace,
                     size_t workspace_bytes, void* stream);
 
+/* Hybrid top-k over PER-ROW candidate lists: the reference's per-user call get_hybrid_recommendations(user, all_items,
+ * ...) (src/hybrid_system.py:95-116) for many users at once, each with its own all_items.  Row r (user operands
+ * Ua[r], Ut[r]) owns the positions p in [cand_rowptr[r], cand_rowptr[r+1]); c = cand[p] names a row of Ia / It /
+ * item_known / als_fallback.  For each position:
+ *   s_t = <Ut[r], It[c]>,  s_a = <Ua[r], Ia[c]>, or s_a = als_fallback[c] when user_known[r] == 0 or item_known[c] == 0
+ *   (the cold-id placeholder of ALSModel.predict_for_user; a NULL mask means all known).  Both dot products are one
+ *   fmaf per feature in ascending order from 0.f: bit-identical to hals_score_one_user.
+ *   raw == 0: blend = w_a*(s_a-min_a)/(max_a-min_a) + w_t*(s_t-min_t)/(max_t-min_t), min / max over the row's OWN
+ *             list, a zero range contributing 0 (hals_fuse_lists on that list, bit for bit);
+ *   raw == 1: blend = w_a*s_a + w_t*s_t (the identity coefficients of hals_score_topk's raw mode).
+ *   (w_a, w_t) = row_weights[2r], row_weights[2r+1] when row_weights is not NULL, else (w_als, w_tt).
+ * Output per row: the first topk positions by blend descending, then lower position; out_pos holds the absolute
+ * position p (int32) into cand, padded with -1 / -inf when the list is shorter.  An empty row is all padding; a list
+ * that repeats an item returns it at every position it holds.  Deterministic: no float atomics.
+ *   - ka <= 128, kt <= 64, ka + kt > 0; topk in [1,256]; n_rows, n_cand_total >= 0, n_cand_total <= INT32_MAX; null
+ *     operands as in hals_score_blend_topk; a mask needs als_fallback: HALS_ERR_INVALID before any CUDA call.
+ *     n_rows == 0 launches nothing.
+ *   - PRECONDITIONS (not checked on the device): cand_rowptr is non-decreasing with cand_rowptr[n_rows] <=
+ *     n_cand_total; every cand entry is a valid row of Ia, It (and of the masks / als_fallback when given).
+ *   - rows longer than 8192 positions are split across warps (partial extrema combined exactly, partial lists merged).
+ * workspace: hals_score_lists_workspace_bytes(n_cand_total, topk) (0 for invalid arguments). */
+size_t hals_score_lists_workspace_bytes(int64_t n_cand_total, int topk);
+int hals_score_blend_topk_lists(const float* Ua, int64_t ua_stride, const float* Ia, int64_t ia_stride, int ka,
+                                const float* Ut, int64_t ut_stride, const float* It, int64_t it_stride, int kt,
+                                int64_t n_rows, int64_t n_cand_total, const int64_t* cand_rowptr /* [n_rows+1] */,
+                                const int32_t* cand, const uint8_t* user_known /* [n_rows] */,
+                                const uint8_t* item_known, const float* als_fallback,
+                                const float* row_weights /* [n_rows,2] */, float w_als, float w_tt, int raw, int topk,
+                                int32_t* out_pos /* [n_rows,topk] */, float* out_score /* [n_rows,topk] */,
+                                void* workspace, size_t workspace_bytes, void* stream);
+
 int hals_topk_merge(const int32_t* part_idx, const float* part_score, int n_parts,
                     int64_t n_users, int topk, int32_t* out_idx, float* out_score, void* stream);
 
