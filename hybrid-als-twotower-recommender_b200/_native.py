@@ -46,6 +46,27 @@ class TowerWeights(ctypes.Structure):
     ]
 
 
+class TowerParams(ctypes.Structure):
+    """struct hals_tower_params (include/hals_b200.h): the tower tensors the training step mutates."""
+    _fields_ = [
+        ("embedding_size", c_i32), ("manu_dim", c_i32), ("cat_dim", c_i32), ("num_hidden", c_i32),
+        ("user_emb", c_vp), ("item_emb", c_vp), ("manu_emb", c_vp), ("cat_emb", c_vp),
+        ("num_w", c_vp), ("num_b", c_vp), ("out_w", c_vp), ("out_b", c_vp),
+        ("user_ln_g", c_vp), ("user_ln_b", c_vp), ("item_ln_g", c_vp), ("item_ln_b", c_vp),
+        ("ln_eps", c_f32),
+        ("num_users", c_i32), ("num_items", c_i32), ("num_manufacturers", c_i32), ("num_categories", c_i32),
+    ]
+
+
+class TowerBatch(ctypes.Structure):
+    """struct hals_tower_batch (include/hals_b200.h)."""
+    _fields_ = [
+        ("n", c_i64), ("user_ids", c_vp), ("item_ids", c_vp), ("manufacturer_ids", c_vp), ("category_ids", c_vp),
+        ("numeric", c_vp), ("labels", c_vp),
+        ("order_user", c_vp), ("order_item", c_vp), ("order_manufacturer", c_vp), ("order_category", c_vp),
+    ]
+
+
 # name -> (restype, argtypes); kept in one table so tests can check it against the header
 SIGNATURES = {
     "hals_abi_version": (ctypes.c_int, []),
@@ -79,6 +100,12 @@ SIGNATURES = {
     "hals_similar_items": (ctypes.c_int, [c_vp, ctypes.c_int, c_vp, c_i64, c_vp, c_i64, ctypes.c_double, c_vp, c_vp, c_vp]),
     "hals_tower_user": (ctypes.c_int, [ctypes.POINTER(TowerWeights), c_vp, c_i64, c_vp, c_i64, c_vp]),
     "hals_tower_item": (ctypes.c_int, [ctypes.POINTER(TowerWeights), c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp]),
+    "hals_tower_train_workspace_bytes": (c_sz, [ctypes.POINTER(TowerParams), c_i64]),
+    "hals_tower_train_step": (ctypes.c_int, [ctypes.POINTER(TowerParams), ctypes.POINTER(TowerBatch), c_i64, c_vp, c_sz,
+                                             c_vp, c_vp]),
+    "hals_tower_adam_step": (ctypes.c_int, [ctypes.POINTER(TowerParams), ctypes.POINTER(TowerParams),
+                                            ctypes.POINTER(TowerParams), ctypes.POINTER(TowerBatch), c_i64, c_vp, c_sz,
+                                            ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double, c_vp]),
     "hals_score_extrema": (ctypes.c_int, [c_vp, c_i64, c_vp, c_i64, ctypes.c_int, c_vp, c_i64, c_vp, c_i64,
                                           ctypes.c_int, c_i64, c_i64, c_vp, c_vp, c_sz, c_vp]),
     "hals_score_workspace_bytes": (c_sz, [c_i64, c_i64, ctypes.c_int, ctypes.c_int, ctypes.c_int]),

@@ -5,26 +5,9 @@
 // once per id and the result feeds the scoring GEMM.
 //   one warp per output row; Dense weights staged once per CTA in shared memory;
 //   LayerNormalization with Keras defaults (biased variance, eps inside the sqrt).
-#include "common.cuh"
+#include "tower_common.cuh"
 
 namespace hals {
-
-constexpr int kTowerThreads = 256;
-constexpr int kTowerMaxE = 64;
-
-// rows == 0: table size unknown, no check (ids are then trusted, as in ABI version 1 before the field existed)
-__device__ __forceinline__ bool in_table(int id, int rows) { return rows <= 0 ? id >= 0 : (id >= 0 && id < rows); }
-
-__device__ __forceinline__ void warp_layer_norm_store(float v0, float v1, int E, int lane, const float* g,
-                                                      const float* b, float eps, float* out) {
-  const bool h0 = lane < E, h1 = lane + 32 < E;
-  const float mean = warp_sum((h0 ? v0 : 0.f) + (h1 ? v1 : 0.f)) / (float)E;
-  const float d0 = h0 ? v0 - mean : 0.f, d1 = h1 ? v1 - mean : 0.f;
-  const float var = warp_sum(d0 * d0 + d1 * d1) / (float)E;
-  const float inv = 1.0f / sqrtf(var + eps);
-  if (h0) out[lane] = fmaf(d0 * inv, g[lane], b[lane]);
-  if (h1) out[lane + 32] = fmaf(d1 * inv, g[lane + 32], b[lane + 32]);
-}
 
 __global__ void __launch_bounds__(kTowerThreads)
 tower_user_kernel(hals_tower_weights w, const int32_t* __restrict__ ids, int64_t n, float* __restrict__ out,

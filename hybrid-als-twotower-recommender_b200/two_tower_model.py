@@ -6,8 +6,9 @@ libhals_b200.so: hals_tower_item / hals_tower_user precompute the tower outputs 
 (the reference recomputes the item tower for every user) and hals_score_one_user takes the
 dot products.  `self.model` is a TowerWeights holder instead of a keras.Model.
 
-Training (two_tower_model.py:91-121) is outside the north-star path; `train` is kept so the
-class stays usable end to end and runs a plain torch Adam/MSE loop over the same graph.
+Training (two_tower_model.py:91-121) runs on the GPU as well: `train` drives the fused training step and the
+multi-tensor Adam step of csrc/tower_train.cu (hals_tower_train_step / hals_tower_adam_step) behind the reference's
+signature.  The torch loop it replaced is kept as the test oracle, oracle/tower_train_oracle.py:train_reference.
 """
 from __future__ import annotations
 
@@ -83,6 +84,25 @@ class TowerParams:
         w.num_users, w.num_items = int(self.t["user_emb"].shape[0]), int(self.t["item_emb"].shape[0])
         w.num_manufacturers, w.num_categories = int(self.t["manu_emb"].shape[0]), int(self.t["cat_emb"].shape[0])
         return w
+
+
+TRAIN_IDS = (("userId", "user_emb"), ("itemId", "item_emb"), ("manufacturer_id", "manu_emb"),
+             ("category_id", "cat_emb"))
+
+
+def nat_params(p: TowerParams):
+    """struct hals_tower_params over the tensors of `p` (the training step and Adam mutate them in place)."""
+    from . import _native as nat
+    s = nat.TowerParams()
+    s.embedding_size = p.embedding_size
+    s.manu_dim, s.cat_dim = int(p.t["manu_emb"].shape[1]), int(p.t["cat_emb"].shape[1])
+    s.num_hidden = int(p.t["num_b"].shape[0])
+    for k in TowerParams.NAMES:
+        setattr(s, k, p.t[k].data_ptr())
+    s.ln_eps = LN_EPS
+    s.num_users, s.num_items = int(p.t["user_emb"].shape[0]), int(p.t["item_emb"].shape[0])
+    s.num_manufacturers, s.num_categories = int(p.t["manu_emb"].shape[0]), int(p.t["cat_emb"].shape[0])
+    return s
 
 
 class TwoTowerModel:
@@ -175,82 +195,121 @@ class TwoTowerModel:
         predictions = out.cpu().numpy()
         return list(zip(item_features["itemId"], predictions.flatten()))
 
-    # -- training (outside the north-star path; plain torch) ----------------------------------------
-    def _torch_forward(self, p, f, dev):
-        import torch
-        import torch.nn.functional as F
-        E = self.embedding_size
-
-        def rows(table, ids):
-            # an id outside its table reads as a zero embedding row: what the tower kernels (csrc/towers.cu) and a Keras
-            # Embedding on the GPU do -- validation users never seen in training land here
-            ids = torch.as_tensor(np.asarray(ids), device=dev).long()
-            ok = (ids >= 0) & (ids < table.shape[0])
-            return table[torch.where(ok, ids, torch.zeros_like(ids))] * ok.unsqueeze(1).to(table.dtype)
-
-        u = F.layer_norm(rows(p["user_emb"], f["user_in"]), (E,), p["user_ln_g"], p["user_ln_b"], LN_EPS)
-        num = torch.as_tensor(np.asarray(f["numeric_in"], dtype=np.float32), device=dev)
-        h = torch.relu(num @ p["num_w"] + p["num_b"])
-        cat = torch.cat([rows(p["item_emb"], f["item_id_in"]), rows(p["manu_emb"], f["manufacturer_in"]),
-                         rows(p["cat_emb"], f["category_in"]), h], dim=1)
-        i = F.layer_norm(cat @ p["out_w"] + p["out_b"], (E,), p["item_ln_g"], p["item_ln_b"], LN_EPS)
-        return (u * i).sum(dim=1)
-
+    # -- training (csrc/tower_train.cu) -----------------------------------------------------------------
     def train(self, train_data, val_data=None, batch_size=256, epochs=10):
-        """Adam(lr) on MSE with EarlyStopping(patience=3, restore_best_weights) when validation data
-        is given (two_tower_model.py:91-121).  Returns a dict of per-epoch losses."""
+        """Adam(lr, eps=1e-7) on MSE with EarlyStopping(patience=3, restore_best_weights) when validation data is
+        given (two_tower_model.py:91-121).  Returns a dict of per-epoch losses.
+
+        Every step runs on the GPU: hals_tower_train_step (fused forward and backward of the batch) and
+        hals_tower_adam_step (one Adam step over every parameter, dense moments).  Per epoch the host draws the
+        permutation (torch.randperm, seeded 0), uploads it once and reads the per-step losses and the validation loss
+        once; there is no host synchronisation per step.  Steps are bitwise reproducible.  The validation loss runs
+        the tower kernels on the pre-scaled features and reduces in fp64.
+
+        Supported widths are those of the tower kernels: embedding_size in [1, 64] (ValueError otherwise, before any
+        device work; predict_for_user and item_vectors reject wider models too), and manufacturer / category / hidden
+        widths whose training step fits in shared memory (the reference widths 8 / 8 / 16 at E = 50 use 38 KB of 200 KB)."""
         import torch
+        from . import _native as nat
+        E = int(self.model.embedding_size if self.model is not None else self.embedding_size)
+        if not 1 <= E <= 64:
+            raise ValueError(f"embedding_size must be in [1, 64] for the GPU trainer (got {E})")
         if self.model is None:
             self.build_model()
         dev = self.model.t["user_emb"].device
-        params = {k: v.clone().requires_grad_(True) for k, v in self.model.t.items()}
-        opt = torch.optim.Adam(list(params.values()), lr=self.learning_rate, eps=1e-7)
         has_val = val_data is not None and len(val_data) > 0
         # Embedding ids are table rows (two_tower_model.py:47-62).  Keras on the CPU raises InvalidArgumentError for a
         # TRAINING id outside its table: checked here on the host.  (Validation rows may name users / items the tables
         # do not have -- the reference's own hyperparameter_tuning holds out whole users -- they read as zero rows.)
-        for frame in (train_data,):
-            for col, table in (("userId", "user_emb"), ("itemId", "item_emb"), ("manufacturer_id", "manu_emb"),
-                               ("category_id", "cat_emb")):
-                ids = frame[col].values
-                n_rows = int(self.model.t[table].shape[0])
-                if len(ids) and (ids.min() < 0 or ids.max() >= n_rows):
-                    raise IndexError(f"{col}: ids must lie in [0, {n_rows}) (found {int(ids.min())}..{int(ids.max())})")
+        for col, table in TRAIN_IDS:
+            ids = train_data[col].values
+            n_rows = int(self.model.t[table].shape[0])
+            if len(ids) and (ids.min() < 0 or ids.max() >= n_rows):
+                raise IndexError(f"{col}: ids must lie in [0, {n_rows}) (found {int(ids.min())}..{int(ids.max())})")
+        n = len(train_data)
+        starts = range(0, n, batch_size)   # TypeError / ValueError for a batch size range() rejects, as before
         tf = self._prepare_features(train_data)
-        y = torch.as_tensor(train_data["average_review_rating"].values.astype(np.float32), device=dev)
         vf = self._prepare_features(val_data) if has_val else None
-        vy = torch.as_tensor(val_data["average_review_rating"].values.astype(np.float32), device=dev) if has_val else None
         if has_val:  # _prepare_features re-fits the scaler (reference behaviour); keep the train fit for predict
             tf = self._prepare_features(train_data)
-        n = len(train_data)
+
+        def ids32(a):  # ids beyond int32 stay outside every table
+            return torch.from_numpy(np.clip(np.asarray(a, dtype=np.int64), -1, 2 ** 31 - 1).astype(np.int32)).to(dev)
+
+        def floats(a):
+            return torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dev)
+
+        feats = [ids32(tf[k]) for k in ("user_in", "item_id_in", "manufacturer_in", "category_in")]
+        num, y = floats(tf["numeric_in"]), floats(train_data["average_review_rating"].values)
+        rows = [int(self.model.t[t].shape[0]) for _, t in TRAIN_IDS]
+        params = TowerParams({k: v.detach().clone().contiguous() for k, v in self.model.t.items()}, E)
+        moments = [TowerParams({k: torch.zeros_like(v) for k, v in params.t.items()}, E) for _ in range(2)]
+        P, M, V = (nat_params(x) for x in (params, *moments))
+        L = nat.lib()
+        stream = nat.current_stream()
+        ws_bytes = int(L.hals_tower_train_workspace_bytes(P, max(1, min(batch_size, n)) if len(starts) else 1))
+        ws = torch.zeros(ws_bytes, dtype=torch.uint8, device=dev)
+        losses = torch.empty(max(len(starts), 1), dtype=torch.float32, device=dev)
+        if has_val:
+            nv = len(val_data)
+            vw = params.struct(None)      # identity scaler: the validation numerics are scaled on the host
+            v_ids = [ids32(vf[k]) for k in ("user_in", "item_id_in", "manufacturer_in", "category_in")]
+            v_num, v_y = floats(vf["numeric_in"]), floats(val_data["average_review_rating"].values)
+            v_rows = torch.arange(nv, dtype=torch.int32, device=dev)
+            uv, iv = (torch.empty((nv, E), dtype=torch.float32, device=dev) for _ in range(2))
+            sse, cnt = torch.empty(1, dtype=torch.float64, device=dev), torch.empty(1, dtype=torch.int64, device=dev)
+            sse_ws = torch.empty(int(L.hals_als_sse_workspace_bytes()), dtype=torch.uint8, device=dev)
+            best_t = {k: torch.empty_like(v) for k, v in params.t.items()}
+        batch = nat.TowerBatch()
         history = {"loss": [], "val_loss": []}
-        best, best_state, bad = float("inf"), None, 0
+        best, have_best, bad, t = float("inf"), False, 0, 0
         g = torch.Generator(device="cpu").manual_seed(0)
         for _ in range(int(epochs)):
-            perm = torch.randperm(n, generator=g).numpy()
+            perm = torch.randperm(n, generator=g).to(dev)
+            if len(starts):
+                ep_ids = [f[perm] for f in feats]
+                ep_num, ep_y = num[perm].contiguous(), y[perm]
+                # each batch's ids sorted stably (key: batch index, then id): the order the Adam step sums rows in
+                b_of = torch.arange(n, device=dev) // batch_size
+                orders = [(torch.sort(b_of * r + e.long(), stable=True).indices - b_of * batch_size).to(torch.int32)
+                          for e, r in zip(ep_ids, rows)]
+                for si, s in enumerate(starts):
+                    t += 1
+                    batch.n = min(batch_size, n - s)
+                    batch.user_ids, batch.item_ids, batch.manufacturer_ids, batch.category_ids = (
+                        a.data_ptr() + 4 * s for a in ep_ids)
+                    batch.numeric, batch.labels = ep_num.data_ptr() + 8 * s, ep_y.data_ptr() + 4 * s
+                    batch.order_user, batch.order_item, batch.order_manufacturer, batch.order_category = (
+                        a.data_ptr() + 4 * s for a in orders)
+                    nat.check(L.hals_tower_train_step(P, batch, t, nat.ptr(ws), ws_bytes,
+                                                      losses.data_ptr() + 4 * si, stream), "hals_tower_train_step")
+                    nat.check(L.hals_tower_adam_step(P, M, V, batch, t, nat.ptr(ws), ws_bytes, self.learning_rate,
+                                                     0.9, 0.999, 1e-7, stream), "hals_tower_adam_step")
+            if has_val:
+                nat.check(L.hals_tower_user(vw, nat.ptr(v_ids[0]), nv, nat.ptr(uv), E, stream), "hals_tower_user")
+                nat.check(L.hals_tower_item(vw, nat.ptr(v_ids[1]), nat.ptr(v_ids[2]), nat.ptr(v_ids[3]), nat.ptr(v_num),
+                                            nv, nat.ptr(iv), E, stream), "hals_tower_item")
+                nat.check(L.hals_als_sse(nat.ptr(uv), nat.ptr(iv), E, nat.ptr(v_rows), nat.ptr(v_rows), nat.ptr(v_y),
+                                         nv, nat.ptr(sse), nat.ptr(cnt), nat.ptr(sse_ws), sse_ws.numel(), stream),
+                          "hals_als_sse")
+            step_losses = losses[:len(starts)].cpu().numpy()     # the epoch's one read-back
             tot = 0.0
-            for s in range(0, n, batch_size):
-                b = perm[s:s + batch_size]
-                fb = {k: np.asarray(v)[b] for k, v in tf.items()}
-                loss = ((self._torch_forward(params, fb, dev) - y[torch.as_tensor(b, device=dev)]) ** 2).mean()
-                opt.zero_grad(set_to_none=True)
-                loss.backward()
-                opt.step()
-                tot += float(loss.detach()) * len(b)
+            for s, ls in zip(starts, step_losses):
+                tot += float(ls) * min(batch_size, n - s)
             history["loss"].append(tot / max(n, 1))
             if has_val:
-                with torch.no_grad():
-                    vl = float(((self._torch_forward(params, vf, dev) - vy) ** 2).mean())
+                vl = float(sse.item()) / nv
                 history["val_loss"].append(vl)
                 if vl < best:
-                    best, bad = vl, 0
-                    best_state = {k: v.detach().clone() for k, v in params.items()}
+                    best, bad, have_best = vl, 0, True
+                    for k, v in params.t.items():
+                        best_t[k].copy_(v)
                 else:
                     bad += 1
                     if bad >= 3:
                         break
-        final = best_state if best_state is not None else {k: v.detach() for k, v in params.items()}
-        self.model = TowerParams({k: v.contiguous() for k, v in final.items()}, self.embedding_size)
+        final = best_t if has_val and have_best else params.t
+        self.model = TowerParams(final, E)
         self.is_trained = True
         return history
 

@@ -264,6 +264,76 @@ int hals_tower_item(const hals_tower_weights* w, const int32_t* item_ids,
                     int64_t out_stride, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Two-tower training.  Replaces model.fit (Adam, MSE, src/two_tower_model.py:91-121) for one minibatch at a time:
+ *   pred_r = <LN_u(E_user[u_r]), LN_i(W_o . concat(E_item[i_r], E_manu[m_r], E_cat[c_r], relu(W_n.x_r + b_n)) + b_o)>
+ *   loss   = mean_r (pred_r - y_r)^2  over the n rows of the batch,
+ * then one Adam step (torch.optim.Adam's update, DENSE gradients: every element's moments decay every step).
+ *
+ * hals_tower_params is hals_tower_weights with mutable tensors (the same fields in the same order, no scaler: the
+ * training step takes numerics already scaled).  Table sizes must be given (> 0); widths as for hals_tower_item with
+ * embedding_size in [1,64].  The same struct describes Adam's first and second moments m / v (same shapes).
+ *
+ * hals_tower_batch: the n rows of one step.  order_* are each table's ids sorted stably: order_user[k] is the batch
+ * position of the k-th smallest user id, ties in ascending position (a stable argsort of user_ids).  An id outside its
+ * table reads as a zero row and produces no gradient.
+ *
+ * hals_tower_train_step: forward and backward of the batch.  Writes the gradients of step `t` into `workspace`:
+ * per-row gradients of the four gathered embedding rows, per-CTA partials of the dense tensors, and for every table
+ * row the batch touches a stamp (t, first sorted position).  *loss (device float) = the batch mean squared error.
+ * hals_tower_adam_step: one Adam step over every parameter from those gradients, in one launch:
+ *   g  = sum of the batch's gradients (embedding rows: over the row's batch positions in ascending order; dense
+ *        tensors: per-CTA partials in CTA order; an embedding row the batch does not touch has g = 0)
+ *   m  = lerp(m, g, 1 - beta1);  v = v * beta2 + (1 - beta2) g^2
+ *   p -= (lr / bc1) m / (sqrt(v) / sqrt(bc2) + eps),   bc_i = 1 - beta_i^t computed in double on the host;
+ *   the scalars are doubles, as torch's are: 1 - beta1, beta2, 1 - beta2, lr / bc1, sqrt(bc2) and eps are computed
+ *   in double and each rounded once to fp32.
+ * Call hals_tower_train_step(t) then hals_tower_adam_step(t) with the same params, batch and workspace, t = 1, 2, ...
+ * increasing (t <= INT32_MAX) between zero-fills of the workspace.
+ *   - workspace: hals_tower_train_workspace_bytes(params, max n) bytes, zero-filled before the first step;
+ *   - no float atomics: both calls are bitwise reproducible for the same inputs;
+ *   - null pointers, bad widths, table sizes <= 0, n < 1, t < 1, a too small workspace: HALS_ERR_INVALID /
+ *     HALS_ERR_WORKSPACE before any CUDA call.
+ * ---------------------------------------------------------------------------------- */
+typedef struct hals_tower_params {
+  int32_t embedding_size, manu_dim, cat_dim, num_hidden;
+  float* user_emb;
+  float* item_emb;
+  float* manu_emb;
+  float* cat_emb;
+  float* num_w;
+  float* num_b;
+  float* out_w;
+  float* out_b;
+  float* user_ln_g;
+  float* user_ln_b;
+  float* item_ln_g;
+  float* item_ln_b;
+  float ln_eps;
+  int32_t num_users, num_items, num_manufacturers, num_categories;
+} hals_tower_params;
+
+typedef struct hals_tower_batch {
+  int64_t n;                                   /* rows in the batch (>= 1)      */
+  const int32_t* user_ids;                     /* [n]                           */
+  const int32_t* item_ids;                     /* [n]                           */
+  const int32_t* manufacturer_ids;             /* [n]                           */
+  const int32_t* category_ids;                 /* [n]                           */
+  const float* numeric;                        /* [n,2] scaled (price, rating)  */
+  const float* labels;                         /* [n] average_review_rating     */
+  const int32_t* order_user;                   /* [n] stable argsort of the ids */
+  const int32_t* order_item;
+  const int32_t* order_manufacturer;
+  const int32_t* order_category;
+} hals_tower_batch;
+
+size_t hals_tower_train_workspace_bytes(const hals_tower_params* params, int64_t max_batch);
+int hals_tower_train_step(const hals_tower_params* params, const hals_tower_batch* batch, int64_t t, void* workspace,
+                          size_t workspace_bytes, float* loss, void* stream);
+int hals_tower_adam_step(const hals_tower_params* params, const hals_tower_params* m, const hals_tower_params* v,
+                         const hals_tower_batch* batch, int64_t t, const void* workspace, size_t workspace_bytes,
+                         double lr, double beta1, double beta2, double eps, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Hybrid scoring.  Replaces, for a batch of users at once, the per-user loop
  *   ALSModel.predict_for_user      src/als_model.py:68-91   (model.transform at :75)
  *   TwoTowerModel.predict_for_user src/two_tower_model.py:136-146 (model.predict at :145)
